@@ -235,6 +235,22 @@ def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as <path>/<name>.npy in float64 (the counts and indices here are exact in it).  An array longer
+    than its even share of DUMP_BYTES is cut to a sample at fixed, seeded positions, so runs with the same arguments stay
+    comparable element for element."""
+    os.makedirs(path, exist_ok=True)
+    share = (DUMP_BYTES // max(1, len(arrays)) - 128) // 8   # elements per file; 128 bytes of .npy header each
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).reshape(-1)
+        if a.size > share:
+            a = a[np.sort(np.random.default_rng(SEED).choice(a.size, share, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- GPU arm helpers
 class Env:
     pass
@@ -617,7 +633,13 @@ def main():
     ap.add_argument("--verify", action="store_true", help="N>1: ALSO check the full-size merged counts against one GPU over the union of all shards (slow)")
     ap.add_argument("--merge", default="lib", choices=["lib", "py-p2p", "py-nccl"], help="N>1: merge inside the library over NCCL with key records routed inside k_pair (default); py-*: round 1's host-driven choreography (routed / NCCL all-to-all)")
     ap.add_argument("--mismatches", type=int, default=0, help="num_mismatches of the library config (C5 sweeps 0/1/2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the counts the top-level timed job returned in its "
+                    "last step as DIR/<name>.npy (float64), to compare two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU arm computed (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = max(args.warmup, 1)
     if args.impl == "reference":
@@ -711,6 +733,7 @@ def main():
         sampler.start()
     tw0 = time.time()
     ms_dev, (counts_dev, uniq_dev) = timed(env, lambda: job(n, True), args.steps)
+    raw_dev = counts_dev
     tw1 = time.time()
     ks = ctx.kernel_stats(reset=True)
     clocks = sampler.stop(tw0, tw1) if rank == 0 else None
@@ -840,6 +863,10 @@ def main():
             c3["block_wall_s"] = time.time() - t0
             out["c3"] = c3
     if rank == 0:
+        if args.dump_outputs:
+            # slot_to_callset maps dictionary slots (where colliding callsets land depends on the order threads insert them)
+            # for per-pair records this job does not ask for; everything else is ordered by callset content
+            dump_outputs(args.dump_outputs, {k: v for k, v in raw_dev.items() if k != "slot_to_callset"})
         emit_json(out)
     if world > 1:
         dist.destroy_process_group()
