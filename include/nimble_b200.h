@@ -127,7 +127,7 @@ int nb_ctx_create(const nb_index* index, const nb_library* lib, int device, void
 void nb_ctx_free(nb_ctx*);
 int nb_ctx_set_config(nb_ctx*, const nb_config* cfg);   /* config is read by pseudoalign / filter_and_coerce per call */
 int nb_ctx_sync(nb_ctx*);
-/* tuning knobs: "max_batch_pairs", "ec_arena_entries", "callset_slots", "key_slots", "agg_slots", "count_work" */
+/* tuning knobs: "max_batch_pairs", "ec_arena_entries", "callset_slots", "key_slots", "agg_slots", "count_work", "cell_slots" */
 int nb_ctx_set_option(nb_ctx*, const char* name, uint64_t value);
 
 /* pinned host memory for the caller's double-buffered batches (src/parse readers feed these) */
@@ -217,6 +217,26 @@ int nb_counts_device_rows(nb_ctx*, const void** row_scope, const void** row_call
 int nb_counts_reset(nb_ctx*);
 uint32_t nb_library_n_groups(const nb_library*);
 const char* nb_library_group_name(const nb_library*, uint32_t group);
+
+/* Per-cell count table of BAM mode: the per-scope rows of successive scoped batches rolled up by cell, in a table of the
+ * context that nb_counts_reset leaves alone.  For cell c and callset S: umis = scopes of c with a row for S (a scope has at
+ * most one), reads = sum of those rows' counts (nimble_score).  Callsets are numbered persistently across batches (every
+ * finalize renumbers its own).
+ *   nb_cells_roll      after nb_counts_finalize of a scoped batch, once per batch: cell_of_scope[scope_id] = cell id (< 2^32 - 1,
+ *                      else NB_ERR_UNSUPPORTED) for the batch's n_scopes scopes.  The table grows on the device as needed;
+ *                      option "cell_slots" sets its first size (before the first roll).  Synchronous: cell_of_scope may be reused
+ *   nb_cells_finalize  rows sorted by (cell id, callset); callsets = those with a row, numbered in Vec<String> Ord
+ *                      (utils::sort_score_vector) with their group lists as in nb_counts.  Pointers stay valid until the next
+ *                      nb_cells_finalize / nb_cells_reset / nb_ctx_free; the table itself is kept (more batches may follow)
+ *   nb_cells_reset     empty table and callset numbering */
+typedef struct nb_cell_counts {
+  uint64_t n_rows; const uint32_t* row_cell; const uint32_t* row_callset; const int64_t* row_umis; const int64_t* row_reads;
+  uint64_t n_callsets; const uint64_t* callset_off; const uint32_t* callset_items;
+  uint64_t n_scopes;           /* scopes rolled in */
+} nb_cell_counts;
+int nb_cells_roll(nb_ctx*, const uint32_t* cell_of_scope, uint64_t n_scopes);
+int nb_cells_finalize(nb_ctx*, nb_cell_counts* out);
+int nb_cells_reset(nb_ctx*);
 
 /* multi-GPU merge of the whole-run scope (SURVEY.md §8e).  Reads shard over ranks with the index replicated; counts
  * are over unique read_keys of the whole run, so ranks exchange their de-duplication records by key range
@@ -340,6 +360,19 @@ int nb_gunzip_parallel(const void* in, uint64_t in_len, int threads, uint64_t ch
 int nb_bam_dump_groups(const char* input_file, int force_bam_paired, int num_cores, const char* out_path);
 int nb_process_bam(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
                    int strand_filter, const char* trim, int num_cores, int force_bam_paired, int device);
+/* The same run with a cell x feature count matrix per library (nb_cells_*): matrix_dirs[i] receives library i's matrix
+ * (nb_write_cell_matrix).  The cell of a scope is the full CB of its first record; the barcodes are the CBs that start a
+ * scope, in order of first appearance (one list for all libraries).  output_paths NULL: no TSV rows at all (the rows stage
+ * is not run); matrix_dirs NULL: exactly nb_process_bam.  One of the two must be given. */
+int nb_process_bam_cells(const char* input_file, const char* const* reference_json, const char* const* output_paths,
+                         const char* const* matrix_dirs, uint32_t n_refs, int strand_filter, const char* trim, int num_cores,
+                         int force_bam_paired, int device);
+/* host-only: a cell x feature matrix in the 10x v3 layout that Seurat's Read10X and scanpy's read_10x_mtx load, into `dir`
+ * (created when missing; its parent must exist): matrix.mtx.gz (Matrix Market coordinate integer, features x barcodes, UMI
+ * counts, 1-based lines sorted by barcode then feature), reads.mtx.gz (the same coordinates with the read counts),
+ * features.tsv.gz ("callset<TAB>callset<TAB>Gene Expression", callset = group names joined by ','), barcodes.tsv.gz.  Gzip
+ * members with mtime 0 and no file name: the same counts give the same bytes. */
+int nb_write_cell_matrix(const char* dir, const nb_library* lib, const nb_cell_counts* counts, const char* const* barcodes, uint64_t n_barcodes);
 
 #ifdef __cplusplus
 }

@@ -68,6 +68,12 @@ class Counts(C.Structure):
                 ("n_slots", C.c_uint64), ("slot_to_callset", C.POINTER(C.c_uint32))]
 
 
+class CellCounts(C.Structure):  # nb_cell_counts
+    _fields_ = [("n_rows", C.c_uint64), ("row_cell", C.POINTER(C.c_uint32)), ("row_callset", C.POINTER(C.c_uint32)),
+                ("row_umis", C.POINTER(C.c_int64)), ("row_reads", C.POINTER(C.c_int64)), ("n_callsets", C.c_uint64),
+                ("callset_off", C.POINTER(C.c_uint64)), ("callset_items", C.POINTER(C.c_uint32)), ("n_scopes", C.c_uint64)]
+
+
 READ_DT = np.dtype([("reason", "u1"), ("pass", "u1"), ("score", "<u2"), ("mismatches", "<u2"), ("trimmed_len", "<u2"),
                     ("ec_len", "<u4"), ("ec_hash", "<u4")])
 PAIR_DT = np.dtype([("callset", "<u4"), ("triage", "u1"), ("fr1", "u1"), ("fr2", "u1"), ("insertable", "u1"),
@@ -143,6 +149,11 @@ _SIGS = {
     "nb_inflate": (C.c_int, [C.c_char_p, C.c_uint64, C.c_int, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
     "nb_process_fastq_devices": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_void_p, C.c_uint32]),
     "nb_process_bam": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]),
+    "nb_process_bam_cells": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]),
+    "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
+    "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
+    "nb_cells_reset": (C.c_int, [C.c_void_p]),
+    "nb_write_cell_matrix": (C.c_int, [C.c_char_p, C.c_void_p, C.POINTER(CellCounts), C.c_void_p, C.c_uint64]),
     "nb_process_fastq": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int]),
 }
 
@@ -519,6 +530,22 @@ class Context:
     def reset(self):
         _ck(lib().nb_counts_reset(self.h))
 
+    # ---- per-cell table (nb_cells_*): survives reset()
+    def cells_roll(self, cell_of_scope):
+        """nb_cells_roll: after counts_raw()/counts() of a scoped batch, cell_of_scope[scope_id] = cell id of each of its scopes."""
+        a = np.ascontiguousarray(cell_of_scope, dtype=np.uint32)
+        _ck(lib().nb_cells_roll(self.h, a.ctypes.data if a.size else None, a.size))
+
+    def cells_finalize(self):
+        """nb_cells_finalize -> dict(row_cell, row_callset, row_umis, row_reads, callset_off, callset_items, n_scopes) (numpy copies);
+        rows sorted by (cell, callset), callsets numbered in Vec<String> Ord."""
+        c = CellCounts()
+        _ck(lib().nb_cells_finalize(self.h, C.byref(c)))
+        return cell_counts_dict(c)
+
+    def cells_reset(self):
+        _ck(lib().nb_cells_reset(self.h))
+
     # ---- peer routing of the whole-run scope (nb_route_*)
     def route_create(self, world, records_per_peer):
         """Allocates the inbox (one region per source rank); returns its 64-byte CUDA IPC handle (np.uint8[64])."""
@@ -638,10 +665,39 @@ def fastq_dump(input_files, out_path, num_cores=1, chunk_bytes=0):
     _ck(lib().nb_fastq_dump(_strs(input_files), len(input_files), num_cores, chunk_bytes, str(out_path).encode()))
 
 
-def process_bam(input_file, reference_json_paths, output_paths, strand_filter="unstranded", trim=None, num_cores=1, force_bam_paired=False, device=0):
-    """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156)."""
+def process_bam(input_file, reference_json_paths, output_paths, strand_filter="unstranded", trim=None, num_cores=1, force_bam_paired=False, device=0,
+                matrix_dirs=None):
+    """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156).
+    matrix_dirs=[dir per library]: also a cell x feature matrix per library (nb_process_bam_cells); output_paths=None with
+    matrix_dirs: no TSV rows at all."""
+    if matrix_dirs is not None or output_paths is None:
+        _ck(lib().nb_process_bam_cells(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths) if output_paths is not None else None,
+                                       _strs(matrix_dirs) if matrix_dirs is not None else None, len(reference_json_paths),
+                                       CHEM[strand_filter], trim.encode() if trim else None, num_cores, int(force_bam_paired), device))
+        return
     _ck(lib().nb_process_bam(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths), len(reference_json_paths),
                              CHEM[strand_filter], trim.encode() if trim else None, num_cores, int(force_bam_paired), device))
+
+
+def cell_counts_dict(c):
+    def arr(p, n, dt):
+        return np.ctypeslib.as_array(p, (n,)).copy() if n else np.zeros(0, dt)
+    n_items = int(c.callset_off[c.n_callsets]) if c.n_callsets else 0
+    return dict(row_cell=arr(c.row_cell, c.n_rows, np.uint32), row_callset=arr(c.row_callset, c.n_rows, np.uint32),
+                row_umis=arr(c.row_umis, c.n_rows, np.int64), row_reads=arr(c.row_reads, c.n_rows, np.int64),
+                callset_off=arr(c.callset_off, c.n_callsets + 1, np.uint64) if c.n_callsets else np.zeros(1, np.uint64),
+                callset_items=arr(c.callset_items, n_items, np.uint32), n_scopes=c.n_scopes)
+
+
+def write_cell_matrix(out_dir, library, counts, barcodes):
+    """nb_write_cell_matrix (host-only): `counts` is a cells_finalize() dict, `barcodes` the cell ids' CB strings."""
+    keep = {k: np.ascontiguousarray(counts[k], dtype=dt) for k, dt in (("row_cell", np.uint32), ("row_callset", np.uint32), ("row_umis", np.int64),
+                                                                      ("row_reads", np.int64), ("callset_off", np.uint64), ("callset_items", np.uint32))}
+    p = lambda k, t: keep[k].ctypes.data_as(C.POINTER(t))
+    c = CellCounts(len(keep["row_cell"]), p("row_cell", C.c_uint32), p("row_callset", C.c_uint32), p("row_umis", C.c_int64), p("row_reads", C.c_int64),
+                   len(keep["callset_off"]) - 1, p("callset_off", C.c_uint64), p("callset_items", C.c_uint32), int(counts.get("n_scopes", 0)))
+    bc = _strs(barcodes)
+    _ck(lib().nb_write_cell_matrix(str(out_dir).encode(), library.h, C.byref(c), bc if len(barcodes) else None, len(barcodes)))
 
 
 def inflate(data, raw=False, window=0, out_cap=None):

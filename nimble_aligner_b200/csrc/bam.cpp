@@ -28,6 +28,7 @@
 #include <thread>
 #include <vector>
 
+#include <errno.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
 #include "host.hpp"
@@ -693,7 +694,102 @@ bool gzip_member(const std::string& text, int level, std::string& out) {
   out.resize(n); return true;
 }
 
+// Run-wide cell barcodes (nb_process_bam_cells): id = order of first appearance.  The fill stage hashes the CB of every
+// group and looks it up (find: read-only, full-string check) on all threads; one serial pass in group order then adds the
+// barcodes not found (tens of millions of groups: a std::unordered_map<std::string, ...> lookup per group, or any serial
+// pass touching every group's record, would cost seconds).
+struct CellDict {
+  std::string names; std::vector<u64> off{0}, hash; std::vector<u32> slot;   // names: NUL-terminated, back to back
+  CellDict() { clear(); }
+  void clear() { names.clear(); off.assign(1, 0); hash.clear(); slot.assign((size_t)1 << 16, NONE32); }
+  size_t size() const { return hash.size(); }
+  static u64 hash_of(const char* p, u32 n) {
+    u64 h = 0x9E3779B97F4A7C15ull ^ n; u32 i = 0;
+    for (; i + 8 <= n; i += 8) { u64 w; memcpy(&w, p + i, 8); h = (h ^ w) * 0xFF51AFD7ED558CCDull; h ^= h >> 32; }
+    u64 w = 0; memcpy(&w, p + i, n - i); h = (h ^ w) * 0xC4CEB9FE1A85EC53ull; return h ^ (h >> 29);
+  }
+  u32 find(const char* p, u32 n, u64 h) const {
+    const u64 m = slot.size() - 1;
+    for (u64 i = h & m;; i = (i + 1) & m) {
+      const u32 id = slot[i]; if (id == NONE32) return NONE32;
+      if (hash[id] == h && off[id + 1] - off[id] - 1 == n && !memcmp(&names[off[id]], p, n)) return id;
+    }
+  }
+  u32 intern(const char* p, u32 n, u64 h) {
+    if (2 * (hash.size() + 1) > slot.size()) {   // grow: the stored hashes place every id again
+      slot.assign(slot.size() * 2, NONE32); const u64 m = slot.size() - 1;
+      for (u32 id = 0; id < hash.size(); id++) { u64 i = hash[id] & m; while (slot[i] != NONE32) i = (i + 1) & m; slot[i] = id; }
+    }
+    const u32 found = find(p, n, h); if (found != NONE32) return found;
+    const u64 m = slot.size() - 1; u64 i = h & m;
+    while (slot[i] != NONE32) i = (i + 1) & m;
+    const u32 id = (u32)hash.size(); slot[i] = id; hash.push_back(h); names.append(p, n); names.push_back('\0'); off.push_back(names.size());
+    return id;
+  }
+};
+
+// text -> gzip members of the rows' compressor, written to `path`; the text is cut into pieces of a fixed size (compressed on
+// several threads) so that the bytes do not depend on the thread count
+int write_gz_pieces(const std::string& path, const std::vector<std::string>& pieces) {
+  std::vector<std::string> member(pieces.size());
+  const int T = (int)std::max<size_t>(1, std::min<size_t>(pieces.size(), std::max(1u, std::min(16u, std::thread::hardware_concurrency()))));
+  std::atomic<size_t> next(0);
+  parallel_ranges(T, (size_t)T, [&](size_t, size_t, int) {
+    std::unique_ptr<nbz::FastDeflate> fd(new nbz::FastDeflate());
+    for (size_t i; (i = next.fetch_add(1)) < pieces.size();) fd->gzip_member((const u8*)pieces[i].data(), pieces[i].size(), member[i]);
+  });
+  FILE* f = fopen(path.c_str(), "wb"); if (!f) return fail(NB_ERR_IO, "could not open " + path);
+  bool ok = true;
+  for (const std::string& m : member) ok = ok && fwrite(m.data(), 1, m.size(), f) == m.size();
+  ok = fclose(f) == 0 && ok;
+  return ok ? NB_OK : fail(NB_ERR_IO, "short write on " + path);
+}
+inline char* put_u64(char* p, u64 v) { char t[20]; int n = 0; do { t[n++] = (char)('0' + v % 10); v /= 10; } while (v); while (n) *p++ = t[--n]; return p; }
+
 }  // namespace
+
+extern "C" int nb_write_cell_matrix(const char* dir, const nb_library* lib, const nb_cell_counts* cc, const char* const* barcodes, uint64_t n_barcodes) {
+  if (!dir || !*dir || !lib || !cc || (!barcodes && n_barcodes)) return fail(NB_ERR_INVALID, "null argument");
+  const u64 n = cc->n_rows, ncs = cc->n_callsets;
+  if ((n && (!cc->row_cell || !cc->row_callset || !cc->row_umis || !cc->row_reads)) || (ncs && (!cc->callset_off || !cc->callset_items))) return fail(NB_ERR_INVALID, "null array in the cell counts");
+  for (u64 b = 0; b < n_barcodes; b++) if (!barcodes[b]) return fail(NB_ERR_INVALID, "null barcode");
+  const u32 n_groups = nb_library_n_groups(lib);
+  for (u64 c = 0; c < ncs; c++) for (u64 k = cc->callset_off[c]; k < cc->callset_off[c + 1]; k++) if (cc->callset_items[k] >= n_groups) return fail(NB_ERR_INVALID, "callset item is not a group of the library");
+  for (u64 i = 0; i < n; i++) {
+    if (cc->row_cell[i] >= n_barcodes || cc->row_callset[i] >= ncs) return fail(NB_ERR_INVALID, "row outside the barcodes / callsets");
+    if (cc->row_umis[i] < 0 || cc->row_reads[i] < 0) return fail(NB_ERR_INVALID, "negative count");
+    if (i && (cc->row_cell[i] < cc->row_cell[i - 1] || (cc->row_cell[i] == cc->row_cell[i - 1] && cc->row_callset[i] <= cc->row_callset[i - 1]))) return fail(NB_ERR_INVALID, "rows are not sorted by (cell, callset)");
+  }
+  if (mkdir(dir, 0777) != 0 && errno != EEXIST) return fail(NB_ERR_IO, std::string("could not create ") + dir);
+  struct stat st; if (stat(dir, &st) != 0 || !S_ISDIR(st.st_mode)) return fail(NB_ERR_IO, std::string(dir) + " is not a directory");
+  const std::string d(dir);
+  std::vector<std::string> pieces(1);
+  for (u64 c = 0; c < ncs; c++) {
+    std::string name;
+    for (u64 k = cc->callset_off[c]; k < cc->callset_off[c + 1]; k++) { if (k > cc->callset_off[c]) name += ','; name += nb_library_group_name(lib, cc->callset_items[k]); }
+    pieces[0] += name; pieces[0] += '\t'; pieces[0] += name; pieces[0] += "\tGene Expression\n";
+  }
+  int rc = write_gz_pieces(d + "/features.tsv.gz", pieces); if (rc) return rc;
+  pieces.assign(1, std::string());
+  for (u64 b = 0; b < n_barcodes; b++) { pieces[0] += barcodes[b]; pieces[0] += '\n'; }
+  rc = write_gz_pieces(d + "/barcodes.tsv.gz", pieces); if (rc) return rc;
+  // Matrix Market: features are the rows, barcodes the columns; lines in (barcode, feature) order as the counts come
+  const u64 PIECE = (u64)1 << 20;   // lines per gzip member
+  for (int which = 0; which < 2; which++) {
+    const i64* val = which ? cc->row_reads : cc->row_umis;
+    pieces.assign(1 + (n + PIECE - 1) / PIECE, std::string());
+    pieces[0] = "%%MatrixMarket matrix coordinate integer general\n" + std::to_string(ncs) + " " + std::to_string(n_barcodes) + " " + std::to_string(n) + "\n";
+    parallel_ranges((int)std::min<u64>(16, pieces.size() - 1), pieces.size() - 1, [&](size_t a, size_t b, int) {
+      for (size_t q = a; q < b; q++) {
+        const u64 r0 = q * PIECE, r1 = std::min(n, r0 + PIECE);
+        std::string& t = pieces[q + 1]; t.resize((r1 - r0) * 64); char* p = &t[0];
+        for (u64 i = r0; i < r1; i++) { p = put_u64(p, (u64)cc->row_callset[i] + 1); *p++ = ' '; p = put_u64(p, (u64)cc->row_cell[i] + 1); *p++ = ' '; p = put_u64(p, (u64)val[i]); *p++ = '\n'; }
+        t.resize((size_t)(p - t.data()));
+      } });
+    rc = write_gz_pieces(d + (which ? "/reads.mtx.gz" : "/matrix.mtx.gz"), pieces); if (rc) return rc;
+  }
+  return NB_OK;
+}
 
 // host-only: one gzip member made by the rows stage's compressor (deflate_fast.hpp) — tests inflate it with zlib
 extern "C" int nb_gzip_fast(const void* in, uint64_t in_len, void* out, uint64_t out_cap, uint64_t* out_len) {
@@ -706,10 +802,18 @@ extern "C" int nb_gzip_fast(const void* in, uint64_t in_len, void* out, uint64_t
   return NB_OK;
 }
 
-// process::bam::process behind main.rs's library loop (src/bin/main.rs:95-156)
 extern "C" int nb_process_bam(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs, int strand_filter,
-                              const char* trim /* "L:S,L:S" or NULL */, int num_cores, int force_bam_paired, int device) {
-  if (!input_file || !reference_json || !output_paths || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference/output pair");
+                              const char* trim, int num_cores, int force_bam_paired, int device) {
+  if (!output_paths) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference/output pair");
+  return nb_process_bam_cells(input_file, reference_json, output_paths, nullptr, n_refs, strand_filter, trim, num_cores, force_bam_paired, device);
+}
+
+// process::bam::process behind main.rs's library loop (src/bin/main.rs:95-156); matrix_dirs: per-cell matrices as well,
+// output_paths NULL: no TSV rows
+extern "C" int nb_process_bam_cells(const char* input_file, const char* const* reference_json, const char* const* output_paths, const char* const* matrix_dirs,
+                                    uint32_t n_refs, int strand_filter, const char* trim /* "L:S,L:S" or NULL */, int num_cores, int force_bam_paired, int device) {
+  if (!input_file || !reference_json || (!output_paths && !matrix_dirs) || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference/output pair");
+  const bool want_rows = output_paths != nullptr, want_cells = matrix_dirs != nullptr;
   int threads = std::max(1, num_cores);
   std::vector<nb_library*> libs(n_refs, nullptr); std::vector<nb_index*> idx(n_refs, nullptr); std::vector<nb_ctx*> ctx(n_refs, nullptr); std::vector<FILE*> outs(n_refs, nullptr);
   std::vector<bool> first_write(n_refs, true);
@@ -727,10 +831,10 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
     if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);   // K5: the CUDA builder (same artefact as the host builder), or $NB_INDEX_CACHE
     if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nullptr, &ctx[i]);
     if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);   // a batch of 2^20 pairs can hold that many one-pair scopes, each with its own (scope, callset) row: stay under half full
-    if (rc == NB_OK) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
+    if (rc == NB_OK && want_rows) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
   }
   auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  double t_load = 0, t_group = 0, t_fill = 0, t_gpu = 0, t_rows = 0, t_align = 0, t_final = 0, t0 = now(); const double t_start = t0;   // NB_BAM_STATS=1 prints the phase times
+  double t_load = 0, t_group = 0, t_fill = 0, t_gpu = 0, t_rows = 0, t_align = 0, t_final = 0, t_roll = 0, t_cells = 0, t0 = now(); const double t_start = t0;   // NB_BAM_STATS=1 prints the phase times
   // window size of the streaming producer: NB_BAM_WINDOW_MB (inflated bytes per window; tests use small ones), default 256 MB
   size_t window_bytes = (size_t)256 << 20;
   if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = (size_t)strtoull(e, nullptr, 10) << 10;
@@ -742,12 +846,13 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
   // Three stages run concurrently on consecutive batches: (F) the host threads fill batch k+1 into pinned buffers,
   // (D) the device aligns batch k and its counts are finalized, (R) the host threads format + gzip the rows of batch k-1.
   struct Pinned { u8* p = nullptr; size_t cap = 0; int ensure(size_t n) { if (n <= cap) return NB_OK; nb_host_free(p); cap = n + n / 4 + 4096; p = (u8*)nb_host_alloc(cap); if (!p) { cap = 0; return fail(NB_ERR_CUDA, "pinned host allocation failed"); } return NB_OK; } ~Pinned() { nb_host_free(p); } };
-  struct BatchIn { const std::vector<Rec>* stream = nullptr; const std::vector<u64>* gstart = nullptr; size_t g0 = 0, g1 = 0, np = 0; u32 maxlen = 1; std::vector<u64> pair0, o1, o2; std::vector<u32> l1, l2; std::vector<u8> f1, f2; std::vector<u32> scope; Pinned r1, r2, q1, q2; };
+  struct BatchIn { const std::vector<Rec>* stream = nullptr; const std::vector<u64>* gstart = nullptr; size_t g0 = 0, g1 = 0, np = 0; u32 maxlen = 1; std::vector<u64> pair0, o1, o2; std::vector<u32> l1, l2; std::vector<u8> f1, f2; std::vector<u32> scope, cell; std::vector<u64> cb_hash; Pinned r1, r2, q1, q2; };
   struct BatchOut { std::vector<nb_read_result> rres; std::vector<nb_pair_result> pres; std::vector<u64> row_begin, callset_off; std::vector<u32> row_callset, callset_items, slot_to_callset; std::vector<i64> row_count; };
   BatchIn bin[3]; BatchOut bout[2];
   // the window being processed (its records and groups): set by the window loop below, read by the three stages
   const std::vector<Rec>* cur_stream = nullptr; const std::vector<u64>* cur_gstart = nullptr;
   std::atomic<u64> ns_fill(0), ns_rows(0);
+  CellDict cells;   // (matrix_dirs) cell of a scope = the full CB of its first record; fills run in stream order, so ids are first-appearance order
   // ---- (F) batch arrays: even record = sequence slot, odd = mate slot (src/process/bam.rs:257-292)
   auto fill = [&](BatchIn& B, size_t g0, size_t g1) -> int {
     double tb = now();
@@ -791,6 +896,16 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
         for (size_t j = 0; j < B.pair0[g + 1] - B.pair0[g]; j++) { size_t x, y; const size_t p = B.pair0[g] + j;
           clip_of(v[2 * j], x, y); by1[p] = 2 * by1[p] + (x & 1); clip_of(v[2 * j + 1], x, y); by2[p] = 2 * by2[p] + (x & 1); } } });
     by1[np] = 2 * tot1; by2[np] = 2 * tot2;
+    if (want_cells) {
+      B.cell.assign(ng, 0); B.cb_hash.resize(ng);
+      std::vector<std::vector<u32>> miss(threads);   // groups whose CB the dictionary did not know yet, per thread in group order
+      parallel_ranges(threads, ng, [&](size_t a, size_t b, int t) {
+        for (size_t g = a; g < b; g++) if (gstart[g0 + g + 1] > gstart[g0 + g]) {   // (a group without records has no pairs: its cell is never read)
+          const Rec& r = stream[gstart[g0 + g]]; const u64 h = B.cb_hash[g] = CellDict::hash_of(r.cb, r.cb_len);
+          if ((B.cell[g] = cells.find(r.cb, r.cb_len, h)) == NONE32) miss[t].push_back((u32)g);
+        } });
+      for (const std::vector<u32>& mt : miss) for (u32 g : mt) { const Rec& r = stream[gstart[g0 + g]]; B.cell[g] = cells.intern(r.cb, r.cb_len, B.cb_hash[g]); }
+    }
     ns_fill += (u64)((now() - tb) * 1e9);
     return NB_OK;
   };
@@ -802,18 +917,20 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
     b.n_pairs = B.np; b.location = NB_MEM_HOST; b.max_read_len = B.maxlen; b.r1 = B.r1.p; b.r1_off = B.o1.data(); b.r2 = B.r2.p; b.r2_off = B.o2.data();
     b.q1 = B.q1.p; b.q2 = B.q2.p; b.flags1 = B.f1.data(); b.flags2 = B.f2.data(); b.scope_id = B.scope.data();
     b.encoding = NB_SEQ_BAM4; b.r1_len = B.l1.data(); b.r2_len = B.l2.data();
-    O.rres.resize(2 * B.np); O.pres.resize(B.np);
+    if (want_rows) { O.rres.resize(2 * B.np); O.pres.resize(B.np); }
     double ta = now();
     int e = nb_counts_reset(ctx[li]); if (e) return e;
     e = nb_ctx_set_option(ctx[li], "max_batch_pairs", std::max<size_t>(B.np, 1)); if (e) return e;
     double tb1 = now();
-    e = nb_align_batch(ctx[li], &b, O.rres.data(), O.pres.data()); if (e) return e;
+    e = nb_align_batch(ctx[li], &b, want_rows ? O.rres.data() : nullptr, want_rows ? O.pres.data() : nullptr); if (e) return e;
     double tb2 = now(); nb_ctx_sync(ctx[li]); double tb3 = now();
     if (getenv("NB_BAM_STATS")) fprintf(stderr, "  batch: np=%zu resize %.1f ms, reset+opt %.1f ms, align call %.1f ms, sync %.1f ms\n", B.np, (ta - tb) * 1e3, (tb1 - ta) * 1e3, (tb2 - tb1) * 1e3, (tb3 - tb2) * 1e3);
     t_align += now() - tb; double tf = now();
     nb_counts cts; e = nb_counts_finalize(ctx[li], &cts); if (e) return e;
     t_final += now() - tf;
     const size_t ng = B.g1 - B.g0;
+    if (want_cells) { const double tr = now(); e = nb_cells_roll(ctx[li], B.cell.data(), ng); t_roll += now() - tr; if (e) return e; }
+    if (!want_rows) { t_gpu += now() - tb; return NB_OK; }
     O.row_begin.assign(ng + 1, 0);
     for (u64 r = 0; r < cts.n_rows; r++) O.row_begin[cts.row_scope[r] + 1]++;
     for (size_t g = 0; g < ng; g++) O.row_begin[g + 1] += O.row_begin[g];
@@ -907,7 +1024,7 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
         if (li == 0 && k + 1 < nb_) fut_fill = std::async(std::launch::async, [&, k, slot]() { return wrap(fill(bin[(slot + k + 1) % 3], batches[k + 1].first, batches[k + 1].second)); });
         e = on_device(bin[(slot + k) % 3], li, bout[it_global % 2]);
         { int er = join(fut_rows); if (er && !e) e = er; }
-        if (!e) { const BatchIn* bi = &bin[(slot + k) % 3]; const BatchOut* bo = &bout[it_global % 2]; fut_rows = std::async(std::launch::async, [&, bi, bo, li]() { return wrap(rows(*bi, li, *bo)); }); }
+        if (!e && want_rows) { const BatchIn* bi = &bin[(slot + k) % 3]; const BatchOut* bo = &bout[it_global % 2]; fut_rows = std::async(std::launch::async, [&, bi, bo, li]() { return wrap(rows(*bi, li, *bo)); }); }
         if (li + 1 == n_refs) { int ef = join(fut_fill); if (ef && !e) e = ef; }
       }
     }
@@ -938,7 +1055,8 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
   if (whole_file) {
     // the serial readers' empty-UMI / key-concatenation quirks need the whole file: start over with everything resident
     rc = NB_OK;
-    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) { if (ftruncate(fileno(outs[li]), 0) != 0 || fseek(outs[li], 0, SEEK_SET) != 0) rc = fail(NB_ERR_IO, "could not rewind the output"); first_write[li] = true; }
+    for (u32 li = 0; li < n_refs && rc == NB_OK && want_rows; li++) { if (ftruncate(fileno(outs[li]), 0) != 0 || fseek(outs[li], 0, SEEK_SET) != 0) rc = fail(NB_ERR_IO, "could not rewind the output"); first_write[li] = true; }
+    if (want_cells) { cells.clear(); for (u32 li = 0; li < n_refs && rc == NB_OK; li++) rc = nb_cells_reset(ctx[li]); }
     Bgzf z; std::vector<Rec> stream; std::vector<u64> gstart;
     if (rc == NB_OK) rc = z.load(input_file, threads);
     if (rc == NB_OK) rc = collect_groups_serial(z, force_bam_paired != 0, threads, stream, gstart);
@@ -947,11 +1065,17 @@ extern "C" int nb_process_bam(const char* input_file, const char* const* referen
   }
   t_load = t_prod; t_group = 0;
   t_fill = ns_fill.load() * 1e-9; t_rows = ns_rows.load() * 1e-9;
-  if (rc == NB_OK) for (u32 li = 0; li < n_refs; li++) if (first_write[li]) { std::string em; if (!gzip_member(std::string(), GZ_LEVEL ? GZ_LEVEL : 2, em) || fwrite(em.data(), 1, em.size(), outs[li]) != em.size()) rc = fail(NB_ERR_IO, "short write on the TSV"); }   // no row at all: an empty gzip stream, like the reference's untouched GzEncoder
+  if (rc == NB_OK && want_rows) for (u32 li = 0; li < n_refs; li++) if (first_write[li]) { std::string em; if (!gzip_member(std::string(), GZ_LEVEL ? GZ_LEVEL : 2, em) || fwrite(em.data(), 1, em.size(), outs[li]) != em.size()) rc = fail(NB_ERR_IO, "short write on the TSV"); }   // no row at all: an empty gzip stream, like the reference's untouched GzEncoder
+  if (rc == NB_OK && want_cells) {
+    const double tc = now();
+    std::vector<const char*> bc(cells.size()); for (size_t i = 0; i < bc.size(); i++) bc[i] = cells.names.data() + cells.off[i];
+    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) { nb_cell_counts cc; rc = nb_cells_finalize(ctx[li], &cc); if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size()); }
+    t_cells = now() - tc;
+  }
   if (getenv("NB_BAM_STATS")) {
     // peak resident set of THIS process image (VmHWM belongs to the mm, so unlike ru_maxrss it does not start at the forking parent's size)
     double hwm_mb = 0; if (FILE* st = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, st)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(st); }
-    fprintf(stderr, "nb_process_bam: %zu records in %zu groups%s; windows (read+inflate+group, overlapped) %.2fs, largest window %.0f MB, batch fill %.2fs, device align+finalize %.2fs (align %.2fs, finalize %.2fs), rows+gzip+write %.2fs (fill and rows overlap the device stage), total %.2fs, peak RSS %.0f MB\n", n_records_total, n_groups_total, whole_file ? " (whole-file fallback)" : "", t_load, peak_window / 1048576.0, t_fill, t_gpu, t_align, t_final, t_rows, now() - t_start, hwm_mb);
+    fprintf(stderr, "nb_process_bam: %zu records in %zu groups%s; windows (read+inflate+group, overlapped) %.2fs, largest window %.0f MB, batch fill %.2fs, device align+finalize %.2fs (align %.2fs, finalize %.2fs), rows+gzip+write %.2fs (fill and rows overlap the device stage), cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, peak RSS %.0f MB\n", n_records_total, n_groups_total, whole_file ? " (whole-file fallback)" : "", t_load, peak_window / 1048576.0, t_fill, t_gpu, t_align, t_final, t_rows, t_roll, t_cells, now() - t_start, hwm_mb);
   }
   cleanup();
   return rc;

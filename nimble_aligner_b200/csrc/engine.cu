@@ -11,6 +11,7 @@
 #include <memory>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <atomic>
 #include <vector>
 
@@ -124,6 +125,14 @@ struct nb_ctx {
   // multi-GPU merge (nb_comm_*, nb_merge_*): the NCCL communicator this context merges over and its exchange blocks
   ncclComm_t comm = nullptr; bool own_comm = false; u32 cworld = 1, crank = 0; u64 merge_cap = 4096;
   DBuf d_blk1, d_all1, d_blk2, d_all2, d_densetab, d_densework; u64* h_hdr = nullptr;
+  // per-cell table (nb_cells_*): survives nb_counts_reset.  Callsets are keyed by a persistent id (pid) because every finalize
+  // renumbers them: cell_pid maps a callset's group list (as bytes) to its pid, pid_off / pid_items hold the lists in pid order
+  DBuf d_cellkey, d_cellumi, d_cellreads, d_cellctr, d_cellscope, d_cellpid, d_cellwork, d_cellrows;
+  u64 cell_slots = 1u << 22, cell_used = 0, cell_scopes = 0; bool cell_alloc = false;
+  bool cells_rows = false, cells_rolled = false;   // the last finalize left scoped rows not rolled yet / a roll happened since nb_counts_reset
+  std::unordered_map<std::string, u32> cell_pid; std::vector<u64> pid_off{0}; std::vector<u32> pid_items, pid_of_dense;
+  std::vector<u64> cc_off; std::vector<u32> cc_items;   // callsets of the last nb_cells_finalize, in Vec<String> Ord
+  u8* h_cellrows = nullptr; size_t h_cellrows_cap = 0;
 };
 
 static Tables make_tables(nb_ctx* c) {
@@ -307,6 +316,8 @@ void nb_ctx_free(nb_ctx* c) {
   c->ipc_opened.clear(); c->d_inbox.release(); c->d_routecur.release();
   nb_comm_free(c);
   c->d_blk1.release(); c->d_all1.release(); c->d_blk2.release(); c->d_all2.release(); c->d_densetab.release(); c->d_densework.release();
+  for (DBuf* b : {&c->d_cellkey, &c->d_cellumi, &c->d_cellreads, &c->d_cellctr, &c->d_cellscope, &c->d_cellpid, &c->d_cellwork, &c->d_cellrows}) b->release();
+  nb_host_free(c->h_cellrows); c->h_cellrows = nullptr;
   nb_host_free(c->h_hdr); c->h_hdr = nullptr;
   for (int i = 0; i < 4; i++) if (c->live.ev[i]) cudaEventDestroy(c->live.ev[i]);
   nb_host_free(c->live.host); c->live.host = nullptr;
@@ -329,6 +340,7 @@ int nb_ctx_set_option(nb_ctx* c, const char* name, uint64_t value) {
   std::string n(name);
   if (n == "count_work") { c->count_work = value != 0; return NB_OK; }
   if (n == "min_read_length") { c->min_read_len = (u32)value; c->dcfg.min_read_len = (u32)value; return NB_OK; }
+  if (n == "cell_slots") { if (c->cell_alloc) return fail(NB_ERR_INVALID, "cell_slots must be set before the first nb_cells_roll (or after nb_cells_reset)"); c->cell_slots = pow2(value); return NB_OK; }
   if (c->tables_ready) return fail(NB_ERR_INVALID, "options must be set before the first nb_align_batch (or after nb_counts_reset)");
   if (n == "max_batch_pairs") c->max_batch_pairs = std::max<u64>(1, value);
   else if (n == "ec_arena_entries") c->arena_entries = std::max<u64>(1024, value);
@@ -699,6 +711,7 @@ static int finalize_impl(nb_ctx* c, nb_counts* out, u64 dense_cells, bool shard 
     CK(cudaMemcpyAsync(c->h_rows, c->d_rowout.p, n_agg * 16, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
   }
+  if (c->mode == 1) c->cells_rows = !c->cells_rolled;
   struct { size_t n; size_t size() const { return n; } } rows{(size_t)n_agg};
   out->n_rows = rows.size(); out->row_scope = h_scope; out->row_callset = h_callset; out->row_count = h_count;
   out->n_callsets = slots.size(); out->callset_off = c->cs_off.data(); out->callset_items = c->cs_items.data();
@@ -721,8 +734,117 @@ int nb_counts_reset(nb_ctx* c) {
   if (!c) return fail(NB_ERR_INVALID, "null argument");
   CK(cudaSetDevice(c->device));
   if (c->tables_ready) { CK(cudaStreamSynchronize(c->stream)); c->tables_ready = false; }
-  c->mode = -1; c->folded = false; c->pairs_seen = 0; c->have_last = false; c->n_rows_dev = 0;
+  c->mode = -1; c->folded = false; c->pairs_seen = 0; c->have_last = false; c->n_rows_dev = 0; c->cells_rows = c->cells_rolled = false;
   if (c->d_routecur.p) CK(cudaMemsetAsync(c->d_routecur.p, 0, nbk::ROUTE_MAX * 8, c->stream));   // a job abandoned before nb_route_sent must not leak its records into the next one
+  return NB_OK;
+}
+
+static nbk::CellTable cell_table(nb_ctx* c) {
+  return nbk::CellTable{(unsigned long long*)c->d_cellkey.p, (unsigned long long*)c->d_cellumi.p, (unsigned long long*)c->d_cellreads.p, c->cell_slots - 1, (unsigned long long*)c->d_cellctr.p};
+}
+
+int nb_cells_roll(nb_ctx* c, const uint32_t* cell_of_scope, uint64_t n_scopes) {
+  if (!c || (!cell_of_scope && n_scopes)) return fail(NB_ERR_INVALID, "null argument");
+  if (!c->cells_rows) return fail(NB_ERR_INVALID, c->cells_rolled ? "these scopes were already rolled: call nb_counts_reset before the next batch" : "no finalized scoped batch to roll: call nb_counts_finalize first");
+  CK(cudaSetDevice(c->device));
+  const u64 n = c->n_rows_dev;
+  const u32* h_scope = (const u32*)c->h_rows;
+  if (n && h_scope[n - 1] >= n_scopes) return fail(NB_ERR_INVALID, "cell_of_scope has fewer entries than the batch has scopes");   // rows are sorted by scope
+  for (u64 i = 0; i < n_scopes; i++) if (cell_of_scope[i] == NONE32) return fail(NB_ERR_UNSUPPORTED, "cell ids must be below 2^32 - 1");
+  cudaStream_t s = c->stream;
+  // persistent ids of this batch's callsets (thousands: a host map is cheap next to the batch)
+  const u64 n_cs = c->cs_off.size() - 1;
+  c->pid_of_dense.resize(n_cs);
+  for (u64 i = 0; i < n_cs; i++) {
+    const u32* it = c->cs_items.data() + c->cs_off[i]; const u64 len = c->cs_off[i + 1] - c->cs_off[i];
+    auto ins = c->cell_pid.emplace(std::string((const char*)it, len * 4), (u32)(c->pid_off.size() - 1));
+    if (ins.second) { c->pid_items.insert(c->pid_items.end(), it, it + len); c->pid_off.push_back(c->pid_items.size()); }
+    c->pid_of_dense[i] = ins.first->second;
+  }
+  if (c->pid_off.size() - 1 >= NONE32) return fail(NB_ERR_UNSUPPORTED, "more than 2^32 - 1 callsets in the per-cell table");
+  if (!c->cell_alloc) {
+    CK(c->d_cellkey.ensure(c->cell_slots * 8, s)); CK(c->d_cellumi.ensure(c->cell_slots * 8, s)); CK(c->d_cellreads.ensure(c->cell_slots * 8, s)); CK(c->d_cellctr.ensure(16, s));
+    CK(cudaMemsetAsync(c->d_cellkey.p, 0, c->cell_slots * 8, s)); CK(cudaMemsetAsync(c->d_cellumi.p, 0, c->cell_slots * 8, s)); CK(cudaMemsetAsync(c->d_cellreads.p, 0, c->cell_slots * 8, s));
+    CK(cudaMemsetAsync(c->d_cellctr.p, 0, 16, s));
+    c->cell_alloc = true; c->cell_used = 0;
+  }
+  // every row may add an entry: grow first so that the table stays at most half full (the roll then never runs out of slots)
+  if (2 * (c->cell_used + n) > c->cell_slots) {
+    u64 ns = c->cell_slots; while (2 * (c->cell_used + n) > ns) ns <<= 1;
+    DBuf nk, nu, nr; auto rel = [&]() { nk.release(); nu.release(); nr.release(); };
+    auto ck2 = [&](cudaError_t e) { if (e == cudaSuccess) return true; rel(); fail(NB_ERR_CUDA, std::string("cell table growth: ") + cudaGetErrorString(e)); return false; };
+    if (!ck2(nk.ensure(ns * 8, s)) || !ck2(nu.ensure(ns * 8, s)) || !ck2(nr.ensure(ns * 8, s))) return NB_ERR_CUDA;
+    if (!ck2(cudaMemsetAsync(nk.p, 0, ns * 8, s)) || !ck2(cudaMemsetAsync(nu.p, 0, ns * 8, s)) || !ck2(cudaMemsetAsync(nr.p, 0, ns * 8, s))) return NB_ERR_CUDA;
+    nbk::CellTable o = cell_table(c), t = o; t.key = (unsigned long long*)nk.p; t.umis = (unsigned long long*)nu.p; t.reads = (unsigned long long*)nr.p; t.mask = ns - 1;
+    nbk::launch_cells_rehash(o, t, s); c->all_launches++;
+    if (!ck2(cudaStreamSynchronize(s))) return NB_ERR_CUDA;
+    c->d_cellkey.release(); c->d_cellumi.release(); c->d_cellreads.release(); c->d_cellkey = nk; c->d_cellumi = nu; c->d_cellreads = nr; c->cell_slots = ns;
+  }
+  if (n) {
+    CK(c->d_cellscope.ensure(n_scopes * 4 + 16, s)); CK(c->d_cellpid.ensure(n_cs * 4 + 16, s));
+    CK(cudaMemcpyAsync(c->d_cellscope.p, cell_of_scope, n_scopes * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(c->d_cellpid.p, c->pid_of_dense.data(), n_cs * 4, cudaMemcpyHostToDevice, s));
+    const u32* d_scope = (const u32*)c->d_rowout.p; const u32* d_callset = d_scope + n; const i64* d_count = (const i64*)((const char*)c->d_rowout.p + 8 * n);
+    nbk::launch_cells_roll(cell_table(c), d_scope, d_callset, d_count, n, (const u32*)c->d_cellscope.p, (const u32*)c->d_cellpid.p, s); c->all_launches++;
+    u64 ctr[2];
+    CK(cudaMemcpyAsync(ctr, c->d_cellctr.p, 16, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));   // (also: cell_of_scope and pid_of_dense may be reused once this returns)
+    if (ctr[1]) return fail(NB_ERR_OVERFLOW, "per-cell table full");
+    c->cell_used = ctr[0];
+  }
+  c->cell_scopes += n_scopes; c->cells_rows = false; c->cells_rolled = true;
+  return NB_OK;
+}
+
+int nb_cells_finalize(nb_ctx* c, nb_cell_counts* out) {
+  if (!c || !out) return fail(NB_ERR_INVALID, "null argument");
+  CK(cudaSetDevice(c->device));
+  memset(out, 0, sizeof *out);
+  cudaStream_t s = c->stream;
+  const u64 n = c->cell_alloc ? c->cell_used : 0, n_pid = c->pid_off.size() - 1;
+  // persistent ids -> rank in Vec<String> Ord (utils::sort_score_vector): lexicographic on the groups' byte ranks, as finalize_impl
+  const std::vector<u32>& gr = c->lib->group_byte_rank;
+  std::vector<u32> order(n_pid), rank_of_pid(n_pid);
+  for (u64 p = 0; p < n_pid; p++) order[p] = (u32)p;
+  std::sort(order.begin(), order.end(), [&](u32 a, u32 b) {
+    const u32* ia = &c->pid_items[c->pid_off[a]]; const u32* ib = &c->pid_items[c->pid_off[b]];
+    return std::lexicographical_compare(ia, ia + (c->pid_off[a + 1] - c->pid_off[a]), ib, ib + (c->pid_off[b + 1] - c->pid_off[b]), [&](u32 x, u32 y) { return gr[x] < gr[y]; });
+  });
+  for (u64 r = 0; r < n_pid; r++) rank_of_pid[order[r]] = (u32)r;
+  if (c->h_cellrows_cap < n * 24 + 64) { nb_host_free(c->h_cellrows); c->h_cellrows_cap = n * 24 + n * 6 + 4096; c->h_cellrows = (u8*)nb_host_alloc(c->h_cellrows_cap); if (!c->h_cellrows) { c->h_cellrows_cap = 0; return fail(NB_ERR_CUDA, "pinned host allocation failed"); } }
+  u32* h_cell = (u32*)c->h_cellrows; u32* h_callset = h_cell + n; i64* h_umis = (i64*)(h_callset + n); i64* h_reads = h_umis + n;
+  if (n) {
+    const size_t tb = nbk::cells_sort_tmp_bytes(n), work = n * 16 + n * 8 + 64;
+    CK(c->d_cellwork.ensure(work + tb, s)); CK(c->d_cellrows.ensure(n * 24, s)); CK(c->d_cellpid.ensure(n_pid * 4 + 16, s)); CK(c->d_nout.ensure(64, s));
+    CK(cudaMemcpyAsync(c->d_cellpid.p, rank_of_pid.data(), n_pid * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemsetAsync(c->d_nout.p, 0, 8, s));
+    u64* d_keys = (u64*)c->d_cellwork.p; u32* d_slots = (u32*)((char*)c->d_cellwork.p + n * 16); void* d_tmp = (char*)c->d_cellwork.p + work;
+    nbk::launch_cells_finalize(cell_table(c), n, (const u32*)c->d_cellpid.p, d_keys, d_slots, (unsigned long long*)c->d_nout.p, d_tmp, tb, c->d_cellrows.p, s); c->all_launches += 3;
+    CK(cudaMemcpyAsync(c->h_cellrows, c->d_cellrows.p, n * 24, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+  }
+  // callsets without a row (interned in some batch's dictionary, never counted) are left out and the ranks closed up
+  std::vector<u32> used(n_pid, 0);
+  for (u64 i = 0; i < n; i++) used[h_callset[i]] = 1;
+  std::vector<u32> new_id(n_pid, NONE32); u32 k = 0;
+  c->cc_off.assign(1, 0); c->cc_items.clear();
+  for (u64 r = 0; r < n_pid; r++) if (used[r]) {
+    new_id[r] = k++; const u32 p = order[r];
+    c->cc_items.insert(c->cc_items.end(), c->pid_items.begin() + c->pid_off[p], c->pid_items.begin() + c->pid_off[p + 1]); c->cc_off.push_back(c->cc_items.size());
+  }
+  for (u64 i = 0; i < n; i++) h_callset[i] = new_id[h_callset[i]];
+  out->n_rows = n; out->row_cell = h_cell; out->row_callset = h_callset; out->row_umis = h_umis; out->row_reads = h_reads;
+  out->n_callsets = k; out->callset_off = c->cc_off.data(); out->callset_items = c->cc_items.data(); out->n_scopes = c->cell_scopes;
+  return NB_OK;
+}
+
+int nb_cells_reset(nb_ctx* c) {
+  if (!c) return fail(NB_ERR_INVALID, "null argument");
+  CK(cudaSetDevice(c->device));
+  CK(cudaStreamSynchronize(c->stream));
+  for (DBuf* b : {&c->d_cellkey, &c->d_cellumi, &c->d_cellreads}) b->release();
+  c->cell_alloc = false; c->cell_used = 0; c->cell_scopes = 0; c->cells_rows = false;
+  c->cell_pid.clear(); c->pid_off.assign(1, 0); c->pid_items.clear();
   return NB_OK;
 }
 

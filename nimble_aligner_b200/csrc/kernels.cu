@@ -1084,4 +1084,66 @@ void launch_keys_export(const Tables& t, void* records, unsigned long long* n_ou
 }
 void launch_keys_import(const Tables& t, const void* records, u64 n, cudaStream_t s) { if (n) k_keys_import<<<blocks_for(n, 256), 256, 0, s>>>(t, (const KeyRec*)records, n); }
 
+// ------------------------------------------------------------------------------------------------ per-cell table (nb_cells_*)
+// returns the slot of `key`, claiming it when absent (fresh = 1); ~0 when every slot was probed
+__device__ __forceinline__ u64 cell_slot(const CellTable& t, unsigned long long key, u32& fresh) {
+  u64 h = mix64(key) & t.mask;
+  for (u64 probes = 0; probes <= t.mask; probes++) {
+    unsigned long long old = atomicCAS(t.key + h, 0ULL, key);
+    if (old == 0ULL || old == key) { fresh = old == 0ULL; return h; }
+    h = (h + 1) & t.mask;
+  }
+  atomicOr(t.ctr + 1, 1ULL);
+  return ~0ULL;
+}
+// one thread per per-scope row of a finalized scoped batch: umis += 1 (a scope has at most one row per callset), reads += count
+__global__ void __launch_bounds__(256) k_cells_roll(CellTable t, const u32* row_scope, const u32* row_callset, const i64* row_count, u64 n, const u32* cell_of_scope, const u32* pid_of_dense) {
+  u64 i = blockIdx.x * (u64)blockDim.x + threadIdx.x;
+  u32 fresh = 0;
+  if (i < n) {
+    const unsigned long long key = (((unsigned long long)cell_of_scope[row_scope[i]] << 32) | pid_of_dense[row_callset[i]]) + 1ULL;
+    const u64 h = cell_slot(t, key, fresh);
+    if (h != ~0ULL) { atomicAdd(t.umis + h, 1ULL); atomicAdd(t.reads + h, (unsigned long long)row_count[i]); }
+  }
+  const u32 nw = __popc(__ballot_sync(0xFFFFFFFFu, fresh));   // new entries: one atomic per warp
+  if ((threadIdx.x & 31) == 0 && nw) atomicAdd(t.ctr, (unsigned long long)nw);
+}
+__global__ void __launch_bounds__(256) k_cells_rehash(CellTable o, CellTable n) {
+  u64 idx = blockIdx.x * (u64)blockDim.x + threadIdx.x;
+  if (idx > o.mask) return;
+  const unsigned long long k = o.key[idx];
+  if (!k) return;
+  u32 fresh = 0;
+  const u64 h = cell_slot(n, k, fresh);
+  if (h != ~0ULL) { n.umis[h] = o.umis[idx]; n.reads[h] = o.reads[idx]; }
+}
+__global__ void __launch_bounds__(256) k_cells_compact(CellTable t, const u32* rank_of_pid, u64* keys, u32* slots, u64 cap, unsigned long long* n_out) {
+  u64 idx = blockIdx.x * (u64)blockDim.x + threadIdx.x;
+  if (idx > t.mask) return;
+  const unsigned long long k = t.key[idx];
+  if (!k) return;
+  const unsigned long long at = atomicAdd(n_out, 1ULL);
+  if (at >= cap) return;
+  const u64 ck = k - 1;
+  keys[at] = (ck & 0xFFFFFFFF00000000ULL) | rank_of_pid[(u32)ck]; slots[at] = (u32)idx;
+}
+__global__ void __launch_bounds__(256) k_cells_split(CellTable t, const u64* keys, const u32* slots, u64 n, u32* cell, u32* callset, i64* umis, i64* reads) {
+  u64 i = blockIdx.x * (u64)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const u64 k = keys[i]; const u32 sl = slots[i];
+  cell[i] = (u32)(k >> 32); callset[i] = (u32)k; umis[i] = (i64)t.umis[sl]; reads[i] = (i64)t.reads[sl];
+}
+void launch_cells_roll(const CellTable& t, const u32* row_scope, const u32* row_callset, const i64* row_count, u64 n_rows, const u32* cell_of_scope, const u32* pid_of_dense, cudaStream_t s) {
+  if (n_rows) k_cells_roll<<<blocks_for(n_rows, 256), 256, 0, s>>>(t, row_scope, row_callset, row_count, n_rows, cell_of_scope, pid_of_dense);
+}
+void launch_cells_rehash(const CellTable& o, const CellTable& n, cudaStream_t s) { k_cells_rehash<<<blocks_for(o.mask + 1, 256), 256, 0, s>>>(o, n); }
+size_t cells_sort_tmp_bytes(u64 n) { size_t tb = 0; cub::DeviceRadixSort::SortPairs(nullptr, tb, (const u64*)nullptr, (u64*)nullptr, (const u32*)nullptr, (u32*)nullptr, (int)n, 0, 64); return tb + 256; }
+void launch_cells_finalize(const CellTable& t, u64 n, const u32* rank_of_pid, u64* keys, u32* slots, unsigned long long* n_out, void* tmp, size_t tmp_bytes, void* out, cudaStream_t s) {
+  if (!n) return;
+  k_cells_compact<<<blocks_for(t.mask + 1, 256), 256, 0, s>>>(t, rank_of_pid, keys, slots, n, n_out);
+  cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, (const u64*)keys, keys + n, (const u32*)slots, slots + n, (int)n, 0, 64, s);
+  u32* cell = (u32*)out; u32* callset = cell + n; i64* umis = (i64*)(callset + n); i64* reads = umis + n;
+  k_cells_split<<<blocks_for(n, 256), 256, 0, s>>>(t, keys + n, slots + n, n, cell, callset, umis, reads);
+}
+
 }  // namespace nbk

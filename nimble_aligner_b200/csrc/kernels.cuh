@@ -131,6 +131,17 @@ void launch_keys_scatter(const Tables& t, void* rec, unsigned long long* cursors
 void launch_callsets_import(const Tables& t, const u32* rows, u64 n, cudaStream_t s);
 void launch_keys_import(const Tables& t, const void* records, u64 n, cudaStream_t s);
 
+// per-cell table of the BAM driver (engine.cu nb_cells_*): open addressing on key (cell << 32 | persistent callset id) + 1
+// with two counters per entry; it outlives nb_counts_reset, and the host grows it (rehash) before a roll could fill it past half.
+// ctr[0] = occupied entries, ctr[1] = error bit (a probe ran through the whole table: cannot happen below half full)
+struct CellTable { unsigned long long* key; unsigned long long* umis; unsigned long long* reads; u64 mask; unsigned long long* ctr; };
+void launch_cells_roll(const CellTable& t, const u32* row_scope, const u32* row_callset, const i64* row_count, u64 n_rows, const u32* cell_of_scope, const u32* pid_of_dense, cudaStream_t s);
+void launch_cells_rehash(const CellTable& o, const CellTable& n, cudaStream_t s);
+size_t cells_sort_tmp_bytes(u64 n);
+// occupied entries -> rows sorted by (cell, rank_of_pid[pid]): out = row_cell u32[n] | row_callset u32[n] | umis i64[n] | reads i64[n];
+// work: 2n u64 keys + 2n u32 slots + tmp
+void launch_cells_finalize(const CellTable& t, u64 n, const u32* rank_of_pid, u64* keys, u32* slots, unsigned long long* n_out, void* tmp, size_t tmp_bytes, void* out, cudaStream_t s);
+
 // multi-GPU merge (engine.cu nb_merge_*): exchange blocks whose sizes the kernels read from the gathered headers on the device
 constexpr u32 MERGE_HDR1_WORDS = 1 + ROUTE_MAX;
 void launch_merge_hdr1(u64* hdr, const unsigned long long* n_rows, const unsigned long long* route_cursor, u32 world, cudaStream_t s);

@@ -12,7 +12,7 @@
 static void die(const std::string& m) { fprintf(stderr, "%s\n", m.c_str()); exit(101); }  // a Rust panic exits 101
 
 int main(int argc, char** argv) {
-  std::vector<std::string> refs, outs, ins; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
+  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
   std::vector<std::string>* cur = nullptr;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
@@ -26,12 +26,25 @@ int main(int argc, char** argv) {
     if (a == "-p" || a == "--force_bam_paired") { force_paired = true; cur = nullptr; continue; }
     if (a == "-d" || a == "--devices") { devs = val("--devices"); cur = nullptr; continue; }   // not in cli.yml: which GPUs to use, "0,1,..." (default: NB_DEVICES or 0)
     if (a == "--index-cache") { const std::string dir = val("--index-cache"); setenv("NB_INDEX_CACHE", dir.c_str(), 1); cur = nullptr; continue; }   // not in cli.yml: keep each library's index in <dir>/<key>.nbix (default: NB_INDEX_CACHE, else rebuilt per run like the reference)
-    if (a == "-h" || a == "--help") { printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"); return 0; }
+    if (a == "--cell-matrix") { cur = &mats; have_mats = true; continue; }   // not in cli.yml: BAM mode, one directory per -r for a cell x feature matrix (10x v3 layout)
+    if (a == "--no-rows") { no_rows = true; cur = nullptr; continue; }          // not in cli.yml: BAM mode, no TSV.gz rows (with --cell-matrix, without -o)
+    if (a == "-h" || a == "--help") {
+      printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"
+             "  -d, --devices <list>          GPUs to use, \"0,1,...\" (default: NB_DEVICES, else 0)\n"
+             "      --index-cache <dir>       keep each library's index in <dir> (default: NB_INDEX_CACHE)\n"
+             "      --cell-matrix <dir>...    BAM input: also write a cell x feature matrix per reference library into <dir>\n"
+             "                                (matrix.mtx.gz UMIs, reads.mtx.gz reads, features.tsv.gz, barcodes.tsv.gz)\n"
+             "      --no-rows                 BAM input with --cell-matrix: skip the TSV.gz rows (no --output)\n");
+      return 0;
+    }
     if (a == "-V" || a == "--version") { printf("nimble 0.8.0\n"); return 0; }
     if (!cur) die("error: Found argument '" + a + "' which wasn't expected, or isn't valid in this context");
     cur->push_back(a);
   }
-  if (refs.empty() || outs.empty() || ins.empty()) die("error: The following required arguments were not provided: --reference/--output/--input");
+  if (no_rows && !outs.empty()) die("error: --no-rows writes no TSV: leave out --output");
+  if (no_rows && !have_mats) die("error: --no-rows needs --cell-matrix (there would be nothing to write)");
+  if (have_mats && mats.size() != refs.size()) die("error: --cell-matrix needs one directory per reference library");
+  if (refs.empty() || (outs.empty() && !no_rows) || ins.empty()) die("error: The following required arguments were not provided: --reference/--output/--input");
   char* end = nullptr; long ncores = strtol(cores.c_str(), &end, 10);
   if (*end || ncores < 0) die("Error -- please provide an integer value for the number of cores");
   int chem;
@@ -50,15 +63,17 @@ int main(int argc, char** argv) {
   for (auto& s : refs) { printf("Loading and preprocessing reference data for %s\n", s.c_str()); r.push_back(s.c_str()); }
   for (auto& s : outs) o.push_back(s.c_str());
   for (auto& s : ins) in.push_back(s.c_str());
-  if (outs.size() < refs.size()) die("index out of bounds: one output path per reference library is required");
+  if (!no_rows && outs.size() < refs.size()) die("index out of bounds: one output path per reference library is required");
   printf("Loading read sequences and aligning\n");
+  std::vector<const char*> m; for (auto& s : mats) m.push_back(s.c_str());
   if (ends(first, ".fastq.gz") || ends(lower, ".fastq")) {
+    if (have_mats || no_rows) die("error: --cell-matrix and --no-rows need a BAM input (FASTQ reads have no cells)");
     printf("Processing as FASTQ file\n");
     int rc = nb_process_fastq_devices(in.data(), (uint32_t)std::min<size_t>(in.size(), 2), r.data(), o.data(), (uint32_t)r.size(), chem, (int)ncores, devices.data(), (uint32_t)devices.size());
     if (rc != NB_OK) die(nb_last_error());
   } else if (ends(lower, ".bam")) {
     printf("Processing as BAM file\n");
-    int rc = nb_process_bam(in[0], r.data(), o.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
+    int rc = nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
     if (rc != NB_OK) die(nb_last_error());
   } else die("Unsupported file format: " + (lower.find('.') == std::string::npos ? std::string("") : lower.substr(lower.rfind('.') + 1)));
   printf("Alignment successful, terminating.\n");
