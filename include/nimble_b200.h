@@ -245,7 +245,9 @@ int nb_cells_reset(nb_ctx*);
  * callset_tag}; dev_records are device pointers; nb_keys_export_partitioned groups them by owning rank (a 16-bit slice of
  * key_lo mod world) so no sort is needed.  Callset dictionaries travel as rows of (4 + gcap) uint32:
  * {slot, len, tag_lo, tag_hi, items[gcap]}; after importing the union every rank's nb_counts lists the same callsets in
- * the same order, so the final merge is one all-reduce(sum) over a dense count vector. */
+ * the same order, so the final merge is one all-reduce(sum) over a dense count vector.  Both exports fail with
+ * NB_ERR_INVALID when cap is below the record count; nb_keys_import fails with NB_ERR_INVALID when a record's callset
+ * tag is not in this context's dictionary (import the peers' rows first). */
 int nb_keys_export_count(nb_ctx*, uint64_t* n);
 int nb_keys_export(nb_ctx*, void* dev_records, uint64_t cap, uint64_t pair_index_base);
 int nb_keys_import(nb_ctx*, const void* dev_records, uint64_t n);

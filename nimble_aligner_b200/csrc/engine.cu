@@ -194,6 +194,7 @@ static int check_device_errors(nb_ctx* c, Counters* out = nullptr) {
   if (h.err & nbk::E_KEY_FULL) return fail(NB_ERR_OVERFLOW, "read-key table full: raise option key_slots");
   if (h.err & nbk::E_AGG_FULL) return fail(NB_ERR_OVERFLOW, "count table full: raise option agg_slots");
   if (h.err & nbk::E_INBOX_FULL) return fail(NB_ERR_OVERFLOW, "routing inbox region full: create the routes with more records_per_peer");
+  if (h.err & nbk::E_CS_UNKNOWN) return fail(NB_ERR_INVALID, "key record names a callset this rank was never given: import the peers' dictionaries (nb_callsets_import) before their key records");
   return NB_OK;
 }
 
@@ -883,7 +884,9 @@ int nb_keys_export(nb_ctx* c, void* dev_records, uint64_t cap, uint64_t pair_ind
   CK(cudaSetDevice(c->device));
   CK(cudaMemsetAsync(c->d_nout.p, 0, 8, c->stream));
   nbk::launch_keys_export(make_tables(c), dev_records, (unsigned long long*)c->d_nout.p, cap, pair_index_base, c->stream); c->all_launches++;
-  CK(cudaStreamSynchronize(c->stream));
+  u64 n = 0;
+  CK(cudaMemcpyAsync(&n, c->d_nout.p, 8, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
+  if (n > cap) return fail(NB_ERR_INVALID, "record buffer too small for nb_keys_export (nb_keys_export_count gives the size)");
   return NB_OK;
 }
 // key records grouped by owning rank: counts_out[world] entries per owner, records of owner o start at sum(counts[0..o))

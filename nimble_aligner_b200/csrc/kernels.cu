@@ -765,7 +765,7 @@ __global__ void __launch_bounds__(256) k_keys_export(Tables t, KeyRec* rec, unsi
   u64 v = t.kval[idx]; u32 cs = (u32)(v & 0xFFFFFFu);
   unsigned long long at = atomicAdd(n_out, 1ULL);
   if (at >= cap) return;
-  KeyRec r; r.k0 = k.x; r.k1 = k.y; r.order = (v >> 24) - 1 + order_base; r.tag = cs == CS_NONE ? 0ULL : t.cs_tag[cs];
+  KeyRec r; r.k0 = k.x; r.k1 = k.y; r.order = (v >> 24) - 1 + order_base; r.tag = ((v >> 24) == 0 || cs == CS_NONE) ? 0ULL : t.cs_tag[cs];   // as k_keys_scatter
   rec[at] = r;
 }
 // import records from other ranks: the tag must already be present in this rank's dictionary (the host merges
@@ -863,7 +863,7 @@ __device__ __forceinline__ u32 key_import_rec(const Tables& t, const KeyRec& r) 
   if (r.tag) {
     u32 h = (u32)(r.tag >> 24) & t.cs_mask; bool ok = false;
     for (u32 probes = 0; probes <= t.cs_mask; probes++) { u64 tg = t.cs_tag[h]; if (tg == r.tag) { ok = true; break; } if (tg == 0) break; h = (h + 1) & t.cs_mask; }
-    if (!ok) { atomicOr(&t.ctr->err, (unsigned)E_CS_FULL); return 0u; }
+    if (!ok) { atomicOr(&t.ctr->err, (unsigned)E_CS_UNKNOWN); return 0u; }
     cs = h;
   }
   bool fresh;

@@ -54,7 +54,7 @@ struct DevCfg {
   u32 discard_multi_hits, max_hits, gcap, min_read_len;
 };
 // device-side error bits (Counters::err)
-enum { E_ARENA = 1, E_CS_FULL = 2, E_KEY_FULL = 4, E_FEATURE = 8, E_AGG_FULL = 16, E_GCAP = 32, E_INBOX_FULL = 64 };
+enum { E_ARENA = 1, E_CS_FULL = 2, E_KEY_FULL = 4, E_FEATURE = 8, E_AGG_FULL = 16, E_GCAP = 32, E_INBOX_FULL = 64, E_CS_UNKNOWN = 128 };
 struct Counters {
   unsigned long long arena_top, queue, seeded_n, wqueue;   // all four zeroed before every map launch (seeded_n / wqueue: k_seed -> k_walk list)
   unsigned long long n_keys; unsigned long long n_callsets; unsigned long long n_agg;

@@ -110,8 +110,8 @@ def merge_across_ranks(shard, torch, dist, rank, world, device, routed=False):
         # after which every peer's last k_pair — and with it every record bound for this rank's inbox — is complete.
         sent = np.asarray(shard.route_sent(), dtype=np.int64)
         hdr = 1 + 2 * world          # k, then sent[] as (lo, hi) int32 halves
+        cap = _ROUTED_CAP[0]
         while True:
-            cap = _ROUTED_CAP[0]
             head = np.zeros(hdr, dtype=np.int32)
             head[0] = k
             head[1:] = sent.astype(np.int64).view(np.int32)
@@ -125,8 +125,11 @@ def merge_across_ranks(shard, torch, dist, rank, world, device, routed=False):
             szs = hb[:, 0].tolist()
             if max(szs) <= cap:
                 break
-            while _ROUTED_CAP[0] < max(szs):
-                _ROUTED_CAP[0] *= 2
+            while cap < max(szs):
+                cap *= 2
+            # raised from this rank's own copy and stored once: ranks that share the module (threads of one process) all
+            # read the same start value before the gather, so each computes, and stores, the same capacity
+            _ROUTED_CAP[0] = cap
         recv = np.ascontiguousarray(hb[:, 1:hdr]).view(np.int64)[:, rank].copy()   # records rank r stored into this rank's inbox
         if on_dev:   # the peers' rows are imported straight out of the all_gather buffer in HBM
             for r in range(world):
@@ -252,14 +255,19 @@ def merge_scoped_across_ranks(shard, torch, dist, rank, world, device, n_cells):
         if stats:
             print("scoped merge: " + ", ".join("%s %.2f ms" % (marks[i][0], (marks[i][1] - marks[i - 1][1]) * 1e3) for i in range(1, len(marks))), file=sys.stderr)
         return raw, out[0], out[1], out[2]
-    cell = np.asarray(raw["row_scope"], dtype=np.int64); cs = np.asarray(raw["row_callset"], dtype=np.int64); cnt = np.asarray(raw["row_count"], dtype=np.int64)
+    dev = shard.device_rows() if device != "cpu" and hasattr(shard, "device_rows") else None
+    if dev is not None:   # a device shard's finalize returns no host rows: they are still on the device
+        mine = torch.stack([dev[0].to(torch.int64), dev[1].to(torch.int64), dev[2]], dim=1)
+    else:
+        cell = np.asarray(raw["row_scope"], dtype=np.int64); cs = np.asarray(raw["row_callset"], dtype=np.int64); cnt = np.asarray(raw["row_count"], dtype=np.int64)
+        mine = torch.from_numpy(np.stack([cell, cs, cnt], axis=1)).to(device)
     n = torch.zeros(world, dtype=torch.int64, device=device)
-    n[rank] = len(cnt)
+    n[rank] = mine.shape[0]
     dist.all_reduce(n)
     ns = n.cpu().tolist(); nmax = max(max(ns), 1)
     tri = torch.zeros((nmax, 3), dtype=torch.int64, device=device)
-    if len(cnt):
-        tri[: len(cnt)] = torch.from_numpy(np.stack([cell, cs, cnt], axis=1)).to(device)
+    if mine.shape[0]:
+        tri[: mine.shape[0]] = mine
     alltri = torch.empty((world, nmax, 3), dtype=torch.int64, device=device)
     dist.all_gather_into_tensor(alltri.view(-1), tri.view(-1))
     t = torch.cat([alltri[r, : int(ns[r])] for r in range(world)]).cpu().numpy()
