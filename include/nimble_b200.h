@@ -369,6 +369,30 @@ int nb_process_bam(const char* input_file, const char* const* reference_json, co
 int nb_process_bam_cells(const char* input_file, const char* const* reference_json, const char* const* output_paths,
                          const char* const* matrix_dirs, uint32_t n_refs, int strand_filter, const char* trim, int num_cores,
                          int force_bam_paired, int device);
+/* The per-cell matrices of nb_process_bam_cells (no TSV rows) from a BAM in ANY record order, e.g. Cell Ranger's
+ * position-sorted possorted_genome_bam.bam: scopes come from the records' tags, not from the file order.  With ordinals
+ * 0..n-1 in file order:
+ *   1. kept records are filtered as SortedBamReader::fill_buffer does: no CB string aux -> skipped; UMI = UB, else UR, and a
+ *      CB without either fails with NB_ERR_PARSE "Error -- Could not read UMI."; UMI AAAAAAAAAA -> skipped
+ *   2. kept records are ordered by (UMI, full CB, ordinal) (byte order), on the GPU
+ *   3. a scope is a maximal run in that order with equal (UMI, CB[..len-2]), compared as a pair
+ *   4. each scope's records go through add_dummy_paired_reads and filter_paired_reads (src/parse/sorted_bam_reader.rs:109-162;
+ *      names compared exactly); TSO clip, REVERSE and quals as in nb_process_bam
+ *   5. the cell of a scope is the full CB of its first record; every scope is aligned (no "last group" is dropped)
+ *   6. the barcodes are the cells of the scopes that have pairs, in order of the first kept record (by ordinal) with that CB
+ * So the matrix equals nb_process_bam_cells (rows NULL) on the file G = the kept records in the order of step 2 followed by
+ * one scope with a UMI no record has: same features, barcode set and (feature, barcode) counts; only the barcode order differs.
+ * Every kept record's nibbles, quals and name stay in device memory (the store; NB_BAM_STATS=1 prints its size) and the
+ * scoped batches point into it.  Refused: a kept record with an empty UMI string, or a UMI that the exact device key cannot
+ * hold (more than 21 characters, or a character outside ACGTN): NB_ERR_UNSUPPORTED naming it; a store that does not fit:
+ * NB_ERR_CUDA with the bytes needed.  There is no force_bam_paired (mates of a position-sorted file are not neighbours) and
+ * no TSV rows (they need every record's 38 fields on the host). */
+int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                   int strand_filter, const char* trim, int num_cores, int device);
+/* test hook: the device grouping of nb_process_bam_cells_any_order, one line per pair:
+ * scope index (counting the scopes with pairs, in sorted order) TAB cell barcode TAB sequence-slot ordinal TAB mate-slot ordinal
+ * TAB flags (NB_FLAG_*) of both slots TAB clipped lengths of both slots */
+int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path);
 /* host-only: a cell x feature matrix in the 10x v3 layout that Seurat's Read10X and scanpy's read_10x_mtx load, into `dir`
  * (created when missing; its parent must exist): matrix.mtx.gz (Matrix Market coordinate integer, features x barcodes, UMI
  * counts, 1-based lines sorted by barcode then feature), reads.mtx.gz (the same coordinates with the read counts),

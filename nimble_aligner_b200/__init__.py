@@ -150,6 +150,8 @@ _SIGS = {
     "nb_process_fastq_devices": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_void_p, C.c_uint32]),
     "nb_process_bam": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]),
     "nb_process_bam_cells": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]),
+    "nb_process_bam_cells_any_order": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int]),
+    "nb_bam_dump_scopes_any_order": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_char_p]),
     "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
     "nb_cells_reset": (C.c_int, [C.c_void_p]),
@@ -666,10 +668,21 @@ def fastq_dump(input_files, out_path, num_cores=1, chunk_bytes=0):
 
 
 def process_bam(input_file, reference_json_paths, output_paths, strand_filter="unstranded", trim=None, num_cores=1, force_bam_paired=False, device=0,
-                matrix_dirs=None):
+                matrix_dirs=None, any_order=False):
     """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156).
     matrix_dirs=[dir per library]: also a cell x feature matrix per library (nb_process_bam_cells); output_paths=None with
-    matrix_dirs: no TSV rows at all."""
+    matrix_dirs: no TSV rows at all.  any_order=True: the matrices only (output_paths=None, matrix_dirs required, no
+    force_bam_paired) from a BAM in any record order, scopes formed on the GPU (nb_process_bam_cells_any_order)."""
+    if any_order:
+        if output_paths is not None:
+            raise NbError(-1, "any_order writes no TSV rows: pass output_paths=None")
+        if matrix_dirs is None:
+            raise NbError(-1, "any_order needs matrix_dirs")
+        if force_bam_paired:
+            raise NbError(-1, "any_order cannot pair mates (force_bam_paired): the mates of a position-sorted file are not neighbours")
+        _ck(lib().nb_process_bam_cells_any_order(str(input_file).encode(), _strs(reference_json_paths), _strs(matrix_dirs), len(reference_json_paths),
+                                                 CHEM[strand_filter], trim.encode() if trim else None, num_cores, device))
+        return
     if matrix_dirs is not None or output_paths is None:
         _ck(lib().nb_process_bam_cells(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths) if output_paths is not None else None,
                                        _strs(matrix_dirs) if matrix_dirs is not None else None, len(reference_json_paths),
@@ -730,3 +743,8 @@ def gzip_fast(data):
 
 def bam_dump_groups(input_file, out_path, force_bam_paired=False, num_cores=1):
     _ck(lib().nb_bam_dump_groups(str(input_file).encode(), int(force_bam_paired), num_cores, str(out_path).encode()))
+
+
+def bam_dump_scopes_any_order(input_file, out_path, num_cores=1, device=0):
+    """The device grouping of process_bam(any_order=True), one line per pair (nb_bam_dump_scopes_any_order)."""
+    _ck(lib().nb_bam_dump_scopes_any_order(str(input_file).encode(), num_cores, device, str(out_path).encode()))

@@ -8,7 +8,7 @@ CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libnimble_b200.so")
 AR = os.path.join(HERE, "libnimble_b200.a")   # the static library north_star names: same objects, for a host that links it in (INTEGRATION.md)
 CLI = os.path.join(HERE, "nimble")
-SOURCES = ["library.cpp", "index_build.cpp", "fastq.cpp", "bam.cpp", "kernels.cu", "engine.cu", "index_build_gpu.cu", "roofs.cu"]
+SOURCES = ["library.cpp", "index_build.cpp", "fastq.cpp", "bam.cpp", "bam_group.cu", "kernels.cu", "engine.cu", "index_build_gpu.cu", "roofs.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-extended-lambda",
          "-Xcompiler", "-fPIC,-pthread,-Wall,-Wno-unused-function", "-cudart", "shared"]
@@ -23,7 +23,7 @@ def _stale(target, deps):
 
 def build(force=False, verbose=False):
     srcs = [os.path.join(CSRC, s) for s in SOURCES]
-    deps = srcs + [os.path.join(CSRC, h) for h in ("host.hpp", "kernels.cuh", "khash.h", "kmap.cuh", "inflate.hpp", "pgunzip.hpp", "deflate_fast.hpp")] + [os.path.join(HERE, "..", "include", "nimble_b200.h")]
+    deps = srcs + [os.path.join(CSRC, h) for h in ("host.hpp", "kernels.cuh", "khash.h", "kmap.cuh", "inflate.hpp", "pgunzip.hpp", "deflate_fast.hpp", "bam_group.hpp")] + [os.path.join(HERE, "..", "include", "nimble_b200.h")]
     if force or _stale(SO, deps):
         objs = []
         for s in srcs:

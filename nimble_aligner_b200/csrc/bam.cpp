@@ -26,6 +26,7 @@
 #include <future>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include <errno.h>
@@ -34,6 +35,7 @@
 #include "host.hpp"
 #include "inflate.hpp"
 #include "deflate_fast.hpp"
+#include "bam_group.hpp"
 
 using namespace nb;
 typedef int32_t i32;
@@ -386,6 +388,73 @@ inline bool key_equal(const Rec& a, const Rec& b) {
   std::string x(a.umi, a.umi_len), y(b.umi, b.umi_len); x.append(a.cb, ca); y.append(b.cb, cb); return x == y;   // different split of the same concatenation
 }
 
+// The complete records of d[cur, len) in file order (tail = first byte that is not part of one; a record cut by the end of the
+// window is left for the next window).  eof: d holds the end of the file.
+int walk_records(const RawBuf& d, size_t len, size_t cur, bool eof, int threads, std::vector<Rec>& all, size_t& tail) {
+  all.clear();
+  const size_t walk_from = cur;
+  // complete records of the window.  The records form a chain (each block_size leads to the next record), and walking it
+  // serially was a quarter of the producer's critical path, every step a cache miss on data another core just inflated.
+  // So the window is cut into segments walked at the same time: a segment starts at a GUESSED record start (the first
+  // offset behind its boundary from which four consecutive records look sound) and the guess is never trusted — the
+  // segments are only accepted if each one begins exactly where the previous one's walk ended, else the serial walk runs.
+  auto sound = [&](size_t o, size_t& next) -> bool {   // does a complete, self-consistent record start at o?
+    if (o + 36 > len) return false;
+    u32 bs; memcpy(&bs, &d[o], 4);
+    if (bs < 32 || bs > (1u << 24) || o + 4 + bs > len) return false;
+    const u8* q = &d[o + 4]; const u32 lrn = q[8], ncig = q[12] | (q[13] << 8); u32 lseq; memcpy(&lseq, q + 16, 4);
+    i32 refid; memcpy(&refid, q, 4);
+    if (lrn == 0 || refid < -1 || 32ull + lrn + 4ull * ncig + ((u64)lseq + 1) / 2 + (u64)lseq > bs || q[32 + lrn - 1] != 0) return false;
+    next = o + 4 + bs; return true;
+  };
+  bool walked = false;
+  const size_t par_min_bytes = getenv("NB_BAM_PAR_MIN_BYTES") ? (size_t)strtoull(getenv("NB_BAM_PAR_MIN_BYTES"), nullptr, 10) : ((size_t)8 << 20);   // (tests force the parallel passes on small files)
+  const int WT = (len - cur > par_min_bytes) ? threads : 1;
+  if (WT > 1) {
+    std::vector<std::vector<Rec>> part(WT); std::vector<size_t> seg_start(WT, 0), seg_end(WT, 0); std::vector<char> ok(WT, 1);
+    const size_t span = len - walk_from;
+    parallel_ranges(WT, (size_t)WT, [&](size_t ta, size_t tb, int) {
+      for (size_t t = ta; t < tb; t++) {
+        const size_t lo = walk_from + span * t / WT, hi = walk_from + span * (t + 1) / WT;   // records STARTING in [lo, hi) belong to segment t
+        size_t o = lo;
+        if (t > 0) {   // guess: first offset >= lo that begins a chain of four sound records (or runs into the window's end)
+          bool found = false;
+          for (; o < hi && o < lo + ((size_t)1 << 20); o++) { size_t n1 = o, n2; int k = 0; while (k < 4 && sound(n1, n2)) { n1 = n2; k++; } if (k == 4 || (k > 0 && n1 + 4 > len)) { found = true; break; } }
+          if (!found) { ok[t] = 0; continue; }
+        }
+        seg_start[t] = o;
+        std::vector<Rec>& out = part[t]; out.reserve((hi - lo) / 160 + 16);
+        while (o < hi) { size_t nx; if (!sound(o, nx)) break; Rec r; r.p = &d[o + 4]; r.block = (u32)(nx - o - 4); out.push_back(r); o = nx; }
+        seg_end[t] = o;     // first offset this segment did not consume: a record start >= hi, the cut record, or something unsound
+      }
+    });
+    bool good = true;
+    for (int t = 0; t < WT && good; t++) good = ok[t] && (t == 0 || seg_start[t] == seg_end[t - 1]);
+    if (good) {
+      // the last segment's end must be where the serial walk would stop: at a record the window cuts (or at the window's end)
+      const size_t e = seg_end[WT - 1]; u32 bs = 0; if (e + 4 <= len) memcpy(&bs, &d[e], 4);
+      good = e + 4 > len || (bs >= 32 && e + 4 + bs > len);
+      if (good) {
+        size_t total = 0; std::vector<size_t> at(WT + 1, 0); for (int t = 0; t < WT; t++) { at[t] = total; total += part[t].size(); }
+        all.resize(total);
+        parallel_ranges(WT, (size_t)WT, [&](size_t ta, size_t tb, int) { for (size_t t = ta; t < tb; t++) if (!part[t].empty()) memcpy(&all[at[t]], part[t].data(), part[t].size() * sizeof(Rec)); });
+        cur = e; walked = true;
+      }
+    }
+  }
+  while (!walked && cur + 4 <= len) {
+    u32 bs; memcpy(&bs, &d[cur], 4);
+    if (bs < 32) { if (!eof) return fail(NB_ERR_PARSE, "corrupt BAM record (block size below the fixed fields)"); break; }   // (trailing garbage at the very end is ignored, as before)
+    if (cur + 4 + bs > len) break;                                                        // cut by the window: carried over
+    Rec r; r.p = &d[cur + 4]; r.block = bs;
+    // l_read_name, n_cigar and l_seq come from the file: qname / cigar / 4-bit bases / quals must lie inside the record
+    if (32ull + r.l_read_name() + 4ull * r.n_cigar() + ((u64)r.l_seq() + 1) / 2 + (u64)r.l_seq() > bs) return fail(NB_ERR_PARSE, "corrupt BAM record (field lengths exceed its block size)");
+    all.push_back(r); cur += 4 + bs;
+  }
+  tail = cur;
+  return NB_OK;
+}
+
 // ------------------------------------------------------------------ windowed producer
 // The same stream and groups as collect_groups_serial, computed window by window on `threads` threads with bounded memory.
 // The serial readers above define the semantics; this restates them over whole runs: a SortedBamReader buffer is a maximal
@@ -438,68 +507,11 @@ struct GroupStreamer {
         if (!ok) { if (eof) return fail(NB_ERR_PARSE, w.len < 12 ? "not a BAM file" : "truncated BAM header"); grow *= 2; continue; }
         cur = p;
       }
-      // complete records of the window.  The records form a chain (each block_size leads to the next record), and walking it
-      // serially was a quarter of the producer's critical path, every step a cache miss on data another core just inflated.
-      // So the window is cut into segments walked at the same time: a segment starts at a GUESSED record start (the first
-      // offset behind its boundary from which four consecutive records look sound) and the guess is never trusted — the
-      // segments are only accepted if each one begins exactly where the previous one's walk ended, else the serial walk runs.
-      w.all.clear();
+      size_t cur_end = cur;
+      { int rw = walk_records(w.data, w.len, cur, eof, threads, w.all, cur_end); if (rw) return rw; }
+      cur = cur_end;
       const RawBuf& d = w.data;
-      const size_t walk_from = cur;
-      auto sound = [&](size_t o, size_t& next) -> bool {   // does a complete, self-consistent record start at o?
-        if (o + 36 > w.len) return false;
-        u32 bs; memcpy(&bs, &d[o], 4);
-        if (bs < 32 || bs > (1u << 24) || o + 4 + bs > w.len) return false;
-        const u8* q = &d[o + 4]; const u32 lrn = q[8], ncig = q[12] | (q[13] << 8); u32 lseq; memcpy(&lseq, q + 16, 4);
-        i32 refid; memcpy(&refid, q, 4);
-        if (lrn == 0 || refid < -1 || 32ull + lrn + 4ull * ncig + ((u64)lseq + 1) / 2 + (u64)lseq > bs || q[32 + lrn - 1] != 0) return false;
-        next = o + 4 + bs; return true;
-      };
-      bool walked = false;
-      const size_t par_min_bytes = getenv("NB_BAM_PAR_MIN_BYTES") ? (size_t)strtoull(getenv("NB_BAM_PAR_MIN_BYTES"), nullptr, 10) : ((size_t)8 << 20);   // (tests force the parallel passes on small files)
       const size_t par_min_recs = getenv("NB_BAM_PAR_MIN_RECS") ? (size_t)strtoull(getenv("NB_BAM_PAR_MIN_RECS"), nullptr, 10) : 65536;
-      const int WT = (w.len - cur > par_min_bytes) ? threads : 1;
-      if (WT > 1) {
-        std::vector<std::vector<Rec>> part(WT); std::vector<size_t> seg_start(WT, 0), seg_end(WT, 0); std::vector<char> ok(WT, 1);
-        const size_t span = w.len - walk_from;
-        parallel_ranges(WT, (size_t)WT, [&](size_t ta, size_t tb, int) {
-          for (size_t t = ta; t < tb; t++) {
-            const size_t lo = walk_from + span * t / WT, hi = walk_from + span * (t + 1) / WT;   // records STARTING in [lo, hi) belong to segment t
-            size_t o = lo;
-            if (t > 0) {   // guess: first offset >= lo that begins a chain of four sound records (or runs into the window's end)
-              bool found = false;
-              for (; o < hi && o < lo + ((size_t)1 << 20); o++) { size_t n1 = o, n2; int k = 0; while (k < 4 && sound(n1, n2)) { n1 = n2; k++; } if (k == 4 || (k > 0 && n1 + 4 > w.len)) { found = true; break; } }
-              if (!found) { ok[t] = 0; continue; }
-            }
-            seg_start[t] = o;
-            std::vector<Rec>& out = part[t]; out.reserve((hi - lo) / 160 + 16);
-            while (o < hi) { size_t nx; if (!sound(o, nx)) break; Rec r; r.p = &d[o + 4]; r.block = (u32)(nx - o - 4); out.push_back(r); o = nx; }
-            seg_end[t] = o;     // first offset this segment did not consume: a record start >= hi, the cut record, or something unsound
-          }
-        });
-        bool good = true;
-        for (int t = 0; t < WT && good; t++) good = ok[t] && (t == 0 || seg_start[t] == seg_end[t - 1]);
-        if (good) {
-          // the last segment's end must be where the serial walk would stop: at a record the window cuts (or at the window's end)
-          const size_t e = seg_end[WT - 1]; u32 bs = 0; if (e + 4 <= w.len) memcpy(&bs, &d[e], 4);
-          good = e + 4 > w.len || (bs >= 32 && e + 4 + bs > w.len);
-          if (good) {
-            size_t total = 0; std::vector<size_t> at(WT + 1, 0); for (int t = 0; t < WT; t++) { at[t] = total; total += part[t].size(); }
-            w.all.resize(total);
-            parallel_ranges(WT, (size_t)WT, [&](size_t ta, size_t tb, int) { for (size_t t = ta; t < tb; t++) if (!part[t].empty()) memcpy(&w.all[at[t]], part[t].data(), part[t].size() * sizeof(Rec)); });
-            cur = e; walked = true;
-          }
-        }
-      }
-      while (!walked && cur + 4 <= w.len) {
-        u32 bs; memcpy(&bs, &d[cur], 4);
-        if (bs < 32) { if (!eof) return fail(NB_ERR_PARSE, "corrupt BAM record (block size below the fixed fields)"); break; }   // (trailing garbage at the very end is ignored, as before)
-        if (cur + 4 + bs > w.len) break;                                                        // cut by the window: carried over
-        Rec r; r.p = &d[cur + 4]; r.block = bs;
-        // l_read_name, n_cigar and l_seq come from the file: qname / cigar / 4-bit bases / quals must lie inside the record
-        if (32ull + r.l_read_name() + 4ull * r.n_cigar() + ((u64)r.l_seq() + 1) / 2 + (u64)r.l_seq() > bs) return fail(NB_ERR_PARSE, "corrupt BAM record (field lengths exceed its block size)");
-        w.all.push_back(r); cur += 4 + bs;
-      }
       const size_t tail = cur;    // first byte that is not part of a complete record
       std::vector<Rec>& all = w.all;
       t_scan += clk() - tc; tc = clk();
@@ -1131,5 +1143,211 @@ extern "C" int nb_bam_dump_groups(const char* input_file, int force_bam_paired, 
   }
   if (rc) { fclose(f); return rc; }
   fclose(f);
+  return NB_OK;
+}
+
+// ------------------------------------------------------------------ BAM mode in any record order (bam_group.hpp)
+namespace {
+
+struct AnyOrderLoad {   // what the producer saw (NB_BAM_STATS)
+  u64 n_records = 0, n_kept = 0; u32 max_len = 1; size_t peak_window = 0; double t_wait = 0;
+};
+
+// Streams the file window by window: the kept records of every window (SortedBamReader::fill_buffer's filters, in its
+// order) are staged into pinned memory on all threads and uploaded into the device store while the next window inflates.
+// cells: every kept record's full CB, ids in order of first appearance.
+int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st) {
+  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  Bgzf z; int rc = z.open(input_file); if (rc) return rc;
+  RawBuf data; size_t len = 0; bool eof = false, header_done = false;
+  std::vector<Rec> all;
+  for (;;) {
+    if (!eof) { size_t n_out = 0; rc = z.next(data, len, window_bytes, threads, n_out, eof); if (rc) return rc; z.compact(); len += n_out; }
+    st.peak_window = std::max(st.peak_window, len);
+    if (!header_done) {
+      bool ok = len >= 12; size_t p = 0;
+      if (ok && memcmp(data.data(), "BAM\1", 4)) return fail(NB_ERR_PARSE, "not a BAM file");
+      if (ok) { u32 l_text; memcpy(&l_text, &data[4], 4); p = 8 + (size_t)l_text; ok = p + 4 <= len; }
+      if (ok) { u32 n_ref; memcpy(&n_ref, &data[p], 4); p += 4; for (u32 i = 0; i < n_ref && ok; i++) { if (p + 4 > len) { ok = false; break; } u32 l; memcpy(&l, &data[p], 4); p += 4 + (size_t)l + 4; } ok = ok && p <= len; }
+      if (!ok) { if (eof) return fail(NB_ERR_PARSE, len < 12 ? "not a BAM file" : "truncated BAM header"); continue; }
+      memmove(data.data(), data.data() + p, len - p); len -= p; header_done = true;
+    }
+    size_t tail = 0;
+    rc = walk_records(data, len, 0, eof, threads, all, tail); if (rc) return rc;
+    if (all.empty()) { if (eof) break; continue; }   // one record larger than the window: read on
+    const size_t n = all.size();
+    const int T = n > 65536 ? threads : 1;
+    parallel_ranges(T, n, [&](size_t a, size_t b, int) { for (size_t i = a; i < b; i++) all[i].scan_keys(); });
+    // keep / skip / fail per record; the first failing record in file order decides the error
+    std::vector<u8> keep(n, 0); std::vector<u64> umi(n); std::vector<u32> cb(n, NONE32); std::vector<u64> cb_hash(n);
+    std::vector<size_t> bad_at(T, (size_t)-1); std::vector<int> bad_kind(T, 0); std::vector<u64> cnt(T + 1, 0), nib(T + 1, 0), nam(T + 1, 0); std::vector<u32> mx(T, 1);
+    std::vector<std::vector<u32>> miss(T);
+    parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
+      u64 c = 0, nb_ = 0, nm = 0; u32 m = 1;
+      for (size_t i = a; i < b; i++) {
+        const Rec& r = all[i];
+        if (!r.cb) continue;
+        if (!r.umi) { bad_at[t] = i; bad_kind[t] = 1; break; }
+        if (r.umi_len == 10 && !memcmp(r.umi, "AAAAAAAAAA", 10)) continue;
+        if (r.umi_len == 0) { bad_at[t] = i; bad_kind[t] = 2; break; }
+        if (!nbg::pack_umi(r.umi, r.umi_len, umi[i])) { bad_at[t] = i; bad_kind[t] = 3; break; }
+        keep[i] = 1; c++; nb_ += (r.l_seq() + 1) / 2; nm += r.qname_len();
+        size_t x, y; clip_of(r, x, y); m = std::max<u32>(m, (u32)(y - x));
+        const u64 h = cb_hash[i] = CellDict::hash_of(r.cb, r.cb_len);
+        if ((cb[i] = cells.find(r.cb, r.cb_len, h)) == NONE32) miss[t].push_back((u32)i);
+      }
+      cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm; mx[t] = m;
+    });
+    { size_t first = (size_t)-1; int kind = 0; for (int t = 0; t < T; t++) if (bad_at[t] < first) { first = bad_at[t]; kind = bad_kind[t]; }
+      if (kind == 1) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
+      if (kind == 2) return fail(NB_ERR_UNSUPPORTED, "a kept record has an empty UMI string (where the reference groups it depends on the file order): record " + std::to_string(st.n_records + first) + " of " + input_file);
+      if (kind == 3) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)"); }
+    for (int t = 0; t < T; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
+    for (int t = 0; t < T; t++) { cnt[t + 1] += cnt[t]; nib[t + 1] += nib[t]; nam[t + 1] += nam[t]; st.max_len = std::max(st.max_len, mx[t]); }
+    const double tw = now();
+    nbg::Stage* sg = nullptr;
+    rc = nbg::stage(dev, cnt[T], nib[T], nam[T], sg); if (rc) return rc;
+    st.t_wait += now() - tw;
+    const u64 ord0 = st.n_records;
+    parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
+      u64 k = cnt[t], bo = nib[t], no = nam[t];
+      for (size_t i = a; i < b; i++) if (keep[i]) {
+        const Rec& r = all[i]; const u32 l = r.l_seq(), nbytes = (l + 1) / 2, ql = r.qname_len();
+        memcpy(sg->nib + bo, r.seq4(), nbytes);
+        memcpy(sg->qual + 2 * bo, r.qual(), l);   // one qual byte per base, at the base's offset
+        memcpy(sg->name + no, r.qname_ptr(), ql);
+        sg->umi[k] = umi[i]; sg->cb[k] = cb[i]; sg->nib_off[k] = sg->nib0 + bo; sg->lseq[k] = l; sg->flag[k] = (u16)r.flag();
+        sg->name_off[k] = sg->name0 + no; sg->name_len[k] = (u8)ql; sg->ordinal[k] = ord0 + i;
+        k++; bo += nbytes; no += ql;
+      } });
+    rc = nbg::upload(dev); if (rc) return rc;
+    st.n_records += n; st.n_kept += cnt[T];
+    memmove(data.data(), data.data() + tail, len - tail); len -= tail;
+    if (eof) break;
+  }
+  return NB_OK;
+}
+
+// At the end of the file: the byte-order rank of every CB and an id for every CB[..len-2], then the device grouping.
+int any_order_group(nbg::Device* dev, const CellDict& cells, nbg::Grouped& g) {
+  const size_t nc = cells.size();
+  auto name = [&](u32 id) { return std::make_pair(cells.names.data() + cells.off[id], (u32)(cells.off[id + 1] - cells.off[id] - 1)); };
+  std::vector<u32> order(nc), rank(nc), prefix(nc);
+  for (u32 i = 0; i < nc; i++) order[i] = i;
+  std::sort(order.begin(), order.end(), [&](u32 a, u32 b) { auto x = name(a), y = name(b); return cmp_bytes(x.first, x.second, y.first, y.second) < 0; });
+  for (u32 i = 0; i < nc; i++) rank[order[i]] = i;
+  std::unordered_map<std::string, u32> pre;
+  for (u32 i = 0; i < nc; i++) { auto x = name(i); prefix[i] = pre.emplace(std::string(x.first, x.second >= 2 ? x.second - 2 : 0), (u32)pre.size()).first->second; }
+  return nbg::group(dev, rank, prefix, g);
+}
+
+}  // namespace
+
+extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                              int strand_filter, const char* trim, int num_cores, int device) {
+  if (!input_file || !reference_json || !matrix_dirs || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / matrix directory pair");
+  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  const double t_start = now();
+  const int threads = std::max(1, num_cores);
+  size_t window_bytes = (size_t)256 << 20;
+  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
+  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
+  std::vector<std::pair<u64, double>> trims;
+  if (trim && *trim) {   // src/bin/main.rs:74-93
+    std::string t(trim); size_t p = 0;
+    while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
+    if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
+  }
+  nbg::Device* dev = nullptr;
+  std::vector<nb_library*> libs(n_refs, nullptr); std::vector<nb_index*> idx(n_refs, nullptr); std::vector<nb_ctx*> ctx(n_refs, nullptr);
+  auto cleanup = [&]() { for (u32 i = 0; i < n_refs; i++) { nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } nbg::destroy(dev); };
+  int rc = nbg::create(device, &dev);
+  for (u32 i = 0; i < n_refs && rc == NB_OK; i++) {
+    rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
+    if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
+    if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);
+    if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nbg::stream_of(dev), &ctx[i]);   // one stream: the batches' scope ids are written on it
+    if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);
+  }
+  if (rc != NB_OK) { cleanup(); return rc; }
+  const double t_setup = now();
+  CellDict cells; AnyOrderLoad ld;
+  rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld);
+  if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); ld.t_wait += now() - tw; }
+  const double t_loaded = now();
+  nbg::Grouped g;
+  if (rc == NB_OK) rc = any_order_group(dev, cells, g);
+  const double t_grouped = now();
+  // barcodes: the cells of the scopes that have pairs, in order of first appearance; scopes without pairs get cell 0 (no rows)
+  std::vector<u32> remap(cells.size(), NONE32), cell_of_scope(g.n_scopes, 0); std::vector<const char*> bc;
+  if (rc == NB_OK) {
+    for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) remap[g.scope_cb[s]] = 0;
+    for (u32 id = 0; id < cells.size(); id++) if (remap[id] != NONE32) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
+    for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) cell_of_scope[s] = remap[g.scope_cb[s]];
+  }
+  // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
+  const u64 BATCH_PAIRS = 1u << 20;
+  double t_align = 0, t_roll = 0; u64 n_batches = 0;
+  for (u64 s0 = 0; rc == NB_OK && s0 < g.n_scopes;) {
+    u64 s1 = s0 + 1;
+    while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
+    const u64 p0 = g.scope_pair0[s0], p1 = g.scope_pair0[s1];
+    if (p1 > p0) {
+      n_batches++;
+      nb_batch b; rc = nbg::batch(dev, p0, p1, s0, ld.max_len, b);
+      for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+        const double tb = now();
+        rc = nb_counts_reset(ctx[li]);
+        if (rc == NB_OK) rc = nb_ctx_set_option(ctx[li], "max_batch_pairs", p1 - p0);   // scoped device batches must fit one chunk
+        if (rc == NB_OK) rc = nb_align_batch(ctx[li], &b, nullptr, nullptr);
+        nb_counts cts;
+        if (rc == NB_OK) rc = nb_counts_finalize(ctx[li], &cts);
+        const double tr = now(); t_align += tr - tb;
+        if (rc == NB_OK) rc = nb_cells_roll(ctx[li], cell_of_scope.data() + s0, s1 - s0);
+        t_roll += now() - tr;
+      }
+    }
+    s0 = s1;
+  }
+  const double t_aligned = now();
+  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) { nb_cell_counts cc; rc = nb_cells_finalize(ctx[li], &cc); if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size()); }
+  const double t_end = now();
+  if (getenv("NB_BAM_STATS")) {
+    double hwm_mb = 0; if (FILE* stf = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, stf)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(stf); }
+    fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB\n",
+            (unsigned long long)ld.n_records, (unsigned long long)ld.n_kept, (unsigned long long)g.n_scopes, (unsigned long long)g.n_pairs, (unsigned long long)n_batches, bc.size(),
+            t_setup - t_start, t_loaded - t_setup, ld.t_wait, ld.peak_window / 1048576.0, t_grouped - t_loaded, t_align, t_roll, t_end - t_aligned, t_end - t_start,
+            (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb);
+  }
+  cleanup();
+  return rc;
+}
+
+// Test hook: the real device grouping, one line per pair in batch order: scope index (counting the scopes with pairs), the
+// scope's cell barcode, the file ordinals of the sequence-slot and mate-slot records, both NB_FLAG_* and both clipped lengths.
+extern "C" int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path) {
+  if (!input_file || !out_path) return fail(NB_ERR_INVALID, "null argument");
+  size_t window_bytes = (size_t)256 << 20;
+  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
+  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
+  nbg::Device* dev = nullptr;
+  int rc = nbg::create(device, &dev);
+  CellDict cells; AnyOrderLoad ld; nbg::Grouped g;
+  if (rc == NB_OK) rc = any_order_load(input_file, std::max(1, num_cores), window_bytes, dev, cells, ld);
+  if (rc == NB_OK) rc = any_order_group(dev, cells, g);
+  std::vector<u64> o1, o2; std::vector<u8> f1, f2; std::vector<u32> l1, l2;
+  if (rc == NB_OK) rc = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
+  nbg::destroy(dev);
+  if (rc) return rc;
+  FILE* f = fopen(out_path, "wb"); if (!f) return fail(NB_ERR_IO, std::string("could not open ") + out_path);
+  u64 shown = 0;
+  for (u64 s = 0; s < g.n_scopes; s++) {
+    if (g.scope_pair0[s + 1] == g.scope_pair0[s]) continue;
+    const char* cb = cells.names.data() + cells.off[g.scope_cb[s]];
+    for (u64 p = g.scope_pair0[s]; p < g.scope_pair0[s + 1]; p++)
+      fprintf(f, "%llu\t%s\t%llu\t%llu\t%u\t%u\t%u\t%u\n", (unsigned long long)shown, cb, (unsigned long long)o1[p], (unsigned long long)o2[p], f1[p], f2[p], l1[p], l2[p]);
+    shown++;
+  }
+  if (fclose(f) != 0) return fail(NB_ERR_IO, std::string("short write on ") + out_path);
   return NB_OK;
 }

@@ -1,0 +1,60 @@
+// bam_group.hpp — the device record store of BAM mode in any record order (nb_process_bam_cells_any_order): the host
+// producer stages every kept record's nibbles, quals, name and keys window by window; the device sorts the records by
+// (UMI, CB), cuts the (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into
+// the store.  Host-only declarations (bam.cpp includes them; bam_group.cu implements them).
+#pragma once
+#include "host.hpp"
+
+namespace nbg {
+
+enum { MAX_UMI_CHARS = 21 };   // 3 bits per character of ACGTN, 63 bits
+
+// UMI -> exact sort key: characters A C G N T as 1..5 (their byte order), first character in the highest bits, 0 after the
+// end, so equal keys are equal strings and the keys sort like the strings.  false: not representable (empty, longer than
+// 21 characters, or a character outside ACGTN).
+inline bool pack_umi(const char* s, u32 n, u64& key) {
+  if (n == 0 || n > MAX_UMI_CHARS) return false;
+  u64 k = 0;
+  for (u32 i = 0; i < n; i++) {
+    u64 c;
+    switch (s[i]) { case 'A': c = 1; break; case 'C': c = 2; break; case 'G': c = 3; break; case 'N': c = 4; break; case 'T': c = 5; break; default: return false; }
+    k |= c << (60 - 3 * i);
+  }
+  key = k; return true;
+}
+
+// Pinned staging of one window's kept records.  Offsets are global: nib_off = byte offset of the record's first nibble byte
+// in the nibble store (its quals start at base offset 2 * nib_off of the qual store), name_off = offset in the name store.
+struct Stage {
+  u64 rec0 = 0, nib0 = 0, name0 = 0;        // store sizes before this window (the first record / byte this window adds)
+  u64 n_rec = 0, n_nib = 0, n_name = 0;     // what this window adds
+  u8* nib = nullptr; u8* qual = nullptr; char* name = nullptr;
+  u64* umi = nullptr; u32* cb = nullptr; u64* nib_off = nullptr; u32* lseq = nullptr; u16* flag = nullptr; u64* name_off = nullptr; u8* name_len = nullptr;
+  u64* ordinal = nullptr;
+};
+
+struct Device;   // the store, the grouping buffers and the stream (bam_group.cu)
+
+int create(int device, Device** out);
+void destroy(Device*);
+void* stream_of(Device*);                                  // cudaStream_t: the library contexts are created on it
+int sync(Device*);                                         // waits for everything queued on that stream
+// Waits until the staging slot's previous upload has run, sizes it for this window and fills rec0 / nib0 / name0.
+int stage(Device*, u64 n_rec, u64 n_nib, u64 n_name, Stage*& st);
+int upload(Device*);                                       // queues the copies of the staged window (plain cudaMemcpyAsync)
+
+struct Grouped {
+  u64 n_records = 0, n_scopes = 0, n_pairs = 0;
+  std::vector<u64> scope_pair0;   // n_scopes + 1: first pair of every scope
+  std::vector<u32> scope_cb;      // CB id (the producer's dictionary) of every scope's first record
+};
+// cb_rank[id] = rank of CB id in byte order, cb_prefix[id] = id of its CB[..len-2]
+int group(Device*, const std::vector<u32>& cb_rank, const std::vector<u32>& cb_prefix, Grouped& g);
+// Fills a device-resident NB_SEQ_BAM4 batch over pairs [p0, p1) whose scope ids are local to the batch (scope - scope0).
+int batch(Device*, u64 p0, u64 p1, u64 scope0, u32 max_read_len, nb_batch& b);
+// Test hook: per pair the file ordinals of both slots, their flags and clipped lengths.
+int pairs_to_host(Device*, std::vector<u64>& ord1, std::vector<u64>& ord2, std::vector<u8>& f1, std::vector<u8>& f2, std::vector<u32>& l1, std::vector<u32>& l2);
+u64 store_bytes(Device*);       // device bytes of the record store (nibbles, quals, names, per-record keys)
+u64 group_bytes(Device*);       // device bytes of the sort, scope and pair arrays
+
+}  // namespace nbg

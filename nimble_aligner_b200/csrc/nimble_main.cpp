@@ -12,7 +12,7 @@
 static void die(const std::string& m) { fprintf(stderr, "%s\n", m.c_str()); exit(101); }  // a Rust panic exits 101
 
 int main(int argc, char** argv) {
-  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
+  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false, any_order = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
   std::vector<std::string>* cur = nullptr;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
@@ -28,19 +28,24 @@ int main(int argc, char** argv) {
     if (a == "--index-cache") { const std::string dir = val("--index-cache"); setenv("NB_INDEX_CACHE", dir.c_str(), 1); cur = nullptr; continue; }   // not in cli.yml: keep each library's index in <dir>/<key>.nbix (default: NB_INDEX_CACHE, else rebuilt per run like the reference)
     if (a == "--cell-matrix") { cur = &mats; have_mats = true; continue; }   // not in cli.yml: BAM mode, one directory per -r for a cell x feature matrix (10x v3 layout)
     if (a == "--no-rows") { no_rows = true; cur = nullptr; continue; }          // not in cli.yml: BAM mode, no TSV.gz rows (with --cell-matrix, without -o)
+    if (a == "--any-order") { any_order = true; cur = nullptr; continue; }      // not in cli.yml: BAM mode, scopes from the tags of a BAM in any record order (with --cell-matrix --no-rows)
     if (a == "-h" || a == "--help") {
       printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"
              "  -d, --devices <list>          GPUs to use, \"0,1,...\" (default: NB_DEVICES, else 0)\n"
              "      --index-cache <dir>       keep each library's index in <dir> (default: NB_INDEX_CACHE)\n"
              "      --cell-matrix <dir>...    BAM input: also write a cell x feature matrix per reference library into <dir>\n"
              "                                (matrix.mtx.gz UMIs, reads.mtx.gz reads, features.tsv.gz, barcodes.tsv.gz)\n"
-             "      --no-rows                 BAM input with --cell-matrix: skip the TSV.gz rows (no --output)\n");
+             "      --no-rows                 BAM input with --cell-matrix: skip the TSV.gz rows (no --output)\n"
+             "      --any-order               BAM input with --cell-matrix --no-rows: records in any order (e.g. position-sorted);\n"
+             "                                (UMI, CB) scopes are formed on the GPU, no sort by UB needed (no -p)\n");
       return 0;
     }
     if (a == "-V" || a == "--version") { printf("nimble 0.8.0\n"); return 0; }
     if (!cur) die("error: Found argument '" + a + "' which wasn't expected, or isn't valid in this context");
     cur->push_back(a);
   }
+  if (any_order && (!have_mats || !no_rows)) die("error: --any-order needs --cell-matrix and --no-rows (it writes no TSV rows)");
+  if (any_order && force_paired) die("error: --any-order cannot pair mates (-p): the mates of a position-sorted file are not neighbours");
   if (no_rows && !outs.empty()) die("error: --no-rows writes no TSV: leave out --output");
   if (no_rows && !have_mats) die("error: --no-rows needs --cell-matrix (there would be nothing to write)");
   if (have_mats && mats.size() != refs.size()) die("error: --cell-matrix needs one directory per reference library");
@@ -67,13 +72,14 @@ int main(int argc, char** argv) {
   printf("Loading read sequences and aligning\n");
   std::vector<const char*> m; for (auto& s : mats) m.push_back(s.c_str());
   if (ends(first, ".fastq.gz") || ends(lower, ".fastq")) {
-    if (have_mats || no_rows) die("error: --cell-matrix and --no-rows need a BAM input (FASTQ reads have no cells)");
+    if (have_mats || no_rows || any_order) die("error: --cell-matrix, --no-rows and --any-order need a BAM input (FASTQ reads have no cells)");
     printf("Processing as FASTQ file\n");
     int rc = nb_process_fastq_devices(in.data(), (uint32_t)std::min<size_t>(in.size(), 2), r.data(), o.data(), (uint32_t)r.size(), chem, (int)ncores, devices.data(), (uint32_t)devices.size());
     if (rc != NB_OK) die(nb_last_error());
   } else if (ends(lower, ".bam")) {
     printf("Processing as BAM file\n");
-    int rc = nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
+    int rc = any_order ? nb_process_bam_cells_any_order(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0])
+                       : nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
     if (rc != NB_OK) die(nb_last_error());
   } else die("Unsupported file format: " + (lower.find('.') == std::string::npos ? std::string("") : lower.substr(lower.rfind('.') + 1)));
   printf("Alignment successful, terminating.\n");
