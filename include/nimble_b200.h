@@ -393,6 +393,28 @@ int nb_process_bam_cells_any_order(const char* input_file, const char* const* re
  * scope index (counting the scopes with pairs, in sorted order) TAB cell barcode TAB sequence-slot ordinal TAB mate-slot ordinal
  * TAB flags (NB_FLAG_*) of both slots TAB clipped lengths of both slots */
 int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path);
+/* nb_process_bam_cells_any_order under a device-memory budget of budget_bytes (0: none, exactly
+ * nb_process_bam_cells_any_order).  The budget covers every device allocation of the any-order path: the record store
+ * (also while an array grows and its old and new copies are both alive), the sort, scope and pair arrays and the scratch of
+ * a compaction.  It does not cover the library contexts: the index, the aggregation tables and the per-cell table.
+ * Records are split by UMI bucket, the top 16 bits of the splitmix64 finalizer of the exact UMI key (nb_any_order_umi_bucket),
+ * so every scope falls whole into one bucket.  Each pass reads the file from the start and keeps buckets [lo, hi), hi
+ * starting at 65536; when the store, the next window and the grouping arrays would not fit the budget, hi falls to the
+ * largest value whose buckets fit 3/4 of it, the store is compacted in place to the records below hi, and later records at
+ * or above hi are dropped.  At the end of the file the pass groups, aligns and rolls as the single pass does; the next pass
+ * starts at lo = hi.  A file that fits takes one pass.  The matrix files are the bytes of the unbudgeted run.  Refused with
+ * NB_ERR_CUDA, naming the budget and the bytes needed: a budget that cannot hold one bucket.  NB_BAM_STATS=1 adds budget,
+ * passes, evictions (compactions), peak device bytes and the windows time of every pass to the stats line.
+ * NB_BAM_COMPACT_TILE_BYTES=N caps the compaction's scratch tile at N bytes (at least 64; default up to 16 MB). */
+int nb_process_bam_cells_any_order_budget(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                          int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes);
+/* test hook: nb_bam_dump_scopes_any_order under a budget; every line starts with the pass index TAB, scope indices count on
+ * across passes, and each line ends with TAB bases TAB quals (hex) of the sequence slot and of the mate slot, clipped, read
+ * back from the device store after the pass (so after any compaction) */
+int nb_bam_dump_scopes_any_order_budget(const char* input_file, int num_cores, int device, uint64_t budget_bytes, const char* out_path);
+/* test hook (host-only): the UMI bucket (0..65535) of nb_process_bam_cells_any_order_budget for a UMI string, so that tests
+ * can check the bucket function against a restatement; NB_ERR_UNSUPPORTED when the exact key cannot hold it */
+int nb_any_order_umi_bucket(const char* umi, uint32_t len, uint32_t* bucket);
 /* host-only: a cell x feature matrix in the 10x v3 layout that Seurat's Read10X and scanpy's read_10x_mtx load, into `dir`
  * (created when missing; its parent must exist): matrix.mtx.gz (Matrix Market coordinate integer, features x barcodes, UMI
  * counts, 1-based lines sorted by barcode then feature), reads.mtx.gz (the same coordinates with the read counts),

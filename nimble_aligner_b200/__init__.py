@@ -152,6 +152,9 @@ _SIGS = {
     "nb_process_bam_cells": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_int]),
     "nb_process_bam_cells_any_order": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int]),
     "nb_bam_dump_scopes_any_order": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_char_p]),
+    "nb_process_bam_cells_any_order_budget": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_uint64]),
+    "nb_bam_dump_scopes_any_order_budget": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_uint64, C.c_char_p]),
+    "nb_any_order_umi_bucket": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
     "nb_cells_reset": (C.c_int, [C.c_void_p]),
@@ -668,11 +671,15 @@ def fastq_dump(input_files, out_path, num_cores=1, chunk_bytes=0):
 
 
 def process_bam(input_file, reference_json_paths, output_paths, strand_filter="unstranded", trim=None, num_cores=1, force_bam_paired=False, device=0,
-                matrix_dirs=None, any_order=False):
+                matrix_dirs=None, any_order=False, device_budget=None):
     """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156).
     matrix_dirs=[dir per library]: also a cell x feature matrix per library (nb_process_bam_cells); output_paths=None with
     matrix_dirs: no TSV rows at all.  any_order=True: the matrices only (output_paths=None, matrix_dirs required, no
-    force_bam_paired) from a BAM in any record order, scopes formed on the GPU (nb_process_bam_cells_any_order)."""
+    force_bam_paired) from a BAM in any record order, scopes formed on the GPU (nb_process_bam_cells_any_order).
+    device_budget=bytes (any_order only): the device memory that path may allocate; it takes passes over the file by UMI
+    bucket when the records do not fit (nb_process_bam_cells_any_order_budget), and writes the same bytes."""
+    if device_budget is not None:
+        _check_budget(device_budget, any_order)
     if any_order:
         if output_paths is not None:
             raise NbError(-1, "any_order writes no TSV rows: pass output_paths=None")
@@ -680,6 +687,10 @@ def process_bam(input_file, reference_json_paths, output_paths, strand_filter="u
             raise NbError(-1, "any_order needs matrix_dirs")
         if force_bam_paired:
             raise NbError(-1, "any_order cannot pair mates (force_bam_paired): the mates of a position-sorted file are not neighbours")
+        if device_budget is not None:
+            _ck(lib().nb_process_bam_cells_any_order_budget(str(input_file).encode(), _strs(reference_json_paths), _strs(matrix_dirs), len(reference_json_paths),
+                                                            CHEM[strand_filter], trim.encode() if trim else None, num_cores, device, int(device_budget)))
+            return
         _ck(lib().nb_process_bam_cells_any_order(str(input_file).encode(), _strs(reference_json_paths), _strs(matrix_dirs), len(reference_json_paths),
                                                  CHEM[strand_filter], trim.encode() if trim else None, num_cores, device))
         return
@@ -745,6 +756,27 @@ def bam_dump_groups(input_file, out_path, force_bam_paired=False, num_cores=1):
     _ck(lib().nb_bam_dump_groups(str(input_file).encode(), int(force_bam_paired), num_cores, str(out_path).encode()))
 
 
-def bam_dump_scopes_any_order(input_file, out_path, num_cores=1, device=0):
-    """The device grouping of process_bam(any_order=True), one line per pair (nb_bam_dump_scopes_any_order)."""
+def _check_budget(device_budget, any_order=True):
+    if not any_order:
+        raise NbError(-1, "device_budget applies to any_order=True only")
+    if isinstance(device_budget, bool) or not isinstance(device_budget, int) or device_budget <= 0:
+        raise NbError(-1, "device_budget must be a positive number of bytes")
+
+
+def bam_dump_scopes_any_order(input_file, out_path, num_cores=1, device=0, device_budget=None):
+    """The device grouping of process_bam(any_order=True), one line per pair (nb_bam_dump_scopes_any_order).  With
+    device_budget: the passes of that budget, each line led by its pass index and followed by both slots' bases and quals
+    as read back from the store (nb_bam_dump_scopes_any_order_budget)."""
+    if device_budget is not None:
+        _check_budget(device_budget)
+        _ck(lib().nb_bam_dump_scopes_any_order_budget(str(input_file).encode(), num_cores, device, int(device_budget), str(out_path).encode()))
+        return
     _ck(lib().nb_bam_dump_scopes_any_order(str(input_file).encode(), num_cores, device, str(out_path).encode()))
+
+
+def any_order_umi_bucket(umi):
+    """The UMI bucket (0..65535) that process_bam(any_order=True, device_budget=...) splits its passes by (host-only)."""
+    b = C.c_uint32(0)
+    u = umi.encode()
+    _ck(lib().nb_any_order_umi_bucket(u, len(u), C.byref(b)))
+    return b.value

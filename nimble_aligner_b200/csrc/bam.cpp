@@ -1153,14 +1153,57 @@ struct AnyOrderLoad {   // what the producer saw (NB_BAM_STATS)
   u64 n_records = 0, n_kept = 0; u32 max_len = 1; size_t peak_window = 0; double t_wait = 0;
 };
 
+// Budget mode: a pass stages the records of UMI buckets [lo, hi) (nbg::umi_bucket); hi starts at N_BUCKETS and only falls.
+struct Passes {
+  u64 budget = 0; int pass = 0; u32 lo = 0, hi = nbg::N_BUCKETS; u64 evictions = 0;
+  std::vector<u64> b_rec, b_nib, b_name;   // what this pass has staged (or is about to) of every bucket
+  void begin(u32 lo_) { lo = lo_; hi = nbg::N_BUCKETS; b_rec.assign(nbg::N_BUCKETS, 0); b_nib.assign(nbg::N_BUCKETS, 0); b_name.assign(nbg::N_BUCKETS, 0); }
+};
+
+// Before a window is staged in budget mode (the per-bucket counts already hold it): when the store plus the window plus the
+// grouping arrays would not fit, hi falls to the largest value whose buckets fit the fill target (3/4 of the budget, grouping
+// arrays included) and the device keeps only the records below it.  The caller drops the window's records at or above hi.
+int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
+  lowered = false;
+  const u32 lo = P.lo, hi = P.hi;
+  std::vector<u64> R(hi - lo + 1, 0), NB(hi - lo + 1, 0), NM(hi - lo + 1, 0);   // sums over buckets [lo, lo + k)
+  for (u32 k = 0; k < hi - lo; k++) { R[k + 1] = R[k] + P.b_rec[lo + k]; NB[k + 1] = NB[k] + P.b_nib[lo + k]; NM[k + 1] = NM[k] + P.b_name[lo + k]; }
+  auto fits = [&](u32 k) { return nbg::fits(dev, R[k], NB[k], NM[k], nbg::group_reserve(dev, R[k], ncb)); };
+  if (fits(hi - lo)) return NB_OK;
+  auto under_target = [&](u32 k) { return 3 * NB[k] + NM[k] + 43 * R[k] + nbg::group_reserve(dev, R[k], ncb) <= P.budget / 4 * 3 && fits(k); };
+  u32 a = 0, b = hi - lo;   // the largest k in (0, hi - lo) under the target: ok(a) (or a = 0), !ok(b)
+  while (b - a > 1) { const u32 m = a + (b - a) / 2; if (under_target(m)) a = m; else b = m; }
+  bool compacted = false;
+  if (a == 0) {
+    if (!fits(1)) {
+      // the store may hold arrays sized for records of other buckets: keep bucket lo alone, shrink the arrays, look again
+      if (nbg::store_records(dev)) { const int rc = nbg::compact(dev, lo + 1); if (rc) return rc; P.evictions++; compacted = true; }
+      { const int rc = nbg::trim(dev); if (rc) return rc; }
+      if (!fits(1)) {
+        const u64 need = nbg::need_bytes(dev, R[1], NB[1], NM[1], nbg::group_reserve(dev, R[1], ncb));
+        return fail(NB_ERR_CUDA, "the device budget of " + std::to_string(P.budget) + " bytes is too small: UMI bucket " + std::to_string(lo) + " needs " + std::to_string(need) +
+                                 " bytes (" + std::to_string(R[1]) + " records with their grouping arrays)");
+      }
+    }
+    a = 1;
+  }
+  const u32 nh = lo + a;
+  if (!compacted && nbg::store_records(dev)) { const int rc = nbg::compact(dev, nh); if (rc) return rc; P.evictions++; }   // an eviction: records already on the device leave
+  for (u32 x = nh; x < hi; x++) P.b_rec[x] = P.b_nib[x] = P.b_name[x] = 0;
+  P.hi = nh; lowered = true;
+  return NB_OK;
+}
+
 // Streams the file window by window: the kept records of every window (SortedBamReader::fill_buffer's filters, in its
 // order) are staged into pinned memory on all threads and uploaded into the device store while the next window inflates.
-// cells: every kept record's full CB, ids in order of first appearance.
-int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st) {
+// cells: every kept record's full CB, ids in order of first appearance.  With P (budget mode) only the records of buckets
+// [P->lo, P->hi) are staged, and passes after the first only look the CBs up.
+int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, Passes* P = nullptr) {
   auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   Bgzf z; int rc = z.open(input_file); if (rc) return rc;
   RawBuf data; size_t len = 0; bool eof = false, header_done = false;
   std::vector<Rec> all;
+  const bool lookup_only = P && P->pass > 0;
   for (;;) {
     if (!eof) { size_t n_out = 0; rc = z.next(data, len, window_bytes, threads, n_out, eof); if (rc) return rc; z.compact(); len += n_out; }
     st.peak_window = std::max(st.peak_window, len);
@@ -1182,6 +1225,7 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
     std::vector<u8> keep(n, 0); std::vector<u64> umi(n); std::vector<u32> cb(n, NONE32); std::vector<u64> cb_hash(n);
     std::vector<size_t> bad_at(T, (size_t)-1); std::vector<int> bad_kind(T, 0); std::vector<u64> cnt(T + 1, 0), nib(T + 1, 0), nam(T + 1, 0); std::vector<u32> mx(T, 1);
     std::vector<std::vector<u32>> miss(T);
+    std::vector<u32> bucket(P ? n : 0);
     parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
       u64 c = 0, nb_ = 0, nm = 0; u32 m = 1;
       for (size_t i = a; i < b; i++) {
@@ -1191,18 +1235,33 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
         if (r.umi_len == 10 && !memcmp(r.umi, "AAAAAAAAAA", 10)) continue;
         if (r.umi_len == 0) { bad_at[t] = i; bad_kind[t] = 2; break; }
         if (!nbg::pack_umi(r.umi, r.umi_len, umi[i])) { bad_at[t] = i; bad_kind[t] = 3; break; }
-        keep[i] = 1; c++; nb_ += (r.l_seq() + 1) / 2; nm += r.qname_len();
         size_t x, y; clip_of(r, x, y); m = std::max<u32>(m, (u32)(y - x));
         const u64 h = cb_hash[i] = CellDict::hash_of(r.cb, r.cb_len);
-        if ((cb[i] = cells.find(r.cb, r.cb_len, h)) == NONE32) miss[t].push_back((u32)i);
+        if ((cb[i] = cells.find(r.cb, r.cb_len, h)) == NONE32) { if (lookup_only) { bad_at[t] = i; bad_kind[t] = 4; break; } miss[t].push_back((u32)i); }
+        if (P) { const u32 bk = bucket[i] = nbg::umi_bucket(umi[i]); if (bk < P->lo || bk >= P->hi) continue; }
+        keep[i] = 1; c++; nb_ += (r.l_seq() + 1) / 2; nm += r.qname_len();
       }
       cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm; mx[t] = m;
     });
     { size_t first = (size_t)-1; int kind = 0; for (int t = 0; t < T; t++) if (bad_at[t] < first) { first = bad_at[t]; kind = bad_kind[t]; }
       if (kind == 1) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
       if (kind == 2) return fail(NB_ERR_UNSUPPORTED, "a kept record has an empty UMI string (where the reference groups it depends on the file order): record " + std::to_string(st.n_records + first) + " of " + input_file);
-      if (kind == 3) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)"); }
+      if (kind == 3) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)");
+      if (kind == 4) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see"); }
     for (int t = 0; t < T; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
+    if (P) {
+      for (size_t i = 0; i < n; i++) if (keep[i]) { const u32 bk = bucket[i]; P->b_rec[bk]++; P->b_nib[bk] += (all[i].l_seq() + 1) / 2; P->b_name[bk] += all[i].qname_len(); }
+      bool lowered = false;
+      rc = plan_window(dev, *P, cells.size(), lowered); if (rc) return rc;
+      if (lowered) parallel_ranges(T, n, [&](size_t a, size_t b, int t) {   // drop this window's records at or above the new hi
+        u64 c = 0, nb_ = 0, nm = 0;
+        for (size_t i = a; i < b; i++) {
+          if (keep[i] && bucket[i] >= P->hi) keep[i] = 0;
+          if (keep[i]) { c++; nb_ += (all[i].l_seq() + 1) / 2; nm += all[i].qname_len(); }
+        }
+        cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm;
+      });
+    }
     for (int t = 0; t < T; t++) { cnt[t + 1] += cnt[t]; nib[t + 1] += nib[t]; nam[t + 1] += nam[t]; st.max_len = std::max(st.max_len, mx[t]); }
     const double tw = now();
     nbg::Stage* sg = nullptr;
@@ -1220,7 +1279,7 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
         sg->name_off[k] = sg->name0 + no; sg->name_len[k] = (u8)ql; sg->ordinal[k] = ord0 + i;
         k++; bo += nbytes; no += ql;
       } });
-    rc = nbg::upload(dev); if (rc) return rc;
+    rc = nbg::upload(dev, P ? nbg::group_reserve(dev, nbg::store_records(dev) + cnt[T], cells.size()) : 0); if (rc) return rc;
     st.n_records += n; st.n_kept += cnt[T];
     memmove(data.data(), data.data() + tail, len - tail); len -= tail;
     if (eof) break;
@@ -1241,17 +1300,58 @@ int any_order_group(nbg::Device* dev, const CellDict& cells, nbg::Grouped& g) {
   return nbg::group(dev, rank, prefix, g);
 }
 
-}  // namespace
+// What a run in any record order did over all its passes (NB_BAM_STATS).
+struct AnyOrderRun {
+  AnyOrderLoad ld;                       // the first pass's producer (every pass reads the same records)
+  int passes = 0; u64 evictions = 0, n_kept = 0, n_scopes = 0, n_pairs = 0;
+  std::vector<double> t_windows; double t_group = 0;
+};
 
-extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
-                                              int strand_filter, const char* trim, int num_cores, int device) {
+// The passes over the file: one without a budget; with one, each pass takes the UMI buckets from where the previous one
+// stopped up to the hi its windows left.  After each pass's grouping: on_pass(pass, grouped, max_read_len) aligns it.
+template <class F>
+int any_order_passes(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, u64 budget, CellDict& cells, AnyOrderRun& run, F on_pass) {
+  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  Passes P; P.budget = budget;
+  nbg::set_budget(dev, budget);
+  for (u32 lo = 0;;) {
+    int rc = NB_OK;
+    if (budget) { P.begin(lo); if (P.pass) rc = nbg::begin_pass(dev); }
+    const double t0 = now();
+    AnyOrderLoad ld;
+    if (rc == NB_OK) rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld, budget ? &P : nullptr);
+    if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); ld.t_wait += now() - tw; }
+    const double t1 = now(); run.t_windows.push_back(t1 - t0);
+    nbg::Grouped g;
+    if (rc == NB_OK) rc = any_order_group(dev, cells, g);
+    run.t_group += now() - t1;
+    if (rc) return rc;
+    if (P.pass == 0) run.ld = ld;
+    else if (ld.n_records != run.ld.n_records) return fail(NB_ERR_IO, std::string("the input changed between passes: ") + input_file);
+    else { run.ld.t_wait += ld.t_wait; run.ld.peak_window = std::max(run.ld.peak_window, ld.peak_window); }
+    run.passes++; run.n_kept += g.n_records; run.n_scopes += g.n_scopes; run.n_pairs += g.n_pairs;
+    rc = on_pass(P.pass, (const nbg::Grouped&)g, run.ld.max_len); if (rc) return rc;
+    if (!budget || P.hi == nbg::N_BUCKETS) break;
+    lo = P.hi; P.pass++;
+  }
+  run.evictions = P.evictions;
+  return NB_OK;
+}
+
+size_t any_order_window_bytes() {
+  size_t window_bytes = (size_t)256 << 20;
+  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
+  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
+  return window_bytes;
+}
+
+int process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
   if (!input_file || !reference_json || !matrix_dirs || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / matrix directory pair");
   auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t_start = now();
   const int threads = std::max(1, num_cores);
-  size_t window_bytes = (size_t)256 << 20;
-  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
-  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
+  const size_t window_bytes = any_order_window_bytes();
   std::vector<std::pair<u64, double>> trims;
   if (trim && *trim) {   // src/bin/main.rs:74-93
     std::string t(trim); size_t p = 0;
@@ -1271,83 +1371,142 @@ extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char
   }
   if (rc != NB_OK) { cleanup(); return rc; }
   const double t_setup = now();
-  CellDict cells; AnyOrderLoad ld;
-  rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld);
-  if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); ld.t_wait += now() - tw; }
-  const double t_loaded = now();
-  nbg::Grouped g;
-  if (rc == NB_OK) rc = any_order_group(dev, cells, g);
-  const double t_grouped = now();
-  // barcodes: the cells of the scopes that have pairs, in order of first appearance; scopes without pairs get cell 0 (no rows)
-  std::vector<u32> remap(cells.size(), NONE32), cell_of_scope(g.n_scopes, 0); std::vector<const char*> bc;
-  if (rc == NB_OK) {
-    for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) remap[g.scope_cb[s]] = 0;
-    for (u32 id = 0; id < cells.size(); id++) if (remap[id] != NONE32) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
-    for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) cell_of_scope[s] = remap[g.scope_cb[s]];
-  }
-  // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
-  const u64 BATCH_PAIRS = 1u << 20;
+  CellDict cells; AnyOrderRun run;
+  // barcodes: the cells of the scopes that have pairs, in order of first appearance.  Without a budget the one pass knows
+  // them before it rolls; with one, the passes roll dictionary ids and the rows are renumbered after the last pass (an
+  // order-preserving map, so the (cell, rank) order of the rows holds).
+  std::vector<u32> remap; std::vector<u8> used; std::vector<const char*> bc;
+  const u64 BATCH_PAIRS = 1u << 20;   // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
   double t_align = 0, t_roll = 0; u64 n_batches = 0;
-  for (u64 s0 = 0; rc == NB_OK && s0 < g.n_scopes;) {
-    u64 s1 = s0 + 1;
-    while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
-    const u64 p0 = g.scope_pair0[s0], p1 = g.scope_pair0[s1];
-    if (p1 > p0) {
-      n_batches++;
-      nb_batch b; rc = nbg::batch(dev, p0, p1, s0, ld.max_len, b);
-      for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
-        const double tb = now();
-        rc = nb_counts_reset(ctx[li]);
-        if (rc == NB_OK) rc = nb_ctx_set_option(ctx[li], "max_batch_pairs", p1 - p0);   // scoped device batches must fit one chunk
-        if (rc == NB_OK) rc = nb_align_batch(ctx[li], &b, nullptr, nullptr);
-        nb_counts cts;
-        if (rc == NB_OK) rc = nb_counts_finalize(ctx[li], &cts);
-        const double tr = now(); t_align += tr - tb;
-        if (rc == NB_OK) rc = nb_cells_roll(ctx[li], cell_of_scope.data() + s0, s1 - s0);
-        t_roll += now() - tr;
-      }
+  rc = any_order_passes(input_file, threads, window_bytes, dev, budget, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
+    std::vector<u32> cell_of_scope(g.n_scopes, 0);   // scopes without pairs get cell 0 (no rows)
+    if (!budget) {
+      remap.assign(cells.size(), NONE32);
+      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) remap[g.scope_cb[s]] = 0;
+      for (u32 id = 0; id < cells.size(); id++) if (remap[id] != NONE32) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
+      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) cell_of_scope[s] = remap[g.scope_cb[s]];
+    } else {
+      used.resize(cells.size(), 0);
+      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) { cell_of_scope[s] = g.scope_cb[s]; used[g.scope_cb[s]] = 1; }
     }
-    s0 = s1;
-  }
+    int e = NB_OK;
+    for (u64 s0 = 0; e == NB_OK && s0 < g.n_scopes;) {
+      u64 s1 = s0 + 1;
+      while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
+      const u64 p0 = g.scope_pair0[s0], p1 = g.scope_pair0[s1];
+      if (p1 > p0) {
+        n_batches++;
+        nb_batch b; e = nbg::batch(dev, p0, p1, s0, max_len, b);
+        for (u32 li = 0; li < n_refs && e == NB_OK; li++) {
+          const double tb = now();
+          e = nb_counts_reset(ctx[li]);
+          if (e == NB_OK) e = nb_ctx_set_option(ctx[li], "max_batch_pairs", p1 - p0);   // scoped device batches must fit one chunk
+          if (e == NB_OK) e = nb_align_batch(ctx[li], &b, nullptr, nullptr);
+          nb_counts cts;
+          if (e == NB_OK) e = nb_counts_finalize(ctx[li], &cts);
+          const double tr = now(); t_align += tr - tb;
+          if (e == NB_OK) e = nb_cells_roll(ctx[li], cell_of_scope.data() + s0, s1 - s0);
+          t_roll += now() - tr;
+        }
+      }
+      s0 = s1;
+    }
+    return e;
+  });
   const double t_aligned = now();
-  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) { nb_cell_counts cc; rc = nb_cells_finalize(ctx[li], &cc); if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size()); }
+  if (rc == NB_OK && budget) {
+    remap.assign(cells.size(), NONE32);
+    for (u32 id = 0; id < used.size(); id++) if (used[id]) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
+  }
+  std::vector<u32> row_cell;
+  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+    nb_cell_counts cc; rc = nb_cells_finalize(ctx[li], &cc);
+    if (rc == NB_OK && budget) { row_cell.resize(cc.n_rows); for (u64 k = 0; k < cc.n_rows; k++) row_cell[k] = remap[cc.row_cell[k]]; cc.row_cell = row_cell.data(); }
+    if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size());
+  }
   const double t_end = now();
   if (getenv("NB_BAM_STATS")) {
     double hwm_mb = 0; if (FILE* stf = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, stf)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(stf); }
-    fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB\n",
-            (unsigned long long)ld.n_records, (unsigned long long)ld.n_kept, (unsigned long long)g.n_scopes, (unsigned long long)g.n_pairs, (unsigned long long)n_batches, bc.size(),
-            t_setup - t_start, t_loaded - t_setup, ld.t_wait, ld.peak_window / 1048576.0, t_grouped - t_loaded, t_align, t_roll, t_end - t_aligned, t_end - t_start,
-            (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb);
+    const AnyOrderLoad& ld = run.ld;
+    double t_win = 0; std::string per_pass;
+    for (double t : run.t_windows) { t_win += t; char b[32]; snprintf(b, sizeof b, "%s%.2fs", per_pass.empty() ? "" : "/", t); per_pass += b; }
+    std::string extra;
+    if (budget) { char b[256]; snprintf(b, sizeof b, ", budget %llu bytes, passes %d, evictions %llu, peak device bytes %llu, windows per pass ", (unsigned long long)budget, run.passes, (unsigned long long)run.evictions, (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0)); extra = b + per_pass; }
+    fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB%s\n",
+            (unsigned long long)ld.n_records, (unsigned long long)run.n_kept, (unsigned long long)run.n_scopes, (unsigned long long)run.n_pairs, (unsigned long long)n_batches, bc.size(),
+            t_setup - t_start, t_win, ld.t_wait, ld.peak_window / 1048576.0, run.t_group, t_align, t_roll, t_end - t_aligned, t_end - t_start,
+            (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb, extra.c_str());
   }
   cleanup();
   return rc;
 }
 
-// Test hook: the real device grouping, one line per pair in batch order: scope index (counting the scopes with pairs), the
-// scope's cell barcode, the file ordinals of the sequence-slot and mate-slot records, both NB_FLAG_* and both clipped lengths.
-extern "C" int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path) {
+// The device grouping, one line per pair in batch order: scope index (counting the scopes with pairs), the scope's cell
+// barcode, the file ordinals of the sequence-slot and mate-slot records, both NB_FLAG_* and both clipped lengths.  With
+// slots: the pass index first, and each slot's clipped bases and quals (hex) as the store holds them after the pass.
+int dump_scopes_any_order(const char* input_file, int num_cores, int device, u64 budget, const char* out_path, bool slots) {
   if (!input_file || !out_path) return fail(NB_ERR_INVALID, "null argument");
-  size_t window_bytes = (size_t)256 << 20;
-  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
-  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
   nbg::Device* dev = nullptr;
   int rc = nbg::create(device, &dev);
-  CellDict cells; AnyOrderLoad ld; nbg::Grouped g;
-  if (rc == NB_OK) rc = any_order_load(input_file, std::max(1, num_cores), window_bytes, dev, cells, ld);
-  if (rc == NB_OK) rc = any_order_group(dev, cells, g);
-  std::vector<u64> o1, o2; std::vector<u8> f1, f2; std::vector<u32> l1, l2;
-  if (rc == NB_OK) rc = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
+  CellDict cells; AnyOrderRun run;
+  std::string out; u64 shown = 0;
+  static const char* SEQ = "=ACMGRSVTWYHKDBN"; static const char* H = "0123456789abcdef";
+  if (rc == NB_OK) rc = any_order_passes(input_file, std::max(1, num_cores), any_order_window_bytes(), dev, budget, cells, run, [&](int pass, const nbg::Grouped& g, u32) -> int {
+    std::vector<u64> o1, o2, b1, b2; std::vector<u8> f1, f2, nib, qual; std::vector<u32> l1, l2;
+    int e = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
+    if (e == NB_OK && slots) e = nbg::slots_to_host(dev, b1, b2, nib, qual);
+    if (e) return e;
+    auto slot = [&](u64 at, u32 n) {
+      out += '\t'; for (u64 k = at; k < at + n; k++) out += SEQ[(nib[k >> 1] >> ((k & 1) ? 0 : 4)) & 15];
+      out += '\t'; for (u64 k = at; k < at + n; k++) { out += H[qual[k] >> 4]; out += H[qual[k] & 15]; }
+    };
+    char line[256];
+    for (u64 s = 0; s < g.n_scopes; s++) {
+      if (g.scope_pair0[s + 1] == g.scope_pair0[s]) continue;
+      const char* cb = cells.names.data() + cells.off[g.scope_cb[s]];
+      for (u64 p = g.scope_pair0[s]; p < g.scope_pair0[s + 1]; p++) {
+        if (slots) { snprintf(line, sizeof line, "%d\t", pass); out += line; }
+        snprintf(line, sizeof line, "%llu\t", (unsigned long long)shown); out += line; out += cb;
+        snprintf(line, sizeof line, "\t%llu\t%llu\t%u\t%u\t%u\t%u", (unsigned long long)o1[p], (unsigned long long)o2[p], f1[p], f2[p], l1[p], l2[p]); out += line;
+        if (slots) { slot(b1[p], l1[p]); slot(b2[p], l2[p]); }
+        out += '\n';
+      }
+      shown++;
+    }
+    return NB_OK;
+  });
   nbg::destroy(dev);
   if (rc) return rc;
   FILE* f = fopen(out_path, "wb"); if (!f) return fail(NB_ERR_IO, std::string("could not open ") + out_path);
-  u64 shown = 0;
-  for (u64 s = 0; s < g.n_scopes; s++) {
-    if (g.scope_pair0[s + 1] == g.scope_pair0[s]) continue;
-    const char* cb = cells.names.data() + cells.off[g.scope_cb[s]];
-    for (u64 p = g.scope_pair0[s]; p < g.scope_pair0[s + 1]; p++)
-      fprintf(f, "%llu\t%s\t%llu\t%llu\t%u\t%u\t%u\t%u\n", (unsigned long long)shown, cb, (unsigned long long)o1[p], (unsigned long long)o2[p], f1[p], f2[p], l1[p], l2[p]);
-    shown++;
-  }
-  if (fclose(f) != 0) return fail(NB_ERR_IO, std::string("short write on ") + out_path);
+  const bool ok = fwrite(out.data(), 1, out.size(), f) == out.size();
+  if (fclose(f) != 0 || !ok) return fail(NB_ERR_IO, std::string("short write on ") + out_path);
+  return NB_OK;
+}
+
+}  // namespace
+
+extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                              int strand_filter, const char* trim, int num_cores, int device) {
+  return process_bam_cells_any_order(input_file, reference_json, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, 0);
+}
+
+extern "C" int nb_process_bam_cells_any_order_budget(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
+                                                     int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes) {
+  return process_bam_cells_any_order(input_file, reference_json, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
+}
+
+extern "C" int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path) {
+  return dump_scopes_any_order(input_file, num_cores, device, 0, out_path, false);
+}
+
+extern "C" int nb_bam_dump_scopes_any_order_budget(const char* input_file, int num_cores, int device, uint64_t budget_bytes, const char* out_path) {
+  return dump_scopes_any_order(input_file, num_cores, device, budget_bytes, out_path, true);
+}
+
+extern "C" int nb_any_order_umi_bucket(const char* umi, uint32_t len, uint32_t* bucket) {
+  if (!umi || !bucket) return fail(NB_ERR_INVALID, "null argument");
+  u64 key;
+  if (!nbg::pack_umi(umi, len, key)) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(umi, len) + "\" cannot be packed into the exact device key");
+  *bucket = nbg::umi_bucket(key);
   return NB_OK;
 }

@@ -23,6 +23,18 @@ inline bool pack_umi(const char* s, u32 n, u64& key) {
   key = k; return true;
 }
 
+// Budget mode (nb_process_bam_cells_any_order_budget) splits the records into passes by UMI bucket: every record of a
+// (UMI, CB[..len-2]) scope has the same UMI, so any set of whole buckets groups on its own.  bucket = the top 16 bits of
+// the splitmix64 finalizer of the exact UMI key; host and device use this one definition.
+enum : u32 { N_BUCKETS = 1u << 16 };
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+inline u32 umi_bucket(u64 k) {
+  k ^= k >> 30; k *= 0xBF58476D1CE4E5B9ull; k ^= k >> 27; k *= 0x94D049BB133111EBull; k ^= k >> 31;
+  return (u32)(k >> 48);
+}
+
 // Pinned staging of one window's kept records.  Offsets are global: nib_off = byte offset of the record's first nibble byte
 // in the nibble store (its quals start at base offset 2 * nib_off of the qual store), name_off = offset in the name store.
 struct Stage {
@@ -41,7 +53,31 @@ void* stream_of(Device*);                                  // cudaStream_t: the 
 int sync(Device*);                                         // waits for everything queued on that stream
 // Waits until the staging slot's previous upload has run, sizes it for this window and fills rec0 / nib0 / name0.
 int stage(Device*, u64 n_rec, u64 n_nib, u64 n_name, Stage*& st);
-int upload(Device*);                                       // queues the copies of the staged window (plain cudaMemcpyAsync)
+// Queues the copies of the staged window (plain cudaMemcpyAsync).  reserve: with a budget, the bytes the grouping will
+// need on top of the store (group_reserve); a store array grows only so far that the store plus reserve stays in budget.
+int upload(Device*, u64 reserve = 0);
+
+// Device-memory budget.  Every cudaMalloc / cudaFree of this file goes through one counter (peak_bytes); with a budget B > 0
+// an allocation that would take the counter over B fails, and a store array that grows keeps old + new copies within B.
+void set_budget(Device*, u64 budget_bytes);
+u64 peak_bytes(Device*);
+// Drops the store and the pair arrays of the previous pass (after its batches ran): the next pass starts empty.
+int begin_pass(Device*);
+// Bytes group() allocates at its peak for n records and ncb CB ids: the sort and scope arrays plus the pair arrays (at most
+// one pair per record).
+u64 group_reserve(Device*, u64 n, u64 ncb);
+// Whether a store of R records, NB nibble bytes and NM name bytes, grown from the present arrays as upload() grows them,
+// and then `reserve` bytes more, stays within the budget at every moment.
+bool fits(Device*, u64 R, u64 NB, u64 NM, u64 reserve);
+// Keeps the records whose bucket is below hi, in their order, in place: nibbles, quals, names and per-record arrays move
+// down through one bounded scratch tile and the offsets are rebased.  Allocates within the budget.
+int compact(Device*, u32 hi);
+// The most device bytes a store of R / NB / NM grown from the present arrays to exactly what it needs, plus reserve, would
+// hold at any moment: what fits() must find within the budget.
+u64 need_bytes(Device*, u64 R, u64 NB, u64 NM, u64 reserve);
+// Shrinks every store array to its contents (plus the read-past padding) where the budget has room for the copy: arrays
+// that grew for records a compaction dropped stop holding room another array needs.
+int trim(Device*);
 
 struct Grouped {
   u64 n_records = 0, n_scopes = 0, n_pairs = 0;
@@ -54,6 +90,9 @@ int group(Device*, const std::vector<u32>& cb_rank, const std::vector<u32>& cb_p
 int batch(Device*, u64 p0, u64 p1, u64 scope0, u32 max_read_len, nb_batch& b);
 // Test hook: per pair the file ordinals of both slots, their flags and clipped lengths.
 int pairs_to_host(Device*, std::vector<u64>& ord1, std::vector<u64>& ord2, std::vector<u8>& f1, std::vector<u8>& f2, std::vector<u32>& l1, std::vector<u32>& l2);
+// Test hook: per pair the base offsets of both slots into the store, and the nibble and qual stores as they are now.
+int slots_to_host(Device*, std::vector<u64>& off1, std::vector<u64>& off2, std::vector<u8>& nib, std::vector<u8>& qual);
+u64 store_records(Device*);     // records in the store
 u64 store_bytes(Device*);       // device bytes of the record store (nibbles, quals, names, per-record keys)
 u64 group_bytes(Device*);       // device bytes of the sort, scope and pair arrays
 

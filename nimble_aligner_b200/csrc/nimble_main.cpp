@@ -1,6 +1,7 @@
 // nimble_main.cpp — `nimble` CLI with the arguments of /root/reference/src/bin/cli.yml:5-50 and the dispatch of
 // src/bin/main.rs:12-162, on top of the C ABI (include/nimble_b200.h).
 #include <algorithm>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -11,8 +12,20 @@
 
 static void die(const std::string& m) { fprintf(stderr, "%s\n", m.c_str()); exit(101); }  // a Rust panic exits 101
 
+// SIZE = decimal bytes with an optional K, M or G suffix (powers of 1024); 0 when malformed, zero or too large
+static uint64_t parse_size(const std::string& t) {
+  size_t n = 0; uint64_t v = 0;
+  while (n < t.size() && t[n] >= '0' && t[n] <= '9') { if (v > (UINT64_MAX - 9) / 10) return 0; v = v * 10 + (uint64_t)(t[n] - '0'); n++; }
+  if (n == 0) return 0;
+  int shift = 0;
+  if (n + 1 == t.size()) { const char c = t[n]; shift = c == 'K' ? 10 : c == 'M' ? 20 : c == 'G' ? 30 : -1; if (shift < 0) return 0; }
+  else if (n != t.size()) return 0;
+  if (v > (UINT64_MAX >> shift)) return 0;
+  return v << shift;
+}
+
 int main(int argc, char** argv) {
-  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false, any_order = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
+  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false, any_order = false; uint64_t device_budget = 0; bool have_budget = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
   std::vector<std::string>* cur = nullptr;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
@@ -29,6 +42,7 @@ int main(int argc, char** argv) {
     if (a == "--cell-matrix") { cur = &mats; have_mats = true; continue; }   // not in cli.yml: BAM mode, one directory per -r for a cell x feature matrix (10x v3 layout)
     if (a == "--no-rows") { no_rows = true; cur = nullptr; continue; }          // not in cli.yml: BAM mode, no TSV.gz rows (with --cell-matrix, without -o)
     if (a == "--any-order") { any_order = true; cur = nullptr; continue; }      // not in cli.yml: BAM mode, scopes from the tags of a BAM in any record order (with --cell-matrix --no-rows)
+    if (a == "--device-budget") { const std::string v = val("--device-budget"); device_budget = parse_size(v); have_budget = true; if (!device_budget) die("error: --device-budget needs a positive number of bytes with an optional K, M or G suffix, not '" + v + "'"); cur = nullptr; continue; }   // not in cli.yml: with --any-order, the device memory it may allocate
     if (a == "-h" || a == "--help") {
       printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"
              "  -d, --devices <list>          GPUs to use, \"0,1,...\" (default: NB_DEVICES, else 0)\n"
@@ -37,13 +51,16 @@ int main(int argc, char** argv) {
              "                                (matrix.mtx.gz UMIs, reads.mtx.gz reads, features.tsv.gz, barcodes.tsv.gz)\n"
              "      --no-rows                 BAM input with --cell-matrix: skip the TSV.gz rows (no --output)\n"
              "      --any-order               BAM input with --cell-matrix --no-rows: records in any order (e.g. position-sorted);\n"
-             "                                (UMI, CB) scopes are formed on the GPU, no sort by UB needed (no -p)\n");
+             "                                (UMI, CB) scopes are formed on the GPU, no sort by UB needed (no -p)\n"
+             "      --device-budget <size>    with --any-order: device memory it may allocate, bytes or with a K/M/G suffix\n"
+             "                                (powers of 1024); records that do not fit take more passes over the file\n");
       return 0;
     }
     if (a == "-V" || a == "--version") { printf("nimble 0.8.0\n"); return 0; }
     if (!cur) die("error: Found argument '" + a + "' which wasn't expected, or isn't valid in this context");
     cur->push_back(a);
   }
+  if (have_budget && !any_order) die("error: --device-budget needs --any-order");
   if (any_order && (!have_mats || !no_rows)) die("error: --any-order needs --cell-matrix and --no-rows (it writes no TSV rows)");
   if (any_order && force_paired) die("error: --any-order cannot pair mates (-p): the mates of a position-sorted file are not neighbours");
   if (no_rows && !outs.empty()) die("error: --no-rows writes no TSV: leave out --output");
@@ -78,7 +95,8 @@ int main(int argc, char** argv) {
     if (rc != NB_OK) die(nb_last_error());
   } else if (ends(lower, ".bam")) {
     printf("Processing as BAM file\n");
-    int rc = any_order ? nb_process_bam_cells_any_order(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0])
+    int rc = any_order ? (have_budget ? nb_process_bam_cells_any_order_budget(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], device_budget)
+                                      : nb_process_bam_cells_any_order(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0]))
                        : nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
     if (rc != NB_OK) die(nb_last_error());
   } else die("Unsupported file format: " + (lower.find('.') == std::string::npos ? std::string("") : lower.substr(lower.rfind('.') + 1)));
