@@ -214,6 +214,9 @@ int nb_counts_finalize(nb_ctx*, nb_counts* out);
 /* device copies of the row columns of the last nb_counts_finalize (row_scope u32[n], row_callset u32[n], row_count i64[n]),
  * valid until the next finalize / reset: lets a multi-GPU host reduce per-cell tables without a host round trip */
 int nb_counts_device_rows(nb_ctx*, const void** row_scope, const void** row_callset, const void** row_count, uint64_t* n_rows);
+/* device copy of the last nb_counts_finalize's slot_to_callset (u32[n_slots], nb_pair_result.callset -> callset id, 0xFFFFFFFF
+ * for a slot without one), on the context's stream; valid until the next finalize / reset, like nb_counts_device_rows */
+int nb_counts_device_slot_map(nb_ctx*, const void** slot_to_callset, uint64_t* n_slots);
 int nb_counts_reset(nb_ctx*);
 uint32_t nb_library_n_groups(const nb_library*);
 const char* nb_library_group_name(const nb_library*, uint32_t group);
@@ -385,8 +388,8 @@ int nb_process_bam_cells(const char* input_file, const char* const* reference_js
  * Every kept record's nibbles, quals and name stay in device memory (the store; NB_BAM_STATS=1 prints its size) and the
  * scoped batches point into it.  Refused: a kept record with an empty UMI string, or a UMI that the exact device key cannot
  * hold (more than 21 characters, or a character outside ACGTN): NB_ERR_UNSUPPORTED naming it; a store that does not fit:
- * NB_ERR_CUDA with the bytes needed.  There is no force_bam_paired (mates of a position-sorted file are not neighbours) and
- * no TSV rows (they need every record's 38 fields on the host). */
+ * NB_ERR_CUDA with the bytes needed.  There is no force_bam_paired (mates of a position-sorted file are not neighbours); the
+ * TSV rows of such a file come from nb_process_bam_rows_any_order. */
 int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                    int strand_filter, const char* trim, int num_cores, int device);
 /* test hook: the device grouping of nb_process_bam_cells_any_order, one line per pair:
@@ -415,6 +418,24 @@ int nb_bam_dump_scopes_any_order_budget(const char* input_file, int num_cores, i
 /* test hook (host-only): the UMI bucket (0..65535) of nb_process_bam_cells_any_order_budget for a UMI string, so that tests
  * can check the bucket function against a restatement; NB_ERR_UNSUPPORTED when the exact key cannot hold it */
 int nb_any_order_umi_bucket(const char* umi, uint32_t len, uint32_t* bucket);
+/* The TSV.gz rows of nb_process_bam (one output_paths[i] per reference library) from a BAM in ANY record order.  The file
+ * is G's rows: G = the kept records (steps 1-2 of nb_process_bam_cells_any_order) in (UMI, CB) order followed by one sentinel
+ * scope, and gunzip(output) equals gunzip of nb_process_bam on G byte for byte: the header, the scopes in that order, in a
+ * scope the count rows in finalize order and then the zero rows in pair order, the same representative pairs, zero-row
+ * rule, reason and score columns and SKIP_ALIGN values.  No row at all: an empty gzip stream.  The gzip member layout is not
+ * part of the output.  Every kept record's 36 reported metadata values are formatted on the host threads and kept in device
+ * memory next to its bases (a fourth byte store); the rows of each batch are assembled on the GPU and only deflated and
+ * written on the host.  budget_bytes (0: none) is the budget of nb_process_bam_cells_any_order_budget, which also covers the
+ * metadata store, the per-pair results and the row buffer; with P passes the file is the header, then the rows of each
+ * pass in pass order, a pass's rows being G's rows of its UMI buckets in G's order.  NB_BAM_ROWS_BUFFER_KB=N sets the cap of
+ * the device row buffer (default 64 MB); a batch whose rows exceed it is written in chunks of whole scopes.  The passes are
+ * planned with the row buffer, the row stage's scratch and 64 KB of callset texts reserved; a batch whose callset texts
+ * need more, or a scope whose rows exceed the buffer (it gets a grown buffer of its own), allocates the rest within the budget
+ * when it comes.  Refused as in nb_process_bam_cells_any_order (no force_bam_paired), and such an allocation that does not fit
+ * the budget: NB_ERR_CUDA naming the bytes.  NB_BAM_STATS=1 adds rows, row bytes, row chunks, the metadata store and text
+ * bytes, the row buffer, the device peak and the row build and deflate times to the any-order stats line. */
+int nb_process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
+                                  int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes);
 /* host-only: a cell x feature matrix in the 10x v3 layout that Seurat's Read10X and scanpy's read_10x_mtx load, into `dir`
  * (created when missing; its parent must exist): matrix.mtx.gz (Matrix Market coordinate integer, features x barcodes, UMI
  * counts, 1-based lines sorted by barcode then feature), reads.mtx.gz (the same coordinates with the read counts),

@@ -155,6 +155,7 @@ _SIGS = {
     "nb_process_bam_cells_any_order_budget": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_uint64]),
     "nb_bam_dump_scopes_any_order_budget": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_uint64, C.c_char_p]),
     "nb_any_order_umi_bucket": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint32)]),
+    "nb_process_bam_rows_any_order": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_uint64]),
     "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
     "nb_cells_reset": (C.c_int, [C.c_void_p]),
@@ -674,19 +675,28 @@ def process_bam(input_file, reference_json_paths, output_paths, strand_filter="u
                 matrix_dirs=None, any_order=False, device_budget=None):
     """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156).
     matrix_dirs=[dir per library]: also a cell x feature matrix per library (nb_process_bam_cells); output_paths=None with
-    matrix_dirs: no TSV rows at all.  any_order=True: the matrices only (output_paths=None, matrix_dirs required, no
-    force_bam_paired) from a BAM in any record order, scopes formed on the GPU (nb_process_bam_cells_any_order).
+    matrix_dirs: no TSV rows at all.  any_order=True: from a BAM in any record order, scopes formed on the GPU, no
+    force_bam_paired; either the TSV rows (output_paths, matrix_dirs=None: nb_process_bam_rows_any_order, the grouped
+    driver's rows on the (UMI, CB)-sorted file) or the matrices (output_paths=None, matrix_dirs: nb_process_bam_cells_any_order).
     device_budget=bytes (any_order only): the device memory that path may allocate; it takes passes over the file by UMI
-    bucket when the records do not fit (nb_process_bam_cells_any_order_budget), and writes the same bytes."""
+    bucket when the records do not fit (nb_process_bam_cells_any_order_budget), and writes the same bytes (the rows: the
+    same lines, pass by pass)."""
     if device_budget is not None:
         _check_budget(device_budget, any_order)
     if any_order:
-        if output_paths is not None:
-            raise NbError(-1, "any_order writes no TSV rows: pass output_paths=None")
-        if matrix_dirs is None:
-            raise NbError(-1, "any_order needs matrix_dirs")
+        if output_paths is not None and matrix_dirs is not None:
+            raise NbError(-1, "any_order writes either TSV rows (output_paths) or matrices (matrix_dirs), not both: run the two modes separately")
+        if output_paths is None and matrix_dirs is None:
+            raise NbError(-1, "any_order needs output_paths or matrix_dirs")
         if force_bam_paired:
             raise NbError(-1, "any_order cannot pair mates (force_bam_paired): the mates of a position-sorted file are not neighbours")
+        if output_paths is not None:
+            if len(output_paths) != len(reference_json_paths):
+                raise NbError(-1, "any_order needs one output path per reference library")
+            _ck(lib().nb_process_bam_rows_any_order(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths), len(reference_json_paths),
+                                                    CHEM[strand_filter], trim.encode() if trim else None, num_cores, device,
+                                                    int(device_budget) if device_budget is not None else 0))
+            return
         if device_budget is not None:
             _ck(lib().nb_process_bam_cells_any_order_budget(str(input_file).encode(), _strs(reference_json_paths), _strs(matrix_dirs), len(reference_json_paths),
                                                             CHEM[strand_filter], trim.encode() if trim else None, num_cores, device, int(device_budget)))

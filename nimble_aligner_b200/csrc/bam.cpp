@@ -638,8 +638,10 @@ inline char* put_u32(char* p, u32 v) { char t[10]; int n = 0; do { t[n++] = (cha
 inline char* put_i32(char* p, i32 v) { if (v < 0) { *p++ = '-'; return put_u32(p, (u32)(-(i64)v)); } return put_u32(p, (u32)v); }
 inline char* put_bool(char* p, bool b) { if (b) { memcpy(p, "true", 4); return p + 4; } memcpy(p, "false", 5); return p + 5; }
 
-// the 36 reported metadata values of one record, tab-joined, straight into the output line (same values as parse_fields)
-void append_data_values(const Rec& r, std::string& s) {
+// the 36 reported metadata values of one record, tab-joined, straight into the output line (same values as parse_fields);
+// skip_align = false leaves out the last one (SKIP_ALIGN and its tab): the any-order rows store that text once per record
+// and add the value of the slot it fills
+void append_data_values(const Rec& r, std::string& s, bool skip_align = true) {
   const char* zv[40]; u32 zl[40]; u64 seen = 0, isz = 0;
   { const u8* a = r.aux(); const u8* e = r.end();
     while (a + 3 <= e) {   // same rule as Rec::aux_z: the FIRST aux with the tag decides, a string only when NUL-terminated inside the record
@@ -654,7 +656,7 @@ void append_data_values(const Rec& r, std::string& s) {
   const size_t old = s.size(); s.resize(old + bound);
   char* p = &s[old];
   const u32 fl = r.flag(); const bool rev = fl & 16, paired = fl & 1, unm = fl & 4, munm = fl & 8, mrev = fl & 32, first = fl & 64;
-  for (int i = 0; i < 38; i++) {
+  for (int i = 0; i < (skip_align ? 38 : 37); i++) {
     if (i == 1 || i == 15) continue;
     if (i) *p++ = '\t';
     if (i == 37 && r.skip_align >= 0) { if (r.skip_align) { memcpy(p, "TRUE", 4); p += 4; } else { memcpy(p, "FALSE", 5); p += 5; } continue; }
@@ -696,14 +698,32 @@ inline void field0(const Rec& r, const char*& ptr, u32& len) {
 std::string data_header(const char* prefix) { std::string s; for (int i = 0; i < 38; i++) { if (i == 1 || i == 15) continue; if (!s.empty()) s += "\t"; s += prefix; s += "_"; s += FIELDS[i]; } return s; }
 
 // one gzip member (concatenated members are one valid .gz stream): lets the writer threads deflate independently
-bool gzip_member(const std::string& text, int level, std::string& out) {
+bool gzip_member(const char* text, size_t len, int level, std::string& out) {
   z_stream zs; memset(&zs, 0, sizeof zs);
   if (deflateInit2(&zs, level, Z_DEFLATED, 15 + 16, 8, Z_DEFAULT_STRATEGY) != Z_OK) return false;
-  out.resize(deflateBound(&zs, (uLong)text.size()) + 32);
-  zs.next_in = (Bytef*)text.data(); zs.avail_in = (uInt)text.size(); zs.next_out = (Bytef*)&out[0]; zs.avail_out = (uInt)out.size();
+  out.resize(deflateBound(&zs, (uLong)len) + 32);
+  zs.next_in = (Bytef*)text; zs.avail_in = (uInt)len; zs.next_out = (Bytef*)&out[0]; zs.avail_out = (uInt)out.size();
   int rc = deflate(&zs, Z_FINISH); size_t n = zs.total_out; deflateEnd(&zs);
   if (rc != Z_STREAM_END) return false;
   out.resize(n); return true;
+}
+bool gzip_member(const std::string& text, int level, std::string& out) { return gzip_member(text.data(), text.size(), level, out); }
+
+// The rows' gzip members (nb_process_bam and nb_process_bam_rows_any_order): a part of the rows with the rows' own
+// compressor, or zlib at NB_BAM_GZ_LEVEL=1..9; the header member before the first rows; an empty stream when there is no row.
+int rows_gz_level() { int v = 0; if (const char* e = getenv("NB_BAM_GZ_LEVEL")) v = atoi(e); return v >= 1 && v <= 9 ? v : 0; }
+bool rows_member(const char* text, size_t n, int level, std::string& out) {
+  if (level) return gzip_member(text, n, level, out);
+  std::unique_ptr<nbz::FastDeflate> fd(new nbz::FastDeflate()); out.reserve(n / 16 + 4096); fd->gzip_member((const u8*)text, n, out); return true;
+}
+int write_rows_header(FILE* f, int level) {
+  const std::string header = "nimble_features\tnimble_score\t" + data_header("r1") + "\t" + data_header("r2") + "\tr1_filter_forward\tr1_forward_score\tr1_filter_reverse\tr1_reverse_score\tr2_filter_forward\tr2_forward_score\tr2_filter_reverse\tr2_reverse_score\ttriage_reason\taligndirection\n";
+  std::string hm; if (!gzip_member(header, level ? level : 2, hm) || fwrite(hm.data(), 1, hm.size(), f) != hm.size()) return fail(NB_ERR_IO, "short write on the TSV");
+  return NB_OK;
+}
+int write_rows_empty(FILE* f, int level) {   // no row at all: an empty gzip stream, like the reference's untouched GzEncoder
+  std::string em; if (!gzip_member(std::string(), level ? level : 2, em) || fwrite(em.data(), 1, em.size(), f) != em.size()) return fail(NB_ERR_IO, "short write on the TSV");
+  return NB_OK;
 }
 
 // Run-wide cell barcodes (nb_process_bam_cells): id = order of first appearance.  The fill stage hashes the CB of every
@@ -853,8 +873,7 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
   else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = (size_t)strtoull(e2, nullptr, 10) << 20;
   if (rc != NB_OK) { cleanup(); return rc; }
   const size_t BATCH_PAIRS = 1u << 20;
-  int GZ_LEVEL = 0;   // 0: the rows' own compressor (deflate_fast.hpp); NB_BAM_GZ_LEVEL=1..9: zlib at that level (the rows are the same, the members smaller or slower to make)
-  if (const char* e = getenv("NB_BAM_GZ_LEVEL")) { int v = atoi(e); if (v >= 1 && v <= 9) GZ_LEVEL = v; }
+  const int GZ_LEVEL = rows_gz_level();   // 0: the rows' own compressor (deflate_fast.hpp); NB_BAM_GZ_LEVEL=1..9: zlib at that level (the rows are the same, the members smaller or slower to make)
   // Three stages run concurrently on consecutive batches: (F) the host threads fill batch k+1 into pinned buffers,
   // (D) the device aligns batch k and its counts are finalized, (R) the host threads format + gzip the rows of batch k-1.
   struct Pinned { u8* p = nullptr; size_t cap = 0; int ensure(size_t n) { if (n <= cap) return NB_OK; nb_host_free(p); cap = n + n / 4 + 4096; p = (u8*)nb_host_alloc(cap); if (!p) { cap = 0; return fail(NB_ERR_CUDA, "pinned host allocation failed"); } return NB_OK; } ~Pinned() { nb_host_free(p); } };
@@ -1000,14 +1019,11 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
         }
         if (!text.empty()) {
           wrote[t] = 1;
-          if (GZ_LEVEL) { if (!gzip_member(text, GZ_LEVEL, member[t])) bad[t] = 1; }
-          else { std::unique_ptr<nbz::FastDeflate> fd(new nbz::FastDeflate()); member[t].reserve(text.size() / 16 + 4096); fd->gzip_member((const u8*)text.data(), text.size(), member[t]); }
+          if (!rows_member(text.data(), text.size(), GZ_LEVEL, member[t])) bad[t] = 1;
         }
       } });
     bool any = false; for (int t = 0; t < parts; t++) { if (bad[t]) return fail(NB_ERR_IO, "gzip of the TSV rows failed"); any = any || wrote[t]; }
-    if (any && first_write[li]) {
-      std::string header = "nimble_features\tnimble_score\t" + data_header("r1") + "\t" + data_header("r2") + "\tr1_filter_forward\tr1_forward_score\tr1_filter_reverse\tr1_reverse_score\tr2_filter_forward\tr2_forward_score\tr2_filter_reverse\tr2_reverse_score\ttriage_reason\taligndirection\n";
-      std::string hm; if (!gzip_member(header, GZ_LEVEL ? GZ_LEVEL : 2, hm) || fwrite(hm.data(), 1, hm.size(), outs[li]) != hm.size()) return fail(NB_ERR_IO, "short write on the TSV"); first_write[li] = false; }
+    if (any && first_write[li]) { const int e = write_rows_header(outs[li], GZ_LEVEL); if (e) return e; first_write[li] = false; }
     for (int t = 0; t < parts; t++) if (wrote[t] && fwrite(member[t].data(), 1, member[t].size(), outs[li]) != member[t].size()) return fail(NB_ERR_IO, "short write on the TSV");
     ns_rows += (u64)((now() - tb) * 1e9);
     return NB_OK;
@@ -1077,7 +1093,7 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
   }
   t_load = t_prod; t_group = 0;
   t_fill = ns_fill.load() * 1e-9; t_rows = ns_rows.load() * 1e-9;
-  if (rc == NB_OK && want_rows) for (u32 li = 0; li < n_refs; li++) if (first_write[li]) { std::string em; if (!gzip_member(std::string(), GZ_LEVEL ? GZ_LEVEL : 2, em) || fwrite(em.data(), 1, em.size(), outs[li]) != em.size()) rc = fail(NB_ERR_IO, "short write on the TSV"); }   // no row at all: an empty gzip stream, like the reference's untouched GzEncoder
+  if (rc == NB_OK && want_rows) for (u32 li = 0; li < n_refs && rc == NB_OK; li++) if (first_write[li]) rc = write_rows_empty(outs[li], GZ_LEVEL);
   if (rc == NB_OK && want_cells) {
     const double tc = now();
     std::vector<const char*> bc(cells.size()); for (size_t i = 0; i < bc.size(); i++) bc[i] = cells.names.data() + cells.off[i];
@@ -1150,14 +1166,14 @@ extern "C" int nb_bam_dump_groups(const char* input_file, int force_bam_paired, 
 namespace {
 
 struct AnyOrderLoad {   // what the producer saw (NB_BAM_STATS)
-  u64 n_records = 0, n_kept = 0; u32 max_len = 1; size_t peak_window = 0; double t_wait = 0;
+  u64 n_records = 0, n_kept = 0, meta_text = 0; u32 max_len = 1; size_t peak_window = 0; double t_wait = 0, t_meta = 0;   // meta_text: M(r) bytes staged
 };
 
 // Budget mode: a pass stages the records of UMI buckets [lo, hi) (nbg::umi_bucket); hi starts at N_BUCKETS and only falls.
 struct Passes {
-  u64 budget = 0; int pass = 0; u32 lo = 0, hi = nbg::N_BUCKETS; u64 evictions = 0;
-  std::vector<u64> b_rec, b_nib, b_name;   // what this pass has staged (or is about to) of every bucket
-  void begin(u32 lo_) { lo = lo_; hi = nbg::N_BUCKETS; b_rec.assign(nbg::N_BUCKETS, 0); b_nib.assign(nbg::N_BUCKETS, 0); b_name.assign(nbg::N_BUCKETS, 0); }
+  u64 budget = 0; int pass = 0; u32 lo = 0, hi = nbg::N_BUCKETS; u64 evictions = 0; bool rows = false;
+  std::vector<u64> b_rec, b_nib, b_name, b_meta;   // what this pass has staged (or is about to) of every bucket
+  void begin(u32 lo_) { lo = lo_; hi = nbg::N_BUCKETS; b_rec.assign(nbg::N_BUCKETS, 0); b_nib.assign(nbg::N_BUCKETS, 0); b_name.assign(nbg::N_BUCKETS, 0); b_meta.assign(nbg::N_BUCKETS, 0); }
 };
 
 // Before a window is staged in budget mode (the per-bucket counts already hold it): when the store plus the window plus the
@@ -1166,11 +1182,12 @@ struct Passes {
 int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
   lowered = false;
   const u32 lo = P.lo, hi = P.hi;
-  std::vector<u64> R(hi - lo + 1, 0), NB(hi - lo + 1, 0), NM(hi - lo + 1, 0);   // sums over buckets [lo, lo + k)
-  for (u32 k = 0; k < hi - lo; k++) { R[k + 1] = R[k] + P.b_rec[lo + k]; NB[k + 1] = NB[k] + P.b_nib[lo + k]; NM[k + 1] = NM[k] + P.b_name[lo + k]; }
-  auto fits = [&](u32 k) { return nbg::fits(dev, R[k], NB[k], NM[k], nbg::group_reserve(dev, R[k], ncb)); };
+  std::vector<u64> R(hi - lo + 1, 0), NB(hi - lo + 1, 0), NM(hi - lo + 1, 0), NT(hi - lo + 1, 0);   // sums over buckets [lo, lo + k)
+  for (u32 k = 0; k < hi - lo; k++) { R[k + 1] = R[k] + P.b_rec[lo + k]; NB[k + 1] = NB[k] + P.b_nib[lo + k]; NM[k + 1] = NM[k] + P.b_name[lo + k]; NT[k + 1] = NT[k] + P.b_meta[lo + k]; }
+  auto fits = [&](u32 k) { return nbg::fits(dev, R[k], NB[k], NM[k], NT[k], nbg::group_reserve(dev, R[k], ncb)); };
   if (fits(hi - lo)) return NB_OK;
-  auto under_target = [&](u32 k) { return 3 * NB[k] + NM[k] + 43 * R[k] + nbg::group_reserve(dev, R[k], ncb) <= P.budget / 4 * 3 && fits(k); };
+  const u64 per_rec = P.rows ? 43 + 16 : 43;   // store bytes per record (rows: metadata offset, length and field-0 length)
+  auto under_target = [&](u32 k) { return 3 * NB[k] + NM[k] + NT[k] + per_rec * R[k] + nbg::group_reserve(dev, R[k], ncb) <= P.budget / 4 * 3 && fits(k); };
   u32 a = 0, b = hi - lo;   // the largest k in (0, hi - lo) under the target: ok(a) (or a = 0), !ok(b)
   while (b - a > 1) { const u32 m = a + (b - a) / 2; if (under_target(m)) a = m; else b = m; }
   bool compacted = false;
@@ -1180,7 +1197,7 @@ int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
       if (nbg::store_records(dev)) { const int rc = nbg::compact(dev, lo + 1); if (rc) return rc; P.evictions++; compacted = true; }
       { const int rc = nbg::trim(dev); if (rc) return rc; }
       if (!fits(1)) {
-        const u64 need = nbg::need_bytes(dev, R[1], NB[1], NM[1], nbg::group_reserve(dev, R[1], ncb));
+        const u64 need = nbg::need_bytes(dev, R[1], NB[1], NM[1], NT[1], nbg::group_reserve(dev, R[1], ncb));
         return fail(NB_ERR_CUDA, "the device budget of " + std::to_string(P.budget) + " bytes is too small: UMI bucket " + std::to_string(lo) + " needs " + std::to_string(need) +
                                  " bytes (" + std::to_string(R[1]) + " records with their grouping arrays)");
       }
@@ -1189,7 +1206,7 @@ int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
   }
   const u32 nh = lo + a;
   if (!compacted && nbg::store_records(dev)) { const int rc = nbg::compact(dev, nh); if (rc) return rc; P.evictions++; }   // an eviction: records already on the device leave
-  for (u32 x = nh; x < hi; x++) P.b_rec[x] = P.b_nib[x] = P.b_name[x] = 0;
+  for (u32 x = nh; x < hi; x++) P.b_rec[x] = P.b_nib[x] = P.b_name[x] = P.b_meta[x] = 0;
   P.hi = nh; lowered = true;
   return NB_OK;
 }
@@ -1197,8 +1214,9 @@ int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
 // Streams the file window by window: the kept records of every window (SortedBamReader::fill_buffer's filters, in its
 // order) are staged into pinned memory on all threads and uploaded into the device store while the next window inflates.
 // cells: every kept record's full CB, ids in order of first appearance.  With P (budget mode) only the records of buckets
-// [P->lo, P->hi) are staged, and passes after the first only look the CBs up.
-int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, Passes* P = nullptr) {
+// [P->lo, P->hi) are staged, and passes after the first only look the CBs up.  rows: every staged record also gets its
+// metadata text M(r) (append_data_values without SKIP_ALIGN) and the length of its field 0, formatted on the host threads.
+int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, bool rows, Passes* P = nullptr) {
   auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   Bgzf z; int rc = z.open(input_file); if (rc) return rc;
   RawBuf data; size_t len = 0; bool eof = false, header_done = false;
@@ -1249,35 +1267,54 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
       if (kind == 3) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)");
       if (kind == 4) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see"); }
     for (int t = 0; t < T; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
+    // rows: M(r) of the kept records, back to back per thread slice (the slices of every parallel_ranges(T, n) below)
+    std::vector<std::string> mt(rows ? T : 0); std::vector<u32> mlen(rows ? n : 0), f0l(rows ? n : 0); std::vector<u64> met(T + 1, 0);
+    if (rows) {
+      const double tf = now();
+      parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
+        std::string& o = mt[t]; u64 m = 0;
+        for (size_t i = a; i < b; i++) if (keep[i]) {
+          const size_t at = o.size(); append_data_values(all[i], o, false); mlen[i] = (u32)(o.size() - at); m += mlen[i];
+          const char* q; u32 l; field0(all[i], q, l); f0l[i] = l;
+        }
+        met[t + 1] = m;
+      });
+      st.t_meta += now() - tf;
+    }
     if (P) {
-      for (size_t i = 0; i < n; i++) if (keep[i]) { const u32 bk = bucket[i]; P->b_rec[bk]++; P->b_nib[bk] += (all[i].l_seq() + 1) / 2; P->b_name[bk] += all[i].qname_len(); }
+      for (size_t i = 0; i < n; i++) if (keep[i]) { const u32 bk = bucket[i]; P->b_rec[bk]++; P->b_nib[bk] += (all[i].l_seq() + 1) / 2; P->b_name[bk] += all[i].qname_len(); if (rows) P->b_meta[bk] += mlen[i]; }
       bool lowered = false;
       rc = plan_window(dev, *P, cells.size(), lowered); if (rc) return rc;
       if (lowered) parallel_ranges(T, n, [&](size_t a, size_t b, int t) {   // drop this window's records at or above the new hi
-        u64 c = 0, nb_ = 0, nm = 0;
+        u64 c = 0, nb_ = 0, nm = 0, mm = 0;
         for (size_t i = a; i < b; i++) {
           if (keep[i] && bucket[i] >= P->hi) keep[i] = 0;
-          if (keep[i]) { c++; nb_ += (all[i].l_seq() + 1) / 2; nm += all[i].qname_len(); }
+          if (keep[i]) { c++; nb_ += (all[i].l_seq() + 1) / 2; nm += all[i].qname_len(); if (rows) mm += mlen[i]; }
         }
-        cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm;
+        cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm; met[t + 1] = mm;
       });
     }
-    for (int t = 0; t < T; t++) { cnt[t + 1] += cnt[t]; nib[t + 1] += nib[t]; nam[t + 1] += nam[t]; st.max_len = std::max(st.max_len, mx[t]); }
+    for (int t = 0; t < T; t++) { cnt[t + 1] += cnt[t]; nib[t + 1] += nib[t]; nam[t + 1] += nam[t]; met[t + 1] += met[t]; st.max_len = std::max(st.max_len, mx[t]); }
     const double tw = now();
     nbg::Stage* sg = nullptr;
-    rc = nbg::stage(dev, cnt[T], nib[T], nam[T], sg); if (rc) return rc;
+    rc = nbg::stage(dev, cnt[T], nib[T], nam[T], met[T], sg); if (rc) return rc;
+    st.meta_text += met[T];
     st.t_wait += now() - tw;
     const u64 ord0 = st.n_records;
     parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
-      u64 k = cnt[t], bo = nib[t], no = nam[t];
-      for (size_t i = a; i < b; i++) if (keep[i]) {
-        const Rec& r = all[i]; const u32 l = r.l_seq(), nbytes = (l + 1) / 2, ql = r.qname_len();
-        memcpy(sg->nib + bo, r.seq4(), nbytes);
-        memcpy(sg->qual + 2 * bo, r.qual(), l);   // one qual byte per base, at the base's offset
-        memcpy(sg->name + no, r.qname_ptr(), ql);
-        sg->umi[k] = umi[i]; sg->cb[k] = cb[i]; sg->nib_off[k] = sg->nib0 + bo; sg->lseq[k] = l; sg->flag[k] = (u16)r.flag();
-        sg->name_off[k] = sg->name0 + no; sg->name_len[k] = (u8)ql; sg->ordinal[k] = ord0 + i;
-        k++; bo += nbytes; no += ql;
+      u64 k = cnt[t], bo = nib[t], no = nam[t], mo = met[t]; size_t src = 0;   // src: this slice's read position in mt[t]
+      for (size_t i = a; i < b; i++) {
+        if (keep[i]) {
+          const Rec& r = all[i]; const u32 l = r.l_seq(), nbytes = (l + 1) / 2, ql = r.qname_len();
+          memcpy(sg->nib + bo, r.seq4(), nbytes);
+          memcpy(sg->qual + 2 * bo, r.qual(), l);   // one qual byte per base, at the base's offset
+          memcpy(sg->name + no, r.qname_ptr(), ql);
+          sg->umi[k] = umi[i]; sg->cb[k] = cb[i]; sg->nib_off[k] = sg->nib0 + bo; sg->lseq[k] = l; sg->flag[k] = (u16)r.flag();
+          sg->name_off[k] = sg->name0 + no; sg->name_len[k] = (u8)ql; sg->ordinal[k] = ord0 + i;
+          if (rows) { memcpy(sg->meta + mo, mt[t].data() + src, mlen[i]); sg->meta_off[k] = sg->meta0 + mo; sg->meta_len[k] = mlen[i]; sg->f0_len[k] = f0l[i]; mo += mlen[i]; }
+          k++; bo += nbytes; no += ql;
+        }
+        if (rows) src += mlen[i];   // (a record dropped by a lowered hi was formatted too)
       } });
     rc = nbg::upload(dev, P ? nbg::group_reserve(dev, nbg::store_records(dev) + cnt[T], cells.size()) : 0); if (rc) return rc;
     st.n_records += n; st.n_kept += cnt[T];
@@ -1303,23 +1340,23 @@ int any_order_group(nbg::Device* dev, const CellDict& cells, nbg::Grouped& g) {
 // What a run in any record order did over all its passes (NB_BAM_STATS).
 struct AnyOrderRun {
   AnyOrderLoad ld;                       // the first pass's producer (every pass reads the same records)
-  int passes = 0; u64 evictions = 0, n_kept = 0, n_scopes = 0, n_pairs = 0;
+  int passes = 0; u64 evictions = 0, n_kept = 0, n_scopes = 0, n_pairs = 0, meta_text = 0;   // meta_text: the M(r) text of the records staged in all passes (dropped ones included)
   std::vector<double> t_windows; double t_group = 0;
 };
 
 // The passes over the file: one without a budget; with one, each pass takes the UMI buckets from where the previous one
 // stopped up to the hi its windows left.  After each pass's grouping: on_pass(pass, grouped, max_read_len) aligns it.
 template <class F>
-int any_order_passes(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, u64 budget, CellDict& cells, AnyOrderRun& run, F on_pass) {
+int any_order_passes(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, u64 budget, bool rows, CellDict& cells, AnyOrderRun& run, F on_pass) {
   auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  Passes P; P.budget = budget;
-  nbg::set_budget(dev, budget);
+  Passes P; P.budget = budget; P.rows = rows;
+  nbg::set_budget(dev, budget); nbg::set_rows(dev, rows);
   for (u32 lo = 0;;) {
     int rc = NB_OK;
     if (budget) { P.begin(lo); if (P.pass) rc = nbg::begin_pass(dev); }
     const double t0 = now();
     AnyOrderLoad ld;
-    if (rc == NB_OK) rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld, budget ? &P : nullptr);
+    if (rc == NB_OK) rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld, rows, budget ? &P : nullptr);
     if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); ld.t_wait += now() - tw; }
     const double t1 = now(); run.t_windows.push_back(t1 - t0);
     nbg::Grouped g;
@@ -1328,8 +1365,8 @@ int any_order_passes(const char* input_file, int threads, size_t window_bytes, n
     if (rc) return rc;
     if (P.pass == 0) run.ld = ld;
     else if (ld.n_records != run.ld.n_records) return fail(NB_ERR_IO, std::string("the input changed between passes: ") + input_file);
-    else { run.ld.t_wait += ld.t_wait; run.ld.peak_window = std::max(run.ld.peak_window, ld.peak_window); }
-    run.passes++; run.n_kept += g.n_records; run.n_scopes += g.n_scopes; run.n_pairs += g.n_pairs;
+    else { run.ld.t_wait += ld.t_wait; run.ld.t_meta += ld.t_meta; run.ld.peak_window = std::max(run.ld.peak_window, ld.peak_window); }
+    run.passes++; run.meta_text += ld.meta_text; run.n_kept += g.n_records; run.n_scopes += g.n_scopes; run.n_pairs += g.n_pairs;
     rc = on_pass(P.pass, (const nbg::Grouped&)g, run.ld.max_len); if (rc) return rc;
     if (!budget || P.hi == nbg::N_BUCKETS) break;
     lo = P.hi; P.pass++;
@@ -1345,6 +1382,46 @@ size_t any_order_window_bytes() {
   return window_bytes;
 }
 
+// The device store and one library context per reference of an any-order run, all on the store's stream (the batches'
+// scope ids are written on it).
+struct AnyOrderSetup {
+  nbg::Device* dev = nullptr; u32 n = 0;
+  std::vector<nb_library*> libs; std::vector<nb_index*> idx; std::vector<nb_ctx*> ctx;
+  ~AnyOrderSetup() { for (u32 i = 0; i < n; i++) { nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } nbg::destroy(dev); }
+  int open(const char* const* reference_json, uint32_t n_refs, int strand_filter, const char* trim, int threads, int device) {
+    std::vector<std::pair<u64, double>> trims;
+    if (trim && *trim) {   // src/bin/main.rs:74-93
+      std::string t(trim); size_t p = 0;
+      while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
+      if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
+    }
+    n = n_refs; libs.assign(n, nullptr); idx.assign(n, nullptr); ctx.assign(n, nullptr);
+    int rc = nbg::create(device, &dev);
+    for (u32 i = 0; i < n && rc == NB_OK; i++) {
+      rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
+      if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
+      if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);
+      if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nbg::stream_of(dev), &ctx[i]);
+      if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);
+    }
+    return rc;
+  }
+};
+
+// The NB_BAM_STATS line of an any-order run; rows: the rows mode's fields, which go before the budget's
+void any_order_stats(const AnyOrderRun& run, nbg::Device* dev, u64 budget, u64 n_batches, size_t n_barcodes, double t_setup, double t_align, double t_roll, double t_out, double t_total, const std::string& rows) {
+  double hwm_mb = 0; if (FILE* stf = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, stf)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(stf); }
+  const AnyOrderLoad& ld = run.ld;
+  double t_win = 0; std::string per_pass;
+  for (double t : run.t_windows) { t_win += t; char b[32]; snprintf(b, sizeof b, "%s%.2fs", per_pass.empty() ? "" : "/", t); per_pass += b; }
+  std::string extra = rows;
+  if (budget) { char b[256]; snprintf(b, sizeof b, ", budget %llu bytes, passes %d, evictions %llu, peak device bytes %llu, windows per pass ", (unsigned long long)budget, run.passes, (unsigned long long)run.evictions, (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0)); extra += b + per_pass; }
+  fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB%s\n",
+          (unsigned long long)ld.n_records, (unsigned long long)run.n_kept, (unsigned long long)run.n_scopes, (unsigned long long)run.n_pairs, (unsigned long long)n_batches, n_barcodes,
+          t_setup, t_win, ld.t_wait, ld.peak_window / 1048576.0, run.t_group, t_align, t_roll, t_out, t_total,
+          (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb, extra.c_str());
+}
+
 int process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                 int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
   if (!input_file || !reference_json || !matrix_dirs || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / matrix directory pair");
@@ -1352,24 +1429,10 @@ int process_bam_cells_any_order(const char* input_file, const char* const* refer
   const double t_start = now();
   const int threads = std::max(1, num_cores);
   const size_t window_bytes = any_order_window_bytes();
-  std::vector<std::pair<u64, double>> trims;
-  if (trim && *trim) {   // src/bin/main.rs:74-93
-    std::string t(trim); size_t p = 0;
-    while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
-    if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
-  }
-  nbg::Device* dev = nullptr;
-  std::vector<nb_library*> libs(n_refs, nullptr); std::vector<nb_index*> idx(n_refs, nullptr); std::vector<nb_ctx*> ctx(n_refs, nullptr);
-  auto cleanup = [&]() { for (u32 i = 0; i < n_refs; i++) { nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } nbg::destroy(dev); };
-  int rc = nbg::create(device, &dev);
-  for (u32 i = 0; i < n_refs && rc == NB_OK; i++) {
-    rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
-    if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
-    if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);
-    if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nbg::stream_of(dev), &ctx[i]);   // one stream: the batches' scope ids are written on it
-    if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);
-  }
-  if (rc != NB_OK) { cleanup(); return rc; }
+  AnyOrderSetup S;
+  int rc = S.open(reference_json, n_refs, strand_filter, trim, threads, device);
+  if (rc != NB_OK) return rc;
+  nbg::Device* dev = S.dev; std::vector<nb_library*>& libs = S.libs; std::vector<nb_ctx*>& ctx = S.ctx;
   const double t_setup = now();
   CellDict cells; AnyOrderRun run;
   // barcodes: the cells of the scopes that have pairs, in order of first appearance.  Without a budget the one pass knows
@@ -1378,7 +1441,7 @@ int process_bam_cells_any_order(const char* input_file, const char* const* refer
   std::vector<u32> remap; std::vector<u8> used; std::vector<const char*> bc;
   const u64 BATCH_PAIRS = 1u << 20;   // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
   double t_align = 0, t_roll = 0; u64 n_batches = 0;
-  rc = any_order_passes(input_file, threads, window_bytes, dev, budget, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
+  rc = any_order_passes(input_file, threads, window_bytes, dev, budget, false, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
     std::vector<u32> cell_of_scope(g.n_scopes, 0);   // scopes without pairs get cell 0 (no rows)
     if (!budget) {
       remap.assign(cells.size(), NONE32);
@@ -1425,19 +1488,113 @@ int process_bam_cells_any_order(const char* input_file, const char* const* refer
     if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size());
   }
   const double t_end = now();
+  if (getenv("NB_BAM_STATS")) any_order_stats(run, dev, budget, n_batches, bc.size(), t_setup - t_start, t_align, t_roll, t_end - t_aligned, t_end - t_start, std::string());
+  return rc;
+}
+
+// The TSV.gz rows of the grouped driver on G (nb_process_bam_rows_any_order): every batch of every library is aligned
+// into device result buffers and its rows are assembled on the device (nbg::rows_build); the host only deflates each
+// chunk, cut at row boundaries into parts compressed on its threads, and writes the members in order.  The deflate of a
+// chunk runs while the device builds the next one.
+int process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
+                               int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
+  if (!input_file || !reference_json || !output_paths || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / output pair");
+  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  const double t_start = now();
+  const int threads = std::max(1, num_cores);
+  const int GZ_LEVEL = rows_gz_level();
+  AnyOrderSetup S;
+  int rc = S.open(reference_json, n_refs, strand_filter, trim, threads, device);
+  if (rc != NB_OK) return rc;
+  nbg::Device* dev = S.dev;
+  std::vector<FILE*> outs(n_refs, nullptr); std::vector<bool> first_write(n_refs, true);
+  struct Closer { std::vector<FILE*>& f; ~Closer() { for (FILE* x : f) if (x) fclose(x); } } closer{outs};
+  for (u32 i = 0; i < n_refs && rc == NB_OK; i++) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
+  if (rc != NB_OK) return rc;
+  const double t_setup = now();
+  std::vector<std::string> reasons(256); for (int r = 0; r < 256; r++) reasons[r] = nb_reason_str(r);
+  // the deflate + write of one chunk, on its own thread while the device goes on; errors come back through the future
+  typedef std::pair<int, std::string> Res;
+  std::future<Res> fut; double t_deflate = 0;
+  auto join = [&]() -> int { if (!fut.valid()) return NB_OK; Res r = fut.get(); if (r.first) set_error(r.second); return r.first; };
+  auto write_chunk = [&, threads, GZ_LEVEL](FILE* f, const char* p, u64 n) -> Res {
+    const double t0 = now();
+    const u64 PART = (u64)1 << 20;
+    std::vector<u64> cut(1, 0);   // parts of about PART bytes, each ending at the end of a row
+    while (cut.back() < n) { u64 e = cut.back() + PART; if (e >= n) e = n; else { const char* nl = (const char*)memchr(p + e - 1, '\n', n - (e - 1)); e = nl ? (u64)(nl - p) + 1 : n; } cut.push_back(e); }
+    const size_t parts = cut.size() - 1;
+    std::vector<std::string> member(parts); std::vector<char> bad(parts, 0); std::atomic<size_t> next(0);
+    parallel_ranges((int)std::min<size_t>(threads, parts), (size_t)std::min<size_t>(threads, parts), [&](size_t, size_t, int) {
+      for (size_t i; (i = next.fetch_add(1)) < parts;) if (!rows_member(p + cut[i], cut[i + 1] - cut[i], GZ_LEVEL, member[i])) bad[i] = 1; });
+    for (size_t i = 0; i < parts; i++) {
+      if (bad[i]) return Res(NB_ERR_IO, "gzip of the TSV rows failed");
+      if (fwrite(member[i].data(), 1, member[i].size(), f) != member[i].size()) return Res(NB_ERR_IO, "short write on the TSV");
+    }
+    t_deflate += now() - t0;
+    return Res(NB_OK, std::string());
+  };
+  CellDict cells; AnyOrderRun run; nbg::RowsStats rst;
+  const u64 BATCH_PAIRS = 1u << 20;   // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
+  double t_align = 0; u64 n_batches = 0;
+  std::string feats; std::vector<u64> feat_off;
+  rc = any_order_passes(input_file, threads, any_order_window_bytes(), dev, budget, true, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
+    std::vector<std::pair<u64, u64>> batches; u64 maxp = 0;
+    for (u64 s0 = 0; s0 < g.n_scopes;) {
+      u64 s1 = s0 + 1;
+      while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
+      if (g.scope_pair0[s1] > g.scope_pair0[s0]) { batches.push_back({s0, s1}); maxp = std::max(maxp, g.scope_pair0[s1] - g.scope_pair0[s0]); }
+      s0 = s1;
+    }
+    if (batches.empty()) return NB_OK;
+    int e = nbg::rows_begin(dev, maxp); if (e) return e;
+    nb_read_result* rres = nullptr; nb_pair_result* pres = nullptr; nbg::rows_results(dev, &rres, &pres);
+    for (const auto& bt : batches) {
+      const u64 s0 = bt.first, p0 = g.scope_pair0[s0], p1 = g.scope_pair0[bt.second];
+      n_batches++;
+      nb_batch b; e = nbg::batch(dev, p0, p1, s0, max_len, b); if (e) return e;
+      for (u32 li = 0; li < n_refs; li++) {
+        const double tb = now();
+        e = nb_counts_reset(S.ctx[li]);
+        if (e == NB_OK) e = nb_ctx_set_option(S.ctx[li], "max_batch_pairs", p1 - p0);
+        if (e == NB_OK) e = nb_align_batch(S.ctx[li], &b, rres, pres);
+        nb_counts cts;
+        if (e == NB_OK) e = nb_counts_finalize(S.ctx[li], &cts);
+        nbg::RowsBatch RB; RB.p0 = p0; RB.p1 = p1; RB.reasons = &reasons;
+        if (e == NB_OK) e = nb_counts_device_rows(S.ctx[li], &RB.row_scope, &RB.row_callset, &RB.row_count, &RB.n_rows);
+        if (e == NB_OK) e = nb_counts_device_slot_map(S.ctx[li], &RB.slot_map, &RB.n_slots);
+        t_align += now() - tb;
+        if (e) return e;
+        if (!RB.n_rows) continue;
+        // the text of every callset of this finalize: its group names joined by ','
+        feats.clear(); feat_off.assign(1, 0);
+        for (u64 c = 0; c < cts.n_callsets; c++) {
+          for (u64 k = cts.callset_off[c]; k < cts.callset_off[c + 1]; k++) { if (k > cts.callset_off[c]) feats += ','; feats += nb_library_group_name(S.libs[li], cts.callset_items[k]); }
+          feat_off.push_back(feats.size());
+        }
+        RB.feats = &feats; RB.feat_off = &feat_off;
+        FILE* f = outs[li];
+        e = nbg::rows_build(dev, RB, [&, f, li](const char* p, u64 n) -> int {
+          int er = join(); if (er) return er;
+          if (first_write[li]) { er = write_rows_header(f, GZ_LEVEL); if (er) return er; first_write[li] = false; }
+          fut = std::async(std::launch::async, [&write_chunk, f, p, n]() { return write_chunk(f, p, n); });
+          return NB_OK;
+        }, rst);
+        if (e) return e;
+      }
+    }
+    return NB_OK;
+  });
+  { const int er = join(); if (er && rc == NB_OK) rc = er; }
+  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) if (first_write[li]) rc = write_rows_empty(outs[li], GZ_LEVEL);
+  for (u32 li = 0; li < n_refs; li++) { if (outs[li] && fclose(outs[li]) != 0 && rc == NB_OK) rc = fail(NB_ERR_IO, std::string("short write on ") + output_paths[li]); outs[li] = nullptr; }
+  const double t_end = now();
   if (getenv("NB_BAM_STATS")) {
-    double hwm_mb = 0; if (FILE* stf = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, stf)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(stf); }
-    const AnyOrderLoad& ld = run.ld;
-    double t_win = 0; std::string per_pass;
-    for (double t : run.t_windows) { t_win += t; char b[32]; snprintf(b, sizeof b, "%s%.2fs", per_pass.empty() ? "" : "/", t); per_pass += b; }
-    std::string extra;
-    if (budget) { char b[256]; snprintf(b, sizeof b, ", budget %llu bytes, passes %d, evictions %llu, peak device bytes %llu, windows per pass ", (unsigned long long)budget, run.passes, (unsigned long long)run.evictions, (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0)); extra = b + per_pass; }
-    fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB%s\n",
-            (unsigned long long)ld.n_records, (unsigned long long)run.n_kept, (unsigned long long)run.n_scopes, (unsigned long long)run.n_pairs, (unsigned long long)n_batches, bc.size(),
-            t_setup - t_start, t_win, ld.t_wait, ld.peak_window / 1048576.0, run.t_group, t_align, t_roll, t_end - t_aligned, t_end - t_start,
-            (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb, extra.c_str());
+    char b[1024];
+    snprintf(b, sizeof b, ", rows %llu, row bytes %llu, row chunks %llu (at most %llu per batch), metadata %llu bytes, metadata text %llu bytes, metadata formatting %.2fs, row buffer %llu bytes, device peak %llu bytes, device row build %.3fs, deflate+write %.3fs",
+             (unsigned long long)rst.rows, (unsigned long long)rst.bytes, (unsigned long long)rst.chunks, (unsigned long long)rst.max_chunks, (unsigned long long)(dev ? nbg::meta_bytes(dev) : 0),
+             (unsigned long long)run.meta_text, run.ld.t_meta, (unsigned long long)nbg::rows_buffer_cap(), (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0), rst.t_device, t_deflate);
+    any_order_stats(run, dev, budget, n_batches, 0, t_setup - t_start, t_align, 0, 0, t_end - t_start, b);
   }
-  cleanup();
   return rc;
 }
 
@@ -1451,7 +1608,7 @@ int dump_scopes_any_order(const char* input_file, int num_cores, int device, u64
   CellDict cells; AnyOrderRun run;
   std::string out; u64 shown = 0;
   static const char* SEQ = "=ACMGRSVTWYHKDBN"; static const char* H = "0123456789abcdef";
-  if (rc == NB_OK) rc = any_order_passes(input_file, std::max(1, num_cores), any_order_window_bytes(), dev, budget, cells, run, [&](int pass, const nbg::Grouped& g, u32) -> int {
+  if (rc == NB_OK) rc = any_order_passes(input_file, std::max(1, num_cores), any_order_window_bytes(), dev, budget, false, cells, run, [&](int pass, const nbg::Grouped& g, u32) -> int {
     std::vector<u64> o1, o2, b1, b2; std::vector<u8> f1, f2, nib, qual; std::vector<u32> l1, l2;
     int e = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
     if (e == NB_OK && slots) e = nbg::slots_to_host(dev, b1, b2, nib, qual);
@@ -1493,6 +1650,11 @@ extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char
 extern "C" int nb_process_bam_cells_any_order_budget(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                                      int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes) {
   return process_bam_cells_any_order(input_file, reference_json, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
+}
+
+extern "C" int nb_process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
+                                             int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes) {
+  return process_bam_rows_any_order(input_file, reference_json, output_paths, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
 }
 
 extern "C" int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path) {

@@ -3,6 +3,9 @@
 // (UMI, CB), cuts the (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into
 // the store.  Host-only declarations (bam.cpp includes them; bam_group.cu implements them).
 #pragma once
+#include <functional>
+#include <string>
+
 #include "host.hpp"
 
 namespace nbg {
@@ -37,12 +40,15 @@ inline u32 umi_bucket(u64 k) {
 
 // Pinned staging of one window's kept records.  Offsets are global: nib_off = byte offset of the record's first nibble byte
 // in the nibble store (its quals start at base offset 2 * nib_off of the qual store), name_off = offset in the name store.
+// With rows (set_rows): meta_off / meta_len = the record's metadata text M(r) in the metadata store (its 36 reported values
+// without SKIP_ALIGN, tab-joined), f0_len = the length of its field 0, the prefix of M(r).
 struct Stage {
-  u64 rec0 = 0, nib0 = 0, name0 = 0;        // store sizes before this window (the first record / byte this window adds)
-  u64 n_rec = 0, n_nib = 0, n_name = 0;     // what this window adds
+  u64 rec0 = 0, nib0 = 0, name0 = 0, meta0 = 0;        // store sizes before this window (the first record / byte this window adds)
+  u64 n_rec = 0, n_nib = 0, n_name = 0, n_meta = 0;    // what this window adds
   u8* nib = nullptr; u8* qual = nullptr; char* name = nullptr;
   u64* umi = nullptr; u32* cb = nullptr; u64* nib_off = nullptr; u32* lseq = nullptr; u16* flag = nullptr; u64* name_off = nullptr; u8* name_len = nullptr;
   u64* ordinal = nullptr;
+  char* meta = nullptr; u64* meta_off = nullptr; u32* meta_len = nullptr; u32* f0_len = nullptr;
 };
 
 struct Device;   // the store, the grouping buffers and the stream (bam_group.cu)
@@ -51,8 +57,10 @@ int create(int device, Device** out);
 void destroy(Device*);
 void* stream_of(Device*);                                  // cudaStream_t: the library contexts are created on it
 int sync(Device*);                                         // waits for everything queued on that stream
-// Waits until the staging slot's previous upload has run, sizes it for this window and fills rec0 / nib0 / name0.
-int stage(Device*, u64 n_rec, u64 n_nib, u64 n_name, Stage*& st);
+// Rows mode (before the first stage): every record also carries its metadata text, and group_reserve() includes the row stage.
+void set_rows(Device*, bool rows);
+// Waits until the staging slot's previous upload has run, sizes it for this window and fills rec0 / nib0 / name0 / meta0.
+int stage(Device*, u64 n_rec, u64 n_nib, u64 n_name, u64 n_meta, Stage*& st);
 // Queues the copies of the staged window (plain cudaMemcpyAsync).  reserve: with a budget, the bytes the grouping will
 // need on top of the store (group_reserve); a store array grows only so far that the store plus reserve stays in budget.
 int upload(Device*, u64 reserve = 0);
@@ -66,15 +74,15 @@ int begin_pass(Device*);
 // Bytes group() allocates at its peak for n records and ncb CB ids: the sort and scope arrays plus the pair arrays (at most
 // one pair per record).
 u64 group_reserve(Device*, u64 n, u64 ncb);
-// Whether a store of R records, NB nibble bytes and NM name bytes, grown from the present arrays as upload() grows them,
-// and then `reserve` bytes more, stays within the budget at every moment.
-bool fits(Device*, u64 R, u64 NB, u64 NM, u64 reserve);
-// Keeps the records whose bucket is below hi, in their order, in place: nibbles, quals, names and per-record arrays move
-// down through one bounded scratch tile and the offsets are rebased.  Allocates within the budget.
+// Whether a store of R records, NB nibble bytes, NM name bytes and NT metadata bytes, grown from the present arrays as
+// upload() grows them, and then `reserve` bytes more, stays within the budget at every moment.
+bool fits(Device*, u64 R, u64 NB, u64 NM, u64 NT, u64 reserve);
+// Keeps the records whose bucket is below hi, in their order, in place: nibbles, quals, names, metadata and per-record
+// arrays move down through one bounded scratch tile and the offsets are rebased.  Allocates within the budget.
 int compact(Device*, u32 hi);
 // The most device bytes a store of R / NB / NM grown from the present arrays to exactly what it needs, plus reserve, would
 // hold at any moment: what fits() must find within the budget.
-u64 need_bytes(Device*, u64 R, u64 NB, u64 NM, u64 reserve);
+u64 need_bytes(Device*, u64 R, u64 NB, u64 NM, u64 NT, u64 reserve);
 // Shrinks every store array to its contents (plus the read-past padding) where the budget has room for the copy: arrays
 // that grew for records a compaction dropped stop holding room another array needs.
 int trim(Device*);
@@ -95,5 +103,31 @@ int slots_to_host(Device*, std::vector<u64>& off1, std::vector<u64>& off2, std::
 u64 store_records(Device*);     // records in the store
 u64 store_bytes(Device*);       // device bytes of the record store (nibbles, quals, names, per-record keys)
 u64 group_bytes(Device*);       // device bytes of the sort, scope and pair arrays
+u64 meta_bytes(Device*);        // device bytes of the metadata store (rows mode; part of store_bytes)
+
+// ---- the rows of nb_process_bam_rows_any_order, assembled on the device
+// Row buffer cap: NB_BAM_ROWS_BUFFER_KB, default 64 MB; independent of the batch size.
+u64 rows_buffer_cap();
+// After group(): allocates, within the budget, the per-read / per-pair result buffers and the row stage's scratch for
+// batches of up to max_batch_pairs pairs, and the row buffer.  Released by begin_pass / destroy.  group_reserve() holds
+// these, 64 KB of callset texts and the reason table; texts beyond that and a row buffer grown for an oversize scope are
+// allocated by rows_build within the budget but outside the reserve (NB_ERR_CUDA naming the bytes when they do not fit).
+int rows_begin(Device*, u64 max_batch_pairs);
+// The device result buffers nb_align_batch writes for a batch of this device (NB_MEM_DEVICE).
+void rows_results(Device*, nb_read_result** rres, nb_pair_result** pres);
+// What one batch of one library gives the row stage, after nb_counts_finalize: its pairs [p0, p1) of the grouping, the
+// device count rows (nb_counts_device_rows), the device slot map (nb_counts_device_slot_map) and the text of every callset
+// id of that finalize (group names joined by ','): feats[feat_off[c] .. feat_off[c + 1]).  reasons[r] = nb_reason_str(r).
+struct RowsBatch {
+  u64 p0 = 0, p1 = 0;
+  const void* row_scope = nullptr; const void* row_callset = nullptr; const void* row_count = nullptr; u64 n_rows = 0;
+  const void* slot_map = nullptr; u64 n_slots = 0;
+  const std::string* feats = nullptr; const std::vector<u64>* feat_off = nullptr; const std::vector<std::string>* reasons = nullptr;
+};
+struct RowsStats { u64 rows = 0, bytes = 0, chunks = 0, batches = 0, max_chunks = 0; double t_device = 0; };
+// Plans the batch's rows on the device (representatives, zero rows, byte lengths, CUB scans), then writes them in chunks of
+// whole scopes into the row buffer; each chunk is copied into pinned memory (two buffers, alternating) and handed to
+// sink(bytes, n) in order.  The sink may go on reading a buffer until its next call returns, not longer.
+int rows_build(Device*, const RowsBatch&, const std::function<int(const char*, u64)>& sink, RowsStats& st);
 
 }  // namespace nbg

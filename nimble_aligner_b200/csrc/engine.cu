@@ -117,6 +117,7 @@ struct nb_ctx {
   double map_ms = 0; u64 map_launches = 0, map_reads = 0, all_launches = 0;
   // results
   std::vector<u32> cs_items, slot_dense, dense_prev, dense_ids; std::vector<u64> cs_off;   // dense_prev: the slots slot_dense held last time (only those are reset); dense_ids: slot of callset i, uploaded to fill d_dense on the device
+  bool dense_dev = false;   // d_dense holds slot_dense of the last finalize
   u32* h_csr = nullptr; size_t h_csr_cap = 0;   // pinned: compacted dictionary rows of the last finalize
   u8* h_rows = nullptr; size_t h_rows_cap = 0; u64 n_rows_dev = 0;   // pinned: row_scope | row_callset | row_count of the last finalize
   DBuf d_rowwork, d_rowout, d_dense, d_denseids;
@@ -571,11 +572,22 @@ static int dense_reduce_scatter(nb_ctx* c, void* dense, u64 chunk);
 // dense_cells > 0 (nb_merge_scoped): the (cell, callset) rows of all ranks are summed through a dense [cells x callsets]
 // table (all-reduce over NCCL) before they are read back; 0: this context's own rows.  shard: reduce-scatter instead — every
 // rank keeps (and reads back) the rows of its own range of cells only
+// d_dense = the host slot -> callset table of the last finalize (c->slot_dense), filled on the device by a scatter of the
+// callset id list
+static int upload_slot_map(nb_ctx* c, cudaStream_t s) {
+  const std::vector<u32>& dense = c->slot_dense;
+  CK(c->d_dense.ensure(dense.size() * 4, s)); CK(c->d_denseids.ensure(c->dense_ids.size() * 4 + 16, s));
+  CK(cudaMemsetAsync(c->d_dense.p, 0xFF, dense.size() * 4, s));
+  if (!c->dense_ids.empty()) { CK(cudaMemcpyAsync(c->d_denseids.p, c->dense_ids.data(), c->dense_ids.size() * 4, cudaMemcpyHostToDevice, s)); nbk::launch_dense_scatter((const u32*)c->d_denseids.p, c->dense_ids.size(), (u32*)c->d_dense.p, s); c->all_launches++; }
+  c->dense_dev = true;
+  return NB_OK;
+}
+
 static int finalize_impl(nb_ctx* c, nb_counts* out, u64 dense_cells, bool shard = false) {
   if (!c || !out) return fail(NB_ERR_INVALID, "null argument");
   CK(cudaSetDevice(c->device));
   memset(out, 0, sizeof *out);
-  c->cs_items.clear(); c->cs_off.assign(1, 0);
+  c->cs_items.clear(); c->cs_off.assign(1, 0); c->dense_dev = false;
   if (!c->tables_ready) { out->callset_off = c->cs_off.data(); return NB_OK; }
   cudaStream_t s = c->stream;
   Tables t = make_tables(c);
@@ -649,12 +661,7 @@ static int finalize_impl(nb_ctx* c, nb_counts* out, u64 dense_cells, bool shard 
       { u64 at = part[t]; for (u64 i = q0; i < q1; i++) { const u32* r = &csr[(size_t)slots[i] * cw]; for (u32 k = 0; k < r[1]; k++) c->cs_items[at + k] = r[4 + k]; at += r[1]; c->cs_off[i + 1] = at; } }
     });
   }
-  auto upload_dense = [&]() -> int {
-    CK(c->d_dense.ensure(dense.size() * 4, s)); CK(c->d_denseids.ensure(c->dense_ids.size() * 4 + 16, s));
-    CK(cudaMemsetAsync(c->d_dense.p, 0xFF, dense.size() * 4, s));
-    if (!c->dense_ids.empty()) { CK(cudaMemcpyAsync(c->d_denseids.p, c->dense_ids.data(), c->dense_ids.size() * 4, cudaMemcpyHostToDevice, s)); nbk::launch_dense_scatter((const u32*)c->d_denseids.p, c->dense_ids.size(), (u32*)c->d_dense.p, s); c->all_launches++; }
-    return NB_OK;
-  };
+  auto upload_dense = [&]() -> int { return upload_slot_map(c, s); };
   if (fstats) ft[3] = fnow();
   // rows ordered by (cell, callset): remap to dense callset ids, radix sort and split on the device (kernels.cu), then one
   // copy into pinned memory — the table can hold millions of (cell, callset) rows
@@ -728,6 +735,16 @@ int nb_counts_device_rows(nb_ctx* c, const void** row_scope, const void** row_ca
   if (!c->folded && c->mode != 1) return fail(NB_ERR_INVALID, "no finalized counts");
   u64 n = c->n_rows_dev; *n_rows = n;
   *row_scope = c->d_rowout.p; *row_callset = (const u32*)c->d_rowout.p + n; *row_count = (const char*)c->d_rowout.p + 8 * n;
+  return NB_OK;
+}
+
+int nb_counts_device_slot_map(nb_ctx* c, const void** slot_to_callset, uint64_t* n_slots) {
+  if (!c || !slot_to_callset || !n_slots) return fail(NB_ERR_INVALID, "null argument");
+  if (!c->folded && c->mode != 1) return fail(NB_ERR_INVALID, "no finalized counts");
+  CK(cudaSetDevice(c->device));
+  // finalize uploads the table only when it has rows to sort: otherwise fill it here (on the context's stream)
+  if (!c->dense_dev) { const int rc = upload_slot_map(c, c->stream); if (rc) return rc; }
+  *slot_to_callset = c->d_dense.p; *n_slots = c->slot_dense.size();
   return NB_OK;
 }
 

@@ -41,7 +41,7 @@ int main(int argc, char** argv) {
     if (a == "--index-cache") { const std::string dir = val("--index-cache"); setenv("NB_INDEX_CACHE", dir.c_str(), 1); cur = nullptr; continue; }   // not in cli.yml: keep each library's index in <dir>/<key>.nbix (default: NB_INDEX_CACHE, else rebuilt per run like the reference)
     if (a == "--cell-matrix") { cur = &mats; have_mats = true; continue; }   // not in cli.yml: BAM mode, one directory per -r for a cell x feature matrix (10x v3 layout)
     if (a == "--no-rows") { no_rows = true; cur = nullptr; continue; }          // not in cli.yml: BAM mode, no TSV.gz rows (with --cell-matrix, without -o)
-    if (a == "--any-order") { any_order = true; cur = nullptr; continue; }      // not in cli.yml: BAM mode, scopes from the tags of a BAM in any record order (with --cell-matrix --no-rows)
+    if (a == "--any-order") { any_order = true; cur = nullptr; continue; }      // not in cli.yml: BAM mode, scopes from the tags of a BAM in any record order (-o rows, or --cell-matrix --no-rows)
     if (a == "--device-budget") { const std::string v = val("--device-budget"); device_budget = parse_size(v); have_budget = true; if (!device_budget) die("error: --device-budget needs a positive number of bytes with an optional K, M or G suffix, not '" + v + "'"); cur = nullptr; continue; }   // not in cli.yml: with --any-order, the device memory it may allocate
     if (a == "-h" || a == "--help") {
       printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"
@@ -50,8 +50,9 @@ int main(int argc, char** argv) {
              "      --cell-matrix <dir>...    BAM input: also write a cell x feature matrix per reference library into <dir>\n"
              "                                (matrix.mtx.gz UMIs, reads.mtx.gz reads, features.tsv.gz, barcodes.tsv.gz)\n"
              "      --no-rows                 BAM input with --cell-matrix: skip the TSV.gz rows (no --output)\n"
-             "      --any-order               BAM input with --cell-matrix --no-rows: records in any order (e.g. position-sorted);\n"
-             "                                (UMI, CB) scopes are formed on the GPU, no sort by UB needed (no -p)\n"
+             "      --any-order               BAM input in any record order (e.g. position-sorted), no sort by UB needed (no -p):\n"
+             "                                with --output, the TSV.gz rows in any order (assembled on the GPU); with\n"
+             "                                --cell-matrix --no-rows, the matrices; (UMI, CB) scopes are formed on the GPU\n"
              "      --device-budget <size>    with --any-order: device memory it may allocate, bytes or with a K/M/G suffix\n"
              "                                (powers of 1024); records that do not fit take more passes over the file\n");
       return 0;
@@ -61,7 +62,7 @@ int main(int argc, char** argv) {
     cur->push_back(a);
   }
   if (have_budget && !any_order) die("error: --device-budget needs --any-order");
-  if (any_order && (!have_mats || !no_rows)) die("error: --any-order needs --cell-matrix and --no-rows (it writes no TSV rows)");
+  if (any_order && have_mats && !no_rows) die("error: --any-order writes either the TSV rows (--output) or the cell matrices (--cell-matrix --no-rows), not both: run the two modes separately");
   if (any_order && force_paired) die("error: --any-order cannot pair mates (-p): the mates of a position-sorted file are not neighbours");
   if (no_rows && !outs.empty()) die("error: --no-rows writes no TSV: leave out --output");
   if (no_rows && !have_mats) die("error: --no-rows needs --cell-matrix (there would be nothing to write)");
@@ -95,7 +96,8 @@ int main(int argc, char** argv) {
     if (rc != NB_OK) die(nb_last_error());
   } else if (ends(lower, ".bam")) {
     printf("Processing as BAM file\n");
-    int rc = any_order ? (have_budget ? nb_process_bam_cells_any_order_budget(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], device_budget)
+    int rc = (any_order && !have_mats) ? nb_process_bam_rows_any_order(in[0], r.data(), o.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], have_budget ? device_budget : 0)
+           : any_order ? (have_budget ? nb_process_bam_cells_any_order_budget(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], device_budget)
                                       : nb_process_bam_cells_any_order(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0]))
                        : nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
     if (rc != NB_OK) die(nb_last_error());

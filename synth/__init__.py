@@ -36,7 +36,7 @@ def lib():
         L.synth_write_fastq.restype = C.c_uint64
         L.synth_write_fastq.argtypes = [C.c_char_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.synth_write_bam.restype = C.c_uint64
-        L.synth_write_bam.argtypes = [C.c_char_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int]
+        L.synth_write_bam.argtypes = [C.c_char_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_void_p]
         L.synth_encode_2bit.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_int]
         _lib = L
     return _lib
@@ -107,10 +107,12 @@ def umi_reads(library, first_group, n_groups, seed=2345, L=91, n_cells=8000, err
     return dict(bases=bases, qual=qual, off=off, cell=cell, scope=scope, sizes=sizes, n_reads=int(tot))
 
 
-def write_umi_bam(path, u, L=91, first_scope=0, level=1, threads=8):
-    """Writes the records of `umi_reads` as a 10x-style unaligned BAM (threaded BGZF).  Returns the file size."""
+def write_umi_bam(path, u, L=91, first_scope=0, level=1, threads=8, name_ids=None):
+    """Writes the records of `umi_reads` as a 10x-style unaligned BAM (threaded BGZF).  Record i is named r<i>, or
+    r<name_ids[i]> (a uint64 array) so that a reordering of another file's records keeps their names.  Returns the file size."""
+    ids = None if name_ids is None else np.ascontiguousarray(name_ids, dtype=np.uint64)
     n = lib().synth_write_bam(str(path).encode(), u["n_reads"], L, u["bases"].ctypes.data, u["qual"].ctypes.data, u["cell"].ctypes.data, u["scope"].ctypes.data,
-                              first_scope, level, threads)
+                              first_scope, level, threads, None if ids is None else ids.ctypes.data)
     if not n:
         raise IOError("could not write %s" % path)
     return int(n)

@@ -105,9 +105,10 @@ void synth_umi_reads(u64 seed, u64 first, u64 n, const u32* sizes, const u64* re
 
 // 10x-style unaligned BAM of the reads synth_umi_reads made (C3): one record per read, tags CB:Z:<16 nt>-1, UB:Z / UR:Z
 // <12 nt> derived from the cell / group ids, CR, NH:i, RE:A; records of one group are contiguous (what UMIReader needs,
-// src/parse/sorted_bam_reader.rs:84).  BGZF blocks are deflated on `threads` threads.  Returns bytes written, 0 on error.
+// src/parse/sorted_bam_reader.rs:84).  BGZF blocks are deflated on `threads` threads.  Record i is named r<name_id[i]>, or
+// r<i> when name_id is null (so a reordering of another file's records can keep their names).  Returns bytes written, 0 on error.
 static void nt_of(u64 v, int n, char* o) { for (int i = 0; i < n; i++) { o[i] = B[v & 3]; v >>= 2; } }
-u64 synth_write_bam(const char* path, u64 n_reads, u32 L, const char* bases, const u8* qual, const u32* cell, const u32* scope, u32 first_scope, int level, int threads) {
+u64 synth_write_bam(const char* path, u64 n_reads, u32 L, const char* bases, const u8* qual, const u32* cell, const u32* scope, u32 first_scope, int level, int threads, const u64* name_id) {
   static const u8 code[256] = {0};
   u8 c4[256]; memset(c4, 15, 256); c4[(u8)'A'] = 1; c4[(u8)'C'] = 2; c4[(u8)'G'] = 4; c4[(u8)'T'] = 8; (void)code;
   const char* text = "@HD\tVN:1.6\tSO:unsorted\n@SQ\tSN:chr1\tLN:100000000\n";
@@ -122,7 +123,7 @@ u64 synth_write_bam(const char* path, u64 n_reads, u32 L, const char* bases, con
     d.reserve((y - x) * rec_guess);
     char name[32], cb[20], ub[13];
     for (u64 i = x; i < y; i++) {
-      int ln = snprintf(name, sizeof name, "r%llu", (unsigned long long)i) + 1;
+      int ln = snprintf(name, sizeof name, "r%llu", (unsigned long long)(name_id ? name_id[i] : i)) + 1;
       u64 g = (u64)scope[i] + first_scope; nt_of(g * 0x9E3779B97F4A7C15ULL >> 8, 12, ub); ub[12] = 0; nt_of((u64)cell[i] * 0xD1B54A32D192ED03ULL >> 8, 16, cb); cb[16] = '-'; cb[17] = '1'; cb[18] = 0;
       std::string aux; aux.append("CBZ"); aux.append(cb, 19); aux.append("CRZ"); aux.append(cb, 16); aux.push_back(0); aux.append("UBZ"); aux.append(ub, 13); aux.append("URZ"); aux.append(ub, 13);
       aux.append("NHC"); aux.push_back(1); aux.append("REA"); aux.push_back('E');
