@@ -256,6 +256,26 @@ void parallel_ranges(int threads, size_t n, const std::function<void(size_t, siz
   for (auto& x : th) x.join();
 }
 
+// wall clock of the NB_BAM_STATS phase times
+double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+
+// peak resident set of THIS process image (the high-water mark belongs to the mm, so unlike ru_maxrss it does not start at
+// the forking parent's size)
+double peak_rss_mb() {
+  double mb = 0;
+  if (FILE* st = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, st)) if (!strncmp(line, "VmHWM:", 6)) mb = strtod(line + 6, nullptr) / 1024.0; fclose(st); }
+  return mb;
+}
+
+// inflated bytes per window of the streaming producers: NB_BAM_WINDOW_KB or NB_BAM_WINDOW_MB (tests use small ones), default
+// 256 MB, at least 64 KiB
+size_t window_bytes() {
+  size_t w = (size_t)256 << 20;
+  if (const char* e = getenv("NB_BAM_WINDOW_KB")) w = (size_t)strtoull(e, nullptr, 10) << 10;
+  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) w = (size_t)strtoull(e2, nullptr, 10) << 20;
+  return std::max<size_t>(w, 1 << 16);
+}
+
 // ------------------------------------------------------------------ SortedBamReader (src/parse/sorted_bam_reader.rs)
 inline bool same(const char* a, u32 al, const char* b, u32 bl) { return al == bl && (al == 0 || !memcmp(a, b, al)); }
 inline int cmp_bytes(const char* a, u32 al, const char* b, u32 bl) { int c = memcmp(a, b, std::min(al, bl)); return c ? c : (al < bl ? -1 : al > bl ? 1 : 0); }
@@ -455,6 +475,40 @@ int walk_records(const RawBuf& d, size_t len, size_t cur, bool eof, int threads,
   return NB_OK;
 }
 
+// Where the BAM header ends in the first `len` inflated bytes of a streamed file: end = 0 while they do not hold all of it
+// (read on), an error when they cannot be a header or eof says that nothing more comes.
+int header_end(const u8* d, size_t len, bool eof, size_t& end) {
+  end = 0;
+  bool ok = len >= 12; size_t p = 0;
+  if (ok && memcmp(d, "BAM\1", 4)) return fail(NB_ERR_PARSE, "not a BAM file");
+  if (ok) { u32 l_text; memcpy(&l_text, d + 4, 4); p = 8 + (size_t)l_text; ok = p + 4 <= len; }
+  if (ok) { u32 n_ref; memcpy(&n_ref, d + p, 4); p += 4; for (u32 i = 0; i < n_ref && ok; i++) { if (p + 4 > len) { ok = false; break; } u32 l; memcpy(&l, d + p, 4); p += 4 + (size_t)l + 4; } ok = ok && p <= len; }
+  if (ok) end = p;
+  else if (eof) return fail(NB_ERR_PARSE, len < 12 ? "not a BAM file" : "truncated BAM header");
+  return NB_OK;
+}
+
+// What SortedBamReader::fill_buffer (src/parse/sorted_bam_reader.rs:31-107) does with a record: keep it, skip it, or fail
+// on it.  The any-order producer adds failures of its own after these kinds.
+enum Keep { KEEP, SKIP, NO_UMI, EMPTY_UMI, UMI_NOT_PACKED, CB_UNKNOWN };
+inline Keep keep_of(const Rec& r, bool force_paired) {
+  if (!r.is_paired() && force_paired) return SKIP;
+  if (!r.cb) return SKIP;
+  if (!r.umi) return NO_UMI;
+  if (r.umi_len == 10 && !memcmp(r.umi, "AAAAAAAAAA", 10)) return SKIP;
+  if (r.umi_len == 0) return EMPTY_UMI;   // (the serial reader keeps it; where it groups depends on the whole file)
+  return KEEP;
+}
+
+// The failing records of a pass over a window on T threads, each thread stopping at its first: the first of them in file
+// order decides the error, as in the serial loop.
+struct FirstBad {
+  std::vector<size_t> at; std::vector<Keep> kind;
+  explicit FirstBad(int T) : at(T, (size_t)-1), kind(T, KEEP) {}
+  void set(int t, size_t i, Keep k) { at[t] = i; kind[t] = k; }
+  Keep first(size_t& i) const { Keep k = KEEP; i = (size_t)-1; for (size_t t = 0; t < at.size(); t++) if (at[t] < i) { i = at[t]; k = kind[t]; } return k; }
+};
+
 // ------------------------------------------------------------------ windowed producer
 // The same stream and groups as collect_groups_serial, computed window by window on `threads` threads with bounded memory.
 // The serial readers above define the semantics; this restates them over whole runs: a SortedBamReader buffer is a maximal
@@ -477,8 +531,7 @@ struct GroupStreamer {
   bool header_done = false, eof = false, ended = false; u64 groups_sent = 0, records_seen = 0; size_t peak_window = 0;
   std::string last_umi, last_cb; bool have_last = false;     // key of the last record sent (cross-window coincidence check)
   double t_inflate = 0, t_scan = 0, t_keys = 0, t_runs = 0, t_emit = 0, t_groups = 0;   // phase times (NB_BAM_STATS)
-  static double clk() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + ts.tv_nsec * 1e-9; }
-  int open(const std::string& path, bool fp, int th, size_t wb) { force_paired = fp; threads = std::max(1, th); window_bytes = std::max<size_t>(wb, 1 << 16); return z.open(path); }
+  int open(const std::string& path, bool fp, int th, size_t wb) { force_paired = fp; threads = std::max(1, th); window_bytes = wb; return z.open(path); }
   // fills w from the file position and the carry-over of `prev` (nullptr for the first window).  done: nothing was produced
   // and nothing more will come.
   int next(Window& w, const Window* prev, bool& done) {
@@ -493,19 +546,14 @@ struct GroupStreamer {
     }
     size_t grow = window_bytes;
     for (;;) {   // (repeats only when the window could not emit anything: one giant UMI run, or a header larger than the window)
-      double tc = clk();
+      double tc = now();
       if (!eof) { size_t n_out = 0; int rc = z.next(w.data, w.len, grow, threads, n_out, eof); if (rc) return rc; z.compact(); w.len += n_out; }
-      t_inflate += clk() - tc; tc = clk();
+      t_inflate += now() - tc; tc = now();
       peak_window = std::max(peak_window, w.len);
       size_t cur = 0;
       if (!header_done) {
-        const RawBuf& d = w.data; bool ok = w.len >= 12;
-        if (ok && memcmp(d.data(), "BAM\1", 4)) return fail(NB_ERR_PARSE, "not a BAM file");
-        size_t p = 0;
-        if (ok) { u32 l_text; memcpy(&l_text, &d[4], 4); p = 8 + (size_t)l_text; ok = p + 4 <= w.len; }
-        if (ok) { u32 n_ref; memcpy(&n_ref, &d[p], 4); p += 4; for (u32 i = 0; i < n_ref && ok; i++) { if (p + 4 > w.len) { ok = false; break; } u32 l; memcpy(&l, &d[p], 4); p += 4 + (size_t)l + 4; } ok = ok && p <= w.len; }
-        if (!ok) { if (eof) return fail(NB_ERR_PARSE, w.len < 12 ? "not a BAM file" : "truncated BAM header"); grow *= 2; continue; }
-        cur = p;
+        int rc = header_end(w.data.data(), w.len, eof, cur); if (rc) return rc;
+        if (!cur) { grow *= 2; continue; }
       }
       size_t cur_end = cur;
       { int rw = walk_records(w.data, w.len, cur, eof, threads, w.all, cur_end); if (rw) return rw; }
@@ -514,32 +562,28 @@ struct GroupStreamer {
       const size_t par_min_recs = getenv("NB_BAM_PAR_MIN_RECS") ? (size_t)strtoull(getenv("NB_BAM_PAR_MIN_RECS"), nullptr, 10) : 65536;
       const size_t tail = cur;    // first byte that is not part of a complete record
       std::vector<Rec>& all = w.all;
-      t_scan += clk() - tc; tc = clk();
+      t_scan += now() - tc; tc = now();
       parallel_ranges(threads, all.size(), [&](size_t a, size_t b, int) { for (size_t i = a; i < b; i++) all[i].scan_keys(); });
-      t_keys += clk() - tc; tc = clk();
+      t_keys += now() - tc; tc = now();
       if (all.size() >= 0xFFFFFFFFull) return fail(NB_ERR_UNSUPPORTED, "more than 2^32 records in one window");
-      // which records the sorted reader keeps, and where its UMI runs start: flags in parallel, compaction by thread-local
-      // counts; the first offending record IN FILE ORDER decides between the two failures, as the serial loop did
+      // which records the sorted reader keeps, and where its UMI runs start: flags in parallel, compaction by thread-local counts
       std::vector<u32> kept; std::vector<size_t> run;
       {
         const int T = all.size() > par_min_recs ? threads : 1;
-        std::vector<u8> flag(all.size(), 0); std::vector<size_t> cnt(T + 1, 0), bad_at(T, (size_t)-1); std::vector<int> bad_kind(T, 0);
+        std::vector<u8> flag(all.size(), 0); std::vector<size_t> cnt(T + 1, 0); FirstBad bad(T);
         parallel_ranges(T, all.size(), [&](size_t a, size_t b, int t) {
           size_t c = 0;
           for (size_t i = a; i < b; i++) {
-            const Rec& r = all[i];
-            if (!r.is_paired() && force_paired) continue;
-            if (!r.cb) continue;
-            if (!r.umi) { bad_at[t] = i; bad_kind[t] = 1; break; }
-            if (r.umi_len == 10 && !memcmp(r.umi, "AAAAAAAAAA", 10)) continue;
-            if (r.umi_len == 0) { bad_at[t] = i; bad_kind[t] = 2; break; }
+            const Keep k = keep_of(all[i], force_paired);
+            if (k == SKIP) continue;
+            if (k != KEEP) { bad.set(t, i, k); break; }
             flag[i] = 1; c++;
           }
           cnt[t + 1] = c;
         });
-        { size_t first = (size_t)-1; int kind = 0; for (int t = 0; t < T; t++) if (bad_at[t] < first) { first = bad_at[t]; kind = bad_kind[t]; }
-          if (kind == 1) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
-          if (kind == 2) return NEED_WHOLE; }
+        { size_t first; const Keep kind = bad.first(first);
+          if (kind == NO_UMI) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
+          if (kind == EMPTY_UMI) return NEED_WHOLE; }
         for (int t = 0; t < T; t++) cnt[t + 1] += cnt[t];
         kept.resize(cnt[T]);
         parallel_ranges(T, all.size(), [&](size_t a, size_t b, int t) { size_t at = cnt[t]; for (size_t i = a; i < b; i++) if (flag[i]) kept[at++] = (u32)i; });
@@ -551,7 +595,7 @@ struct GroupStreamer {
         parallel_ranges(T, nk, [&](size_t a, size_t b, int t) { size_t at = hc[t]; for (size_t j = a; j < b; j++) if (head[j]) run[at++] = j; });
       }
       const size_t nr = run.size(); run.push_back(kept.size());
-      t_runs += clk() - tc; tc = clk();
+      t_runs += now() - tc; tc = now();
       // one run -> the records the sorted reader hands on (CB sort unless it is the file's last run, dummy mates, pairing)
       auto emit_run = [&](size_t r, std::vector<Rec>& out, std::vector<Rec>& buf, std::vector<Rec>& tmp) {
         buf.clear(); for (size_t j = run[r]; j < run[r + 1]; j++) buf.push_back(all[kept[j]]);
@@ -603,7 +647,7 @@ struct GroupStreamer {
       if (cut) { ended = true; w.carry_from = w.len; }   // the reference's reader stops for good at an empty buffer
       const bool final = eof || ended;
       header_done = true; records_seen += all.size();
-      t_emit += clk() - tc; tc = clk();
+      t_emit += now() - tc; tc = now();
       std::vector<u64>& gstart = w.gstart; gstart.clear();
       if (stream.empty()) { gstart.assign(1, 0); if (final && groups_sent == 0) gstart.push_back(0); done = gstart.size() < 2; return NB_OK; }
       // groups: runs of equal (UMI + CB[..len-2]) over the stream
@@ -615,7 +659,7 @@ struct GroupStreamer {
       if (final && groups_sent + (gstart.size() - 1) >= 2) { stream.resize(gstart[gstart.size() - 2]); gstart.pop_back(); }   // the last group is never sent when a group was sent before
       groups_sent += gstart.size() - 1;
       if (!stream.empty()) { const Rec& l = stream.back(); last_umi.assign(l.umi, l.umi_len); last_cb.assign(l.cb ? l.cb : "", l.cb_len); have_last = true; }
-      t_groups += clk() - tc;
+      t_groups += now() - tc;
       return NB_OK;
     }
   }
@@ -760,6 +804,34 @@ struct CellDict {
   }
 };
 
+// The reference libraries of a BAM run, one context each.  parse_trim checks --trim before anything is loaded; open loads
+// every library with its trim, builds its index (or loads it from $NB_INDEX_CACHE) and creates its context on `stream`
+// (nullptr: a stream of its own).
+struct Libraries {
+  std::vector<std::pair<u64, double>> trims;   // (target length, strictness) per library, or none
+  std::vector<nb_library*> libs; std::vector<nb_index*> idx; std::vector<nb_ctx*> ctx;
+  ~Libraries() { for (size_t i = 0; i < ctx.size(); i++) { nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } }
+  int parse_trim(const char* trim /* "L:S,L:S" or NULL */, u32 n_refs) {   // src/bin/main.rs:74-93
+    if (!trim || !*trim) return NB_OK;
+    std::string t(trim); size_t p = 0;
+    while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
+    if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
+    return NB_OK;
+  }
+  int open(const char* const* reference_json, u32 n_refs, int strand_filter, int threads, int device, void* stream) {
+    libs.assign(n_refs, nullptr); idx.assign(n_refs, nullptr); ctx.assign(n_refs, nullptr);
+    int rc = NB_OK;
+    for (u32 i = 0; i < n_refs && rc == NB_OK; i++) {
+      rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
+      if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
+      if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);   // K5: the CUDA builder (same artefact as the host builder), or $NB_INDEX_CACHE
+      if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, stream, &ctx[i]);
+      if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);   // a batch of 2^20 pairs can hold that many one-pair scopes, each with its own (scope, callset) row: stay under half full
+    }
+    return rc;
+  }
+};
+
 // text -> gzip members of the rows' compressor, written to `path`; the text is cut into pieces of a fixed size (compressed on
 // several threads) so that the bytes do not depend on the thread count
 int write_gz_pieces(const std::string& path, const std::vector<std::string>& pieces) {
@@ -847,30 +919,14 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
   if (!input_file || !reference_json || (!output_paths && !matrix_dirs) || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference/output pair");
   const bool want_rows = output_paths != nullptr, want_cells = matrix_dirs != nullptr;
   int threads = std::max(1, num_cores);
-  std::vector<nb_library*> libs(n_refs, nullptr); std::vector<nb_index*> idx(n_refs, nullptr); std::vector<nb_ctx*> ctx(n_refs, nullptr); std::vector<FILE*> outs(n_refs, nullptr);
+  Libraries L; std::vector<nb_library*>& libs = L.libs; std::vector<nb_ctx*>& ctx = L.ctx;
+  std::vector<FILE*> outs(n_refs, nullptr);
   std::vector<bool> first_write(n_refs, true);
-  int rc = NB_OK;
-  auto cleanup = [&]() { for (u32 i = 0; i < n_refs; i++) { if (outs[i]) fclose(outs[i]); nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } };
-  std::vector<std::pair<u64, double>> trims;
-  if (trim && *trim) {   // src/bin/main.rs:74-93
-    std::string t(trim); size_t p = 0;
-    while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
-    if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
-  }
-  for (u32 i = 0; i < n_refs && rc == NB_OK; i++) {
-    rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
-    if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
-    if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);   // K5: the CUDA builder (same artefact as the host builder), or $NB_INDEX_CACHE
-    if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nullptr, &ctx[i]);
-    if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);   // a batch of 2^20 pairs can hold that many one-pair scopes, each with its own (scope, callset) row: stay under half full
-    if (rc == NB_OK && want_rows) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
-  }
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+  auto cleanup = [&]() { for (FILE* f : outs) if (f) fclose(f); };
+  int rc = L.parse_trim(trim, n_refs); if (rc) return rc;
+  rc = L.open(reference_json, n_refs, strand_filter, threads, device, nullptr);
+  for (u32 i = 0; i < n_refs && rc == NB_OK && want_rows; i++) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
   double t_load = 0, t_group = 0, t_fill = 0, t_gpu = 0, t_rows = 0, t_align = 0, t_final = 0, t_roll = 0, t_cells = 0, t0 = now(); const double t_start = t0;   // NB_BAM_STATS=1 prints the phase times
-  // window size of the streaming producer: NB_BAM_WINDOW_MB (inflated bytes per window; tests use small ones), default 256 MB
-  size_t window_bytes = (size_t)256 << 20;
-  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = (size_t)strtoull(e, nullptr, 10) << 10;
-  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = (size_t)strtoull(e2, nullptr, 10) << 20;
   if (rc != NB_OK) { cleanup(); return rc; }
   const size_t BATCH_PAIRS = 1u << 20;
   const int GZ_LEVEL = rows_gz_level();   // 0: the rows' own compressor (deflate_fast.hpp); NB_BAM_GZ_LEVEL=1..9: zlib at that level (the rows are the same, the members smaller or slower to make)
@@ -1064,7 +1120,7 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
   double t_prod = 0; size_t peak_window = 0; bool whole_file = false;
   {
     GroupStreamer gs; Window win[2];
-    rc = gs.open(input_file, force_bam_paired != 0, threads, window_bytes);
+    rc = gs.open(input_file, force_bam_paired != 0, threads, window_bytes());
     bool done = false; int cur = 0;
     if (rc == NB_OK) { double tp = now(); rc = gs.next(win[0], nullptr, done); t_prod += now() - tp; }
     while (rc == NB_OK && !done) {
@@ -1101,9 +1157,7 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
     t_cells = now() - tc;
   }
   if (getenv("NB_BAM_STATS")) {
-    // peak resident set of THIS process image (VmHWM belongs to the mm, so unlike ru_maxrss it does not start at the forking parent's size)
-    double hwm_mb = 0; if (FILE* st = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, st)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(st); }
-    fprintf(stderr, "nb_process_bam: %zu records in %zu groups%s; windows (read+inflate+group, overlapped) %.2fs, largest window %.0f MB, batch fill %.2fs, device align+finalize %.2fs (align %.2fs, finalize %.2fs), rows+gzip+write %.2fs (fill and rows overlap the device stage), cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, peak RSS %.0f MB\n", n_records_total, n_groups_total, whole_file ? " (whole-file fallback)" : "", t_load, peak_window / 1048576.0, t_fill, t_gpu, t_align, t_final, t_rows, t_roll, t_cells, now() - t_start, hwm_mb);
+    fprintf(stderr, "nb_process_bam: %zu records in %zu groups%s; windows (read+inflate+group, overlapped) %.2fs, largest window %.0f MB, batch fill %.2fs, device align+finalize %.2fs (align %.2fs, finalize %.2fs), rows+gzip+write %.2fs (fill and rows overlap the device stage), cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, peak RSS %.0f MB\n", n_records_total, n_groups_total, whole_file ? " (whole-file fallback)" : "", t_load, peak_window / 1048576.0, t_fill, t_gpu, t_align, t_final, t_rows, t_roll, t_cells, now() - t_start, peak_rss_mb());
   }
   cleanup();
   return rc;
@@ -1113,9 +1167,6 @@ extern "C" int nb_process_bam_cells(const char* input_file, const char* const* r
 // group index, clipped sequence, hex of the clipped (unreversed) quals, then the 38 metadata fields (QUAL as hex).
 extern "C" int nb_bam_dump_groups(const char* input_file, int force_bam_paired, int num_cores, const char* out_path) {
   if (!input_file || !out_path) return fail(NB_ERR_INVALID, "null argument");
-  size_t window_bytes = (size_t)256 << 20;
-  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = (size_t)strtoull(e, nullptr, 10) << 10;
-  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = (size_t)strtoull(e2, nullptr, 10) << 20;
   FILE* f = fopen(out_path, "wb"); if (!f) return fail(NB_ERR_IO, std::string("could not open ") + out_path);
   auto hex = [](const std::string& s) { static const char* H = "0123456789abcdef"; std::string o; for (unsigned char c : s) { o += H[c >> 4]; o += H[c & 15]; } return o; };
   size_t gi0 = 0;
@@ -1137,12 +1188,12 @@ extern "C" int nb_bam_dump_groups(const char* input_file, int force_bam_paired, 
   int rc = NB_OK;
   {
     GroupStreamer gs; Window win[2]; bool done = false; int cur = 0;
-    rc = getenv("NB_BAM_SERIAL_GROUPING") ? NEED_WHOLE : gs.open(input_file, force_bam_paired != 0, std::max(1, num_cores), window_bytes);
+    rc = getenv("NB_BAM_SERIAL_GROUPING") ? NEED_WHOLE : gs.open(input_file, force_bam_paired != 0, std::max(1, num_cores), window_bytes());
     if (rc == NB_OK) rc = gs.next(win[0], nullptr, done);
     const bool none = out_path[0] && !strcmp(out_path, "/dev/null") && getenv("NB_BAM_DUMP_NONE");   // producer only (timing the reader)
     double t_fmt = 0; size_t n_fmt = 0;
     while (rc == NB_OK && !done) {
-      if (rowfmt) { double tf = GroupStreamer::clk(); dump_rowfmt(win[cur].stream, !none); n_fmt += win[cur].stream.size(); t_fmt += GroupStreamer::clk() - tf; }
+      if (rowfmt) { double tf = now(); dump_rowfmt(win[cur].stream, !none); n_fmt += win[cur].stream.size(); t_fmt += now() - tf; }
       else if (!none) dump(win[cur].stream, win[cur].gstart);
       rc = gs.next(win[cur ^ 1], &win[cur], done); cur ^= 1;
     }
@@ -1217,7 +1268,6 @@ int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
 // [P->lo, P->hi) are staged, and passes after the first only look the CBs up.  rows: every staged record also gets its
 // metadata text M(r) (append_data_values without SKIP_ALIGN) and the length of its field 0, formatted on the host threads.
 int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, bool rows, Passes* P = nullptr) {
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   Bgzf z; int rc = z.open(input_file); if (rc) return rc;
   RawBuf data; size_t len = 0; bool eof = false, header_done = false;
   std::vector<Rec> all;
@@ -1226,11 +1276,8 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
     if (!eof) { size_t n_out = 0; rc = z.next(data, len, window_bytes, threads, n_out, eof); if (rc) return rc; z.compact(); len += n_out; }
     st.peak_window = std::max(st.peak_window, len);
     if (!header_done) {
-      bool ok = len >= 12; size_t p = 0;
-      if (ok && memcmp(data.data(), "BAM\1", 4)) return fail(NB_ERR_PARSE, "not a BAM file");
-      if (ok) { u32 l_text; memcpy(&l_text, &data[4], 4); p = 8 + (size_t)l_text; ok = p + 4 <= len; }
-      if (ok) { u32 n_ref; memcpy(&n_ref, &data[p], 4); p += 4; for (u32 i = 0; i < n_ref && ok; i++) { if (p + 4 > len) { ok = false; break; } u32 l; memcpy(&l, &data[p], 4); p += 4 + (size_t)l + 4; } ok = ok && p <= len; }
-      if (!ok) { if (eof) return fail(NB_ERR_PARSE, len < 12 ? "not a BAM file" : "truncated BAM header"); continue; }
+      size_t p; rc = header_end(data.data(), len, eof, p); if (rc) return rc;
+      if (!p) continue;
       memmove(data.data(), data.data() + p, len - p); len -= p; header_done = true;
     }
     size_t tail = 0;
@@ -1241,31 +1288,30 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
     parallel_ranges(T, n, [&](size_t a, size_t b, int) { for (size_t i = a; i < b; i++) all[i].scan_keys(); });
     // keep / skip / fail per record; the first failing record in file order decides the error
     std::vector<u8> keep(n, 0); std::vector<u64> umi(n); std::vector<u32> cb(n, NONE32); std::vector<u64> cb_hash(n);
-    std::vector<size_t> bad_at(T, (size_t)-1); std::vector<int> bad_kind(T, 0); std::vector<u64> cnt(T + 1, 0), nib(T + 1, 0), nam(T + 1, 0); std::vector<u32> mx(T, 1);
+    FirstBad bad(T); std::vector<u64> cnt(T + 1, 0), nib(T + 1, 0), nam(T + 1, 0); std::vector<u32> mx(T, 1);
     std::vector<std::vector<u32>> miss(T);
     std::vector<u32> bucket(P ? n : 0);
     parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
       u64 c = 0, nb_ = 0, nm = 0; u32 m = 1;
       for (size_t i = a; i < b; i++) {
         const Rec& r = all[i];
-        if (!r.cb) continue;
-        if (!r.umi) { bad_at[t] = i; bad_kind[t] = 1; break; }
-        if (r.umi_len == 10 && !memcmp(r.umi, "AAAAAAAAAA", 10)) continue;
-        if (r.umi_len == 0) { bad_at[t] = i; bad_kind[t] = 2; break; }
-        if (!nbg::pack_umi(r.umi, r.umi_len, umi[i])) { bad_at[t] = i; bad_kind[t] = 3; break; }
+        Keep k = keep_of(r, false);
+        if (k == SKIP) continue;
+        if (k == KEEP && !nbg::pack_umi(r.umi, r.umi_len, umi[i])) k = UMI_NOT_PACKED;
+        if (k != KEEP) { bad.set(t, i, k); break; }
         size_t x, y; clip_of(r, x, y); m = std::max<u32>(m, (u32)(y - x));
         const u64 h = cb_hash[i] = CellDict::hash_of(r.cb, r.cb_len);
-        if ((cb[i] = cells.find(r.cb, r.cb_len, h)) == NONE32) { if (lookup_only) { bad_at[t] = i; bad_kind[t] = 4; break; } miss[t].push_back((u32)i); }
+        if ((cb[i] = cells.find(r.cb, r.cb_len, h)) == NONE32) { if (lookup_only) { bad.set(t, i, CB_UNKNOWN); break; } miss[t].push_back((u32)i); }
         if (P) { const u32 bk = bucket[i] = nbg::umi_bucket(umi[i]); if (bk < P->lo || bk >= P->hi) continue; }
         keep[i] = 1; c++; nb_ += (r.l_seq() + 1) / 2; nm += r.qname_len();
       }
       cnt[t + 1] = c; nib[t + 1] = nb_; nam[t + 1] = nm; mx[t] = m;
     });
-    { size_t first = (size_t)-1; int kind = 0; for (int t = 0; t < T; t++) if (bad_at[t] < first) { first = bad_at[t]; kind = bad_kind[t]; }
-      if (kind == 1) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
-      if (kind == 2) return fail(NB_ERR_UNSUPPORTED, "a kept record has an empty UMI string (where the reference groups it depends on the file order): record " + std::to_string(st.n_records + first) + " of " + input_file);
-      if (kind == 3) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)");
-      if (kind == 4) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see"); }
+    { size_t first; const Keep kind = bad.first(first);
+      if (kind == NO_UMI) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
+      if (kind == EMPTY_UMI) return fail(NB_ERR_UNSUPPORTED, "a kept record has an empty UMI string (where the reference groups it depends on the file order): record " + std::to_string(st.n_records + first) + " of " + input_file);
+      if (kind == UMI_NOT_PACKED) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)");
+      if (kind == CB_UNKNOWN) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see"); }
     for (int t = 0; t < T; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
     // rows: M(r) of the kept records, back to back per thread slice (the slices of every parallel_ranges(T, n) below)
     std::vector<std::string> mt(rows ? T : 0); std::vector<u32> mlen(rows ? n : 0), f0l(rows ? n : 0); std::vector<u64> met(T + 1, 0);
@@ -1348,7 +1394,6 @@ struct AnyOrderRun {
 // stopped up to the hi its windows left.  After each pass's grouping: on_pass(pass, grouped, max_read_len) aligns it.
 template <class F>
 int any_order_passes(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, u64 budget, bool rows, CellDict& cells, AnyOrderRun& run, F on_pass) {
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   Passes P; P.budget = budget; P.rows = rows;
   nbg::set_budget(dev, budget); nbg::set_rows(dev, rows);
   for (u32 lo = 0;;) {
@@ -1375,145 +1420,58 @@ int any_order_passes(const char* input_file, int threads, size_t window_bytes, n
   return NB_OK;
 }
 
-size_t any_order_window_bytes() {
-  size_t window_bytes = (size_t)256 << 20;
-  if (const char* e = getenv("NB_BAM_WINDOW_KB")) window_bytes = std::max<size_t>((size_t)strtoull(e, nullptr, 10) << 10, 1 << 16);
-  else if (const char* e2 = getenv("NB_BAM_WINDOW_MB")) window_bytes = std::max<size_t>((size_t)strtoull(e2, nullptr, 10) << 20, 1 << 16);
-  return window_bytes;
-}
-
-// The device store and one library context per reference of an any-order run, all on the store's stream (the batches'
-// scope ids are written on it).
-struct AnyOrderSetup {
-  nbg::Device* dev = nullptr; u32 n = 0;
-  std::vector<nb_library*> libs; std::vector<nb_index*> idx; std::vector<nb_ctx*> ctx;
-  ~AnyOrderSetup() { for (u32 i = 0; i < n; i++) { nb_ctx_free(ctx[i]); nb_index_free(idx[i]); nb_library_free(libs[i]); } nbg::destroy(dev); }
-  int open(const char* const* reference_json, uint32_t n_refs, int strand_filter, const char* trim, int threads, int device) {
-    std::vector<std::pair<u64, double>> trims;
-    if (trim && *trim) {   // src/bin/main.rs:74-93
-      std::string t(trim); size_t p = 0;
-      while (p <= t.size()) { size_t e = t.find(',', p); if (e == std::string::npos) e = t.size(); std::string one = t.substr(p, e - p); size_t c = one.find(':'); if (c == std::string::npos) return fail(NB_ERR_INVALID, "Invalid strictness"); trims.push_back({strtoull(one.substr(0, c).c_str(), nullptr, 10), strtod(one.substr(c + 1).c_str(), nullptr)}); p = e + 1; }
-      if (trims.size() != n_refs) return fail(NB_ERR_INVALID, "The number of trim options does not match the number of reference libraries");
-    }
-    n = n_refs; libs.assign(n, nullptr); idx.assign(n, nullptr); ctx.assign(n, nullptr);
-    int rc = nbg::create(device, &dev);
-    for (u32 i = 0; i < n && rc == NB_OK; i++) {
-      rc = nb_library_load_json(reference_json[i], strand_filter, &libs[i]);
-      if (rc == NB_OK && !trims.empty()) { nb_config c; nb_library_get_config(libs[i], &c); c.trim_target_length = trims[i].first; c.trim_strictness = trims[i].second; rc = nb_library_set_config(libs[i], &c); }
-      if (rc == NB_OK) rc = nb_index_build_cached(libs[i], nullptr, device, threads, &idx[i]);
-      if (rc == NB_OK) rc = nb_ctx_create(idx[i], libs[i], device, nbg::stream_of(dev), &ctx[i]);
-      if (rc == NB_OK) rc = nb_ctx_set_option(ctx[i], "agg_slots", 1u << 23);
-    }
-    return rc;
+// Batches of an any-order pass: runs of whole scopes [s0, s1) that have pairs, at most 2^20 pairs each (a larger scope is
+// a batch of its own).
+std::vector<std::pair<u64, u64>> scope_batches(const nbg::Grouped& g) {
+  const u64 BATCH_PAIRS = 1u << 20;
+  std::vector<std::pair<u64, u64>> batches;
+  for (u64 s0 = 0; s0 < g.n_scopes;) {
+    u64 s1 = s0 + 1;
+    while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
+    if (g.scope_pair0[s1] > g.scope_pair0[s0]) batches.push_back({s0, s1});
+    s0 = s1;
   }
-};
-
-// The NB_BAM_STATS line of an any-order run; rows: the rows mode's fields, which go before the budget's
-void any_order_stats(const AnyOrderRun& run, nbg::Device* dev, u64 budget, u64 n_batches, size_t n_barcodes, double t_setup, double t_align, double t_roll, double t_out, double t_total, const std::string& rows) {
-  double hwm_mb = 0; if (FILE* stf = fopen("/proc/self/status", "r")) { char line[256]; while (fgets(line, sizeof line, stf)) if (!strncmp(line, "VmHWM:", 6)) hwm_mb = strtod(line + 6, nullptr) / 1024.0; fclose(stf); }
-  const AnyOrderLoad& ld = run.ld;
-  double t_win = 0; std::string per_pass;
-  for (double t : run.t_windows) { t_win += t; char b[32]; snprintf(b, sizeof b, "%s%.2fs", per_pass.empty() ? "" : "/", t); per_pass += b; }
-  std::string extra = rows;
-  if (budget) { char b[256]; snprintf(b, sizeof b, ", budget %llu bytes, passes %d, evictions %llu, peak device bytes %llu, windows per pass ", (unsigned long long)budget, run.passes, (unsigned long long)run.evictions, (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0)); extra += b + per_pass; }
-  fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB%s\n",
-          (unsigned long long)ld.n_records, (unsigned long long)run.n_kept, (unsigned long long)run.n_scopes, (unsigned long long)run.n_pairs, (unsigned long long)n_batches, n_barcodes,
-          t_setup, t_win, ld.t_wait, ld.peak_window / 1048576.0, run.t_group, t_align, t_roll, t_out, t_total,
-          (unsigned long long)(dev ? nbg::store_bytes(dev) : 0), (unsigned long long)(dev ? nbg::group_bytes(dev) : 0), hwm_mb, extra.c_str());
+  return batches;
 }
 
-int process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
-                                int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
-  if (!input_file || !reference_json || !matrix_dirs || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / matrix directory pair");
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+// One library's counts of a scoped batch: reset, align (rres / pres: the rows' device result buffers, or none) and finalize.
+int align_finalize(nb_ctx* ctx, const nb_batch& b, nb_read_result* rres, nb_pair_result* pres, nb_counts& cts) {
+  int e = nb_counts_reset(ctx);
+  if (e == NB_OK) e = nb_ctx_set_option(ctx, "max_batch_pairs", b.n_pairs);   // scoped device batches must fit one chunk
+  if (e == NB_OK) e = nb_align_batch(ctx, &b, rres, pres);
+  if (e == NB_OK) e = nb_counts_finalize(ctx, &cts);
+  return e;
+}
+
+// BAM mode in any record order, with or without a device budget: the per-cell matrices (matrix_dirs) or the TSV.gz rows of
+// the grouped driver on G (output_paths), exactly one of the two.  Every batch of every pass is aligned and finalized
+// library by library.  Matrices: the batch's scopes are rolled into the per-cell table by CB dictionary id; after the last
+// pass the barcodes are the cells of the scopes that have pairs, in order of first appearance, and the rows are renumbered
+// through that order-preserving map, so their (cell, rank) order holds.  Rows: the batch is aligned into device result
+// buffers and its rows are assembled on the device (nbg::rows_build); the host only deflates each chunk, cut at row
+// boundaries into parts compressed on its threads, and writes the members in order.  The deflate of a chunk runs while the
+// device builds the next one.
+int process_bam_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, const char* const* matrix_dirs,
+                          uint32_t n_refs, int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
+  const bool rows = output_paths != nullptr;
+  if (!input_file || !reference_json || (!output_paths && !matrix_dirs) || n_refs < 1)
+    return fail(NB_ERR_INVALID, rows ? "need an input BAM and >=1 reference library / output pair" : "need an input BAM and >=1 reference library / matrix directory pair");
   const double t_start = now();
   const int threads = std::max(1, num_cores);
-  const size_t window_bytes = any_order_window_bytes();
-  AnyOrderSetup S;
-  int rc = S.open(reference_json, n_refs, strand_filter, trim, threads, device);
-  if (rc != NB_OK) return rc;
-  nbg::Device* dev = S.dev; std::vector<nb_library*>& libs = S.libs; std::vector<nb_ctx*>& ctx = S.ctx;
-  const double t_setup = now();
-  CellDict cells; AnyOrderRun run;
-  // barcodes: the cells of the scopes that have pairs, in order of first appearance.  Without a budget the one pass knows
-  // them before it rolls; with one, the passes roll dictionary ids and the rows are renumbered after the last pass (an
-  // order-preserving map, so the (cell, rank) order of the rows holds).
-  std::vector<u32> remap; std::vector<u8> used; std::vector<const char*> bc;
-  const u64 BATCH_PAIRS = 1u << 20;   // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
-  double t_align = 0, t_roll = 0; u64 n_batches = 0;
-  rc = any_order_passes(input_file, threads, window_bytes, dev, budget, false, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
-    std::vector<u32> cell_of_scope(g.n_scopes, 0);   // scopes without pairs get cell 0 (no rows)
-    if (!budget) {
-      remap.assign(cells.size(), NONE32);
-      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) remap[g.scope_cb[s]] = 0;
-      for (u32 id = 0; id < cells.size(); id++) if (remap[id] != NONE32) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
-      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) cell_of_scope[s] = remap[g.scope_cb[s]];
-    } else {
-      used.resize(cells.size(), 0);
-      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) { cell_of_scope[s] = g.scope_cb[s]; used[g.scope_cb[s]] = 1; }
-    }
-    int e = NB_OK;
-    for (u64 s0 = 0; e == NB_OK && s0 < g.n_scopes;) {
-      u64 s1 = s0 + 1;
-      while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
-      const u64 p0 = g.scope_pair0[s0], p1 = g.scope_pair0[s1];
-      if (p1 > p0) {
-        n_batches++;
-        nb_batch b; e = nbg::batch(dev, p0, p1, s0, max_len, b);
-        for (u32 li = 0; li < n_refs && e == NB_OK; li++) {
-          const double tb = now();
-          e = nb_counts_reset(ctx[li]);
-          if (e == NB_OK) e = nb_ctx_set_option(ctx[li], "max_batch_pairs", p1 - p0);   // scoped device batches must fit one chunk
-          if (e == NB_OK) e = nb_align_batch(ctx[li], &b, nullptr, nullptr);
-          nb_counts cts;
-          if (e == NB_OK) e = nb_counts_finalize(ctx[li], &cts);
-          const double tr = now(); t_align += tr - tb;
-          if (e == NB_OK) e = nb_cells_roll(ctx[li], cell_of_scope.data() + s0, s1 - s0);
-          t_roll += now() - tr;
-        }
-      }
-      s0 = s1;
-    }
-    return e;
-  });
-  const double t_aligned = now();
-  if (rc == NB_OK && budget) {
-    remap.assign(cells.size(), NONE32);
-    for (u32 id = 0; id < used.size(); id++) if (used[id]) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
-  }
-  std::vector<u32> row_cell;
-  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
-    nb_cell_counts cc; rc = nb_cells_finalize(ctx[li], &cc);
-    if (rc == NB_OK && budget) { row_cell.resize(cc.n_rows); for (u64 k = 0; k < cc.n_rows; k++) row_cell[k] = remap[cc.row_cell[k]]; cc.row_cell = row_cell.data(); }
-    if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], libs[li], &cc, bc.data(), bc.size());
-  }
-  const double t_end = now();
-  if (getenv("NB_BAM_STATS")) any_order_stats(run, dev, budget, n_batches, bc.size(), t_setup - t_start, t_align, t_roll, t_end - t_aligned, t_end - t_start, std::string());
-  return rc;
-}
-
-// The TSV.gz rows of the grouped driver on G (nb_process_bam_rows_any_order): every batch of every library is aligned
-// into device result buffers and its rows are assembled on the device (nbg::rows_build); the host only deflates each
-// chunk, cut at row boundaries into parts compressed on its threads, and writes the members in order.  The deflate of a
-// chunk runs while the device builds the next one.
-int process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
-                               int strand_filter, const char* trim, int num_cores, int device, u64 budget) {
-  if (!input_file || !reference_json || !output_paths || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / output pair");
-  auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-  const double t_start = now();
-  const int threads = std::max(1, num_cores);
-  const int GZ_LEVEL = rows_gz_level();
-  AnyOrderSetup S;
-  int rc = S.open(reference_json, n_refs, strand_filter, trim, threads, device);
-  if (rc != NB_OK) return rc;
-  nbg::Device* dev = S.dev;
-  std::vector<FILE*> outs(n_refs, nullptr); std::vector<bool> first_write(n_refs, true);
+  nbg::Device* dev = nullptr;
+  struct Store { nbg::Device*& d; ~Store() { nbg::destroy(d); } } store{dev};   // declared before L: the contexts on its stream go first
+  Libraries L;
+  int rc = L.parse_trim(trim, n_refs);
+  if (rc == NB_OK) rc = nbg::create(device, &dev);
+  if (rc == NB_OK) rc = L.open(reference_json, n_refs, strand_filter, threads, device, nbg::stream_of(dev));   // the batches' scope ids are written on the store's stream
+  std::vector<FILE*> outs(rows ? n_refs : 0, nullptr); std::vector<bool> first_write(n_refs, true);
   struct Closer { std::vector<FILE*>& f; ~Closer() { for (FILE* x : f) if (x) fclose(x); } } closer{outs};
-  for (u32 i = 0; i < n_refs && rc == NB_OK; i++) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
+  for (u32 i = 0; i < outs.size() && rc == NB_OK; i++) { outs[i] = fopen(output_paths[i], "wb"); if (!outs[i]) rc = fail(NB_ERR_IO, std::string("could not open output ") + output_paths[i]); }
   if (rc != NB_OK) return rc;
   const double t_setup = now();
-  std::vector<std::string> reasons(256); for (int r = 0; r < 256; r++) reasons[r] = nb_reason_str(r);
-  // the deflate + write of one chunk, on its own thread while the device goes on; errors come back through the future
+  const int GZ_LEVEL = rows_gz_level();
+  std::vector<std::string> reasons(rows ? 256 : 0); for (size_t r = 0; r < reasons.size(); r++) reasons[r] = nb_reason_str((int)r);
+  // rows: the deflate + write of one chunk, on its own thread while the device goes on; errors come back through the future
   typedef std::pair<int, std::string> Res;
   std::future<Res> fut; double t_deflate = 0;
   auto join = [&]() -> int { if (!fut.valid()) return NB_OK; Res r = fut.get(); if (r.first) set_error(r.second); return r.first; };
@@ -1534,41 +1492,41 @@ int process_bam_rows_any_order(const char* input_file, const char* const* refere
     return Res(NB_OK, std::string());
   };
   CellDict cells; AnyOrderRun run; nbg::RowsStats rst;
-  const u64 BATCH_PAIRS = 1u << 20;   // batches: whole scopes, at most 2^20 pairs (a larger scope is a batch of its own)
-  double t_align = 0; u64 n_batches = 0;
-  std::string feats; std::vector<u64> feat_off;
-  rc = any_order_passes(input_file, threads, any_order_window_bytes(), dev, budget, true, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
-    std::vector<std::pair<u64, u64>> batches; u64 maxp = 0;
-    for (u64 s0 = 0; s0 < g.n_scopes;) {
-      u64 s1 = s0 + 1;
-      while (s1 < g.n_scopes && g.scope_pair0[s1 + 1] - g.scope_pair0[s0] <= BATCH_PAIRS) s1++;
-      if (g.scope_pair0[s1] > g.scope_pair0[s0]) { batches.push_back({s0, s1}); maxp = std::max(maxp, g.scope_pair0[s1] - g.scope_pair0[s0]); }
-      s0 = s1;
-    }
+  double t_align = 0, t_roll = 0; u64 n_batches = 0;
+  std::vector<u8> used;                           // matrices: the CB ids of the scopes that have pairs, over all passes
+  std::string feats; std::vector<u64> feat_off;   // rows: the callset texts of one finalize
+  rc = any_order_passes(input_file, threads, window_bytes(), dev, budget, rows, cells, run, [&](int, const nbg::Grouped& g, u32 max_len) -> int {
+    const std::vector<std::pair<u64, u64>> batches = scope_batches(g);
     if (batches.empty()) return NB_OK;
-    int e = nbg::rows_begin(dev, maxp); if (e) return e;
-    nb_read_result* rres = nullptr; nb_pair_result* pres = nullptr; nbg::rows_results(dev, &rres, &pres);
+    nb_read_result* rres = nullptr; nb_pair_result* pres = nullptr;
+    std::vector<u32> cell_of_scope;   // matrices: the CB id of every scope (scopes without pairs get 0: they have no rows)
+    if (rows) {
+      u64 maxp = 0; for (const auto& bt : batches) maxp = std::max(maxp, g.scope_pair0[bt.second] - g.scope_pair0[bt.first]);
+      const int e = nbg::rows_begin(dev, maxp); if (e) return e;
+      nbg::rows_results(dev, &rres, &pres);
+    } else {
+      cell_of_scope.assign(g.n_scopes, 0); used.resize(cells.size(), 0);
+      for (u64 s = 0; s < g.n_scopes; s++) if (g.scope_pair0[s + 1] > g.scope_pair0[s]) { cell_of_scope[s] = g.scope_cb[s]; used[g.scope_cb[s]] = 1; }
+    }
     for (const auto& bt : batches) {
-      const u64 s0 = bt.first, p0 = g.scope_pair0[s0], p1 = g.scope_pair0[bt.second];
+      const u64 s0 = bt.first, s1 = bt.second, p0 = g.scope_pair0[s0], p1 = g.scope_pair0[s1];
       n_batches++;
-      nb_batch b; e = nbg::batch(dev, p0, p1, s0, max_len, b); if (e) return e;
+      nb_batch b; int e = nbg::batch(dev, p0, p1, s0, max_len, b); if (e) return e;
       for (u32 li = 0; li < n_refs; li++) {
         const double tb = now();
-        e = nb_counts_reset(S.ctx[li]);
-        if (e == NB_OK) e = nb_ctx_set_option(S.ctx[li], "max_batch_pairs", p1 - p0);
-        if (e == NB_OK) e = nb_align_batch(S.ctx[li], &b, rres, pres);
-        nb_counts cts;
-        if (e == NB_OK) e = nb_counts_finalize(S.ctx[li], &cts);
-        nbg::RowsBatch RB; RB.p0 = p0; RB.p1 = p1; RB.reasons = &reasons;
-        if (e == NB_OK) e = nb_counts_device_rows(S.ctx[li], &RB.row_scope, &RB.row_callset, &RB.row_count, &RB.n_rows);
-        if (e == NB_OK) e = nb_counts_device_slot_map(S.ctx[li], &RB.slot_map, &RB.n_slots);
-        t_align += now() - tb;
+        nb_counts cts; nbg::RowsBatch RB;
+        e = align_finalize(L.ctx[li], b, rres, pres, cts);
+        if (e == NB_OK && rows) e = nb_counts_device_rows(L.ctx[li], &RB.row_scope, &RB.row_callset, &RB.row_count, &RB.n_rows);
+        if (e == NB_OK && rows) e = nb_counts_device_slot_map(L.ctx[li], &RB.slot_map, &RB.n_slots);
+        const double ta = now(); t_align += ta - tb;
         if (e) return e;
+        if (!rows) { e = nb_cells_roll(L.ctx[li], cell_of_scope.data() + s0, s1 - s0); t_roll += now() - ta; if (e) return e; continue; }
         if (!RB.n_rows) continue;
+        RB.p0 = p0; RB.p1 = p1; RB.reasons = &reasons;
         // the text of every callset of this finalize: its group names joined by ','
         feats.clear(); feat_off.assign(1, 0);
         for (u64 c = 0; c < cts.n_callsets; c++) {
-          for (u64 k = cts.callset_off[c]; k < cts.callset_off[c + 1]; k++) { if (k > cts.callset_off[c]) feats += ','; feats += nb_library_group_name(S.libs[li], cts.callset_items[k]); }
+          for (u64 k = cts.callset_off[c]; k < cts.callset_off[c + 1]; k++) { if (k > cts.callset_off[c]) feats += ','; feats += nb_library_group_name(L.libs[li], cts.callset_items[k]); }
           feat_off.push_back(feats.size());
         }
         RB.feats = &feats; RB.feat_off = &feat_off;
@@ -1585,15 +1543,35 @@ int process_bam_rows_any_order(const char* input_file, const char* const* refere
     return NB_OK;
   });
   { const int er = join(); if (er && rc == NB_OK) rc = er; }
-  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) if (first_write[li]) rc = write_rows_empty(outs[li], GZ_LEVEL);
-  for (u32 li = 0; li < n_refs; li++) { if (outs[li] && fclose(outs[li]) != 0 && rc == NB_OK) rc = fail(NB_ERR_IO, std::string("short write on ") + output_paths[li]); outs[li] = nullptr; }
+  std::vector<const char*> bc; double t_out = 0;
+  if (rows) {
+    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) if (first_write[li]) rc = write_rows_empty(outs[li], GZ_LEVEL);
+    for (u32 li = 0; li < n_refs; li++) { if (outs[li] && fclose(outs[li]) != 0 && rc == NB_OK) rc = fail(NB_ERR_IO, std::string("short write on ") + output_paths[li]); outs[li] = nullptr; }
+  } else if (rc == NB_OK) {
+    const double tc = now();
+    used.resize(cells.size(), 0);
+    std::vector<u32> remap(cells.size(), NONE32), row_cell;
+    for (u32 id = 0; id < used.size(); id++) if (used[id]) { remap[id] = (u32)bc.size(); bc.push_back(cells.names.data() + cells.off[id]); }
+    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+      nb_cell_counts cc; rc = nb_cells_finalize(L.ctx[li], &cc);
+      if (rc == NB_OK) { row_cell.resize(cc.n_rows); for (u64 k = 0; k < cc.n_rows; k++) row_cell[k] = remap[cc.row_cell[k]]; cc.row_cell = row_cell.data(); }
+      if (rc == NB_OK) rc = nb_write_cell_matrix(matrix_dirs[li], L.libs[li], &cc, bc.data(), bc.size());
+    }
+    t_out = now() - tc;
+  }
   const double t_end = now();
   if (getenv("NB_BAM_STATS")) {
-    char b[1024];
-    snprintf(b, sizeof b, ", rows %llu, row bytes %llu, row chunks %llu (at most %llu per batch), metadata %llu bytes, metadata text %llu bytes, metadata formatting %.2fs, row buffer %llu bytes, device peak %llu bytes, device row build %.3fs, deflate+write %.3fs",
-             (unsigned long long)rst.rows, (unsigned long long)rst.bytes, (unsigned long long)rst.chunks, (unsigned long long)rst.max_chunks, (unsigned long long)(dev ? nbg::meta_bytes(dev) : 0),
-             (unsigned long long)run.meta_text, run.ld.t_meta, (unsigned long long)nbg::rows_buffer_cap(), (unsigned long long)(dev ? nbg::peak_bytes(dev) : 0), rst.t_device, t_deflate);
-    any_order_stats(run, dev, budget, n_batches, 0, t_setup - t_start, t_align, 0, 0, t_end - t_start, b);
+    char b[1024] = "";
+    if (rows) snprintf(b, sizeof b, ", rows %llu, row bytes %llu, row chunks %llu (at most %llu per batch), metadata %llu bytes, metadata text %llu bytes, metadata formatting %.2fs, row buffer %llu bytes, device peak %llu bytes, device row build %.3fs, deflate+write %.3fs",
+                       (unsigned long long)rst.rows, (unsigned long long)rst.bytes, (unsigned long long)rst.chunks, (unsigned long long)rst.max_chunks, (unsigned long long)nbg::meta_bytes(dev),
+                       (unsigned long long)run.meta_text, run.ld.t_meta, (unsigned long long)nbg::rows_buffer_cap(), (unsigned long long)nbg::peak_bytes(dev), rst.t_device, t_deflate);
+    std::string extra = b, per_pass; double t_win = 0;
+    for (double t : run.t_windows) { t_win += t; char w[32]; snprintf(w, sizeof w, "%s%.2fs", per_pass.empty() ? "" : "/", t); per_pass += w; }
+    if (budget) { snprintf(b, sizeof b, ", budget %llu bytes, passes %d, evictions %llu, peak device bytes %llu, windows per pass ", (unsigned long long)budget, run.passes, (unsigned long long)run.evictions, (unsigned long long)nbg::peak_bytes(dev)); extra += b + per_pass; }
+    fprintf(stderr, "nb_process_bam_any_order: %llu records, %llu kept, %llu scopes, %llu pairs, %llu batches, %zu barcodes; setup %.2fs, windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+scope build %.3fs, device align+finalize %.3fs, cell roll %.3fs, cell finalize+matrix write %.3fs, total %.2fs, store %llu bytes, grouping %llu bytes, peak RSS %.0f MB%s\n",
+            (unsigned long long)run.ld.n_records, (unsigned long long)run.n_kept, (unsigned long long)run.n_scopes, (unsigned long long)run.n_pairs, (unsigned long long)n_batches, bc.size(),
+            t_setup - t_start, t_win, run.ld.t_wait, run.ld.peak_window / 1048576.0, run.t_group, t_align, t_roll, t_out, t_end - t_start,
+            (unsigned long long)nbg::store_bytes(dev), (unsigned long long)nbg::group_bytes(dev), peak_rss_mb(), extra.c_str());
   }
   return rc;
 }
@@ -1608,7 +1586,7 @@ int dump_scopes_any_order(const char* input_file, int num_cores, int device, u64
   CellDict cells; AnyOrderRun run;
   std::string out; u64 shown = 0;
   static const char* SEQ = "=ACMGRSVTWYHKDBN"; static const char* H = "0123456789abcdef";
-  if (rc == NB_OK) rc = any_order_passes(input_file, std::max(1, num_cores), any_order_window_bytes(), dev, budget, false, cells, run, [&](int pass, const nbg::Grouped& g, u32) -> int {
+  if (rc == NB_OK) rc = any_order_passes(input_file, std::max(1, num_cores), window_bytes(), dev, budget, false, cells, run, [&](int pass, const nbg::Grouped& g, u32) -> int {
     std::vector<u64> o1, o2, b1, b2; std::vector<u8> f1, f2, nib, qual; std::vector<u32> l1, l2;
     int e = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
     if (e == NB_OK && slots) e = nbg::slots_to_host(dev, b1, b2, nib, qual);
@@ -1644,17 +1622,18 @@ int dump_scopes_any_order(const char* input_file, int num_cores, int device, u64
 
 extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                               int strand_filter, const char* trim, int num_cores, int device) {
-  return process_bam_cells_any_order(input_file, reference_json, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, 0);
+  return process_bam_any_order(input_file, reference_json, nullptr, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, 0);
 }
 
 extern "C" int nb_process_bam_cells_any_order_budget(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                                      int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes) {
-  return process_bam_cells_any_order(input_file, reference_json, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
+  return process_bam_any_order(input_file, reference_json, nullptr, matrix_dirs, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
 }
 
 extern "C" int nb_process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
                                              int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes) {
-  return process_bam_rows_any_order(input_file, reference_json, output_paths, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
+  if (!output_paths) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference library / output pair");   // (a null output_paths means matrices to the driver)
+  return process_bam_any_order(input_file, reference_json, output_paths, nullptr, n_refs, strand_filter, trim, num_cores, device, budget_bytes);
 }
 
 extern "C" int nb_bam_dump_scopes_any_order(const char* input_file, int num_cores, int device, const char* out_path) {

@@ -8,7 +8,8 @@
 // so no bases move: the scoped batches handed to nb_align_batch are NB_MEM_DEVICE views of the store.  Under a device
 // budget every allocation here is counted against it, and compact() drops the records of the UMI buckets a pass gives up.
 // Rows mode (nb_process_bam_rows_any_order) keeps every record's metadata text in a fourth byte store, and the row kernels
-// below turn each aligned batch into the grouped driver's TSV rows next to it.
+// below turn each aligned batch into the grouped driver's TSV rows next to it.  One driver, process_bam_any_order in bam.cpp,
+// runs both modes, with or without a budget: they differ only in what follows each batch's finalize.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 

@@ -1,7 +1,8 @@
-// bam_group.hpp — the device record store of BAM mode in any record order (nb_process_bam_cells_any_order): the host
-// producer stages every kept record's nibbles, quals, name and keys window by window; the device sorts the records by
-// (UMI, CB), cuts the (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into
-// the store.  Host-only declarations (bam.cpp includes them; bam_group.cu implements them).
+// bam_group.hpp — the device record store of BAM mode in any record order (bam.cpp's process_bam_any_order, the one driver
+// behind nb_process_bam_cells_any_order[_budget] and nb_process_bam_rows_any_order): the host producer stages every kept
+// record's nibbles, quals, name and keys window by window; the device sorts the records by (UMI, CB), cuts the
+// (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into the store.
+// Host-only declarations (bam.cpp includes them; bam_group.cu implements them).
 #pragma once
 #include <functional>
 #include <string>
