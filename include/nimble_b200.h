@@ -135,7 +135,9 @@ void* nb_host_alloc(size_t bytes);
 void nb_host_free(void*);
 
 enum { NB_MEM_HOST = 0, NB_MEM_DEVICE = 1 };
-enum { NB_FLAG_SKIP_ALIGN = 1 /* metadata[37]=="TRUE", src/align.rs:527 */, NB_FLAG_REVCOMP = 2 /* REVERSE, src/process/bam.rs:407-415 */ };
+enum { NB_FLAG_SKIP_ALIGN = 1 /* metadata[37]=="TRUE", src/align.rs:527 */, NB_FLAG_REVCOMP = 2 /* REVERSE, src/process/bam.rs:407-415 */,
+       NB_FLAG_REVCOMP_FASTQ = 4 /* NB_SEQ_BAM4 only: reverse complement as in the FASTQ samtools writes for a REVERSE record read
+                                    back by FASTQ mode: A<->T, C<->G, and a non-ACGT code stays A (NB_FLAG_REVCOMP makes it T) */ };
 
 /* One batch of read pairs = the iterators score::call receives (src/score.rs:14-31).  Sequences are ASCII bases
  * (DnaString::from_acgt_bytes semantics: ACGT either case, anything else -> A), concatenated, with n_pairs+1 offsets.
@@ -436,6 +438,33 @@ int nb_any_order_umi_bucket(const char* umi, uint32_t len, uint32_t* bucket);
  * bytes, the row buffer, the device peak and the row build and deflate times to the any-order stats line. */
 int nb_process_bam_rows_any_order(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
                                   int strand_filter, const char* trim, int num_cores, int device, uint64_t budget_bytes);
+/* Bulk BAM mode: FASTQ-mode counts from a BAM without cell barcodes (STAR, HISAT2, ...) in any record order.  The output
+ * files are exactly the bytes nb_process_fastq writes (same libraries, outputs, strand filter, append / header-if-empty
+ * behaviour and failures) on the FASTQs the BAM stands for, r1.fastq + r2.fastq for a paired file and r.fastq for a
+ * single-end one, defined with ordinals 0..n-1 in file order by:
+ *   1. kept records: flag & 0x900 == 0 (neither secondary nor supplementary, samtools fastq's default); QC-fail, duplicate
+ *      and unmapped records are kept; no CB, UB or UR tag is read
+ *   2. paired file: every kept record has flag 0x1; single-end: none has (one read per kept record); both kinds:
+ *      NB_ERR_UNSUPPORTED before any alignment, naming one record of each kind by ordinal
+ *   3. paired file: a template is the kept records with byte-equal QNAME; it gives one pair iff it has exactly two kept
+ *      records, one READ1-only (0x40 without 0x80) and one READ2-only: R1 = the READ1 record, R2 = the READ2 record.  Every
+ *      other kept record is dropped (singletons, READ_OTHER / both-bits records, templates of three or more)
+ *   4. read text: SEQ with every non-ACGT code read as A; a REVERSE (0x10) record reversed and complemented (A<->T, C<->G),
+ *      a non-ACGT position staying A (NB_FLAG_REVCOMP_FASTQ; not BAM mode's NB_FLAG_REVCOMP).  No TSO clip, no trim, QUAL unused
+ *   5. a kept record with SEQ "*" (l_seq 0): NB_ERR_UNSUPPORTED naming its ordinal; reads longer than 1024 bases fail as in
+ *      nb_process_fastq; a file without kept records writes what nb_process_fastq writes for empty inputs
+ * The counts do not depend on the pair order (equal read_keys come from equal sequences and get equal callsets), so pairs
+ * are fed in the order the device forms them.  The records are loaded by the streaming loader of
+ * nb_process_bam_cells_any_order (nibbles, names and flags only: no quals) into device memory, whose size bounds the file
+ * (a store that does not fit fails with NB_ERR_CUDA naming the bytes); the mates are paired by name key on the GPU.
+ * NB_BAM_STATS=1: one stats line (records, kept, pairs, dropped records by reason, windows, upload wait, key + sort + pairing
+ * and align + finalize times, store bytes, peak RSS).  NB_BULK_BATCH_PAIRS=N: batches of at most N pairs (default and cap 2^20). */
+int nb_process_bam_bulk(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
+                        int strand_filter, int num_cores, int device);
+/* test hook: the pairs of nb_process_bam_bulk, one line per pair sorted by R1 ordinal: R1 ordinal TAB R2 ordinal TAB R1 length
+ * TAB R2 length TAB R1 flags TAB R2 flags (NB_FLAG_*); a single-end file has '-' for every R2 field.  NB_BULK_NAME_HASH_BITS=b
+ * (1..64) keeps b bits of the name key, so that names collide and the exact compare separates them. */
+int nb_bam_dump_pairs_bulk(const char* input_file, int num_cores, int device, const char* out_path);
 /* host-only: a cell x feature matrix in the 10x v3 layout that Seurat's Read10X and scanpy's read_10x_mtx load, into `dir`
  * (created when missing; its parent must exist): matrix.mtx.gz (Matrix Market coordinate integer, features x barcodes, UMI
  * counts, 1-based lines sorted by barcode then feature), reads.mtx.gz (the same coordinates with the read counts),

@@ -156,6 +156,8 @@ _SIGS = {
     "nb_bam_dump_scopes_any_order_budget": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_uint64, C.c_char_p]),
     "nb_any_order_umi_bucket": (C.c_int, [C.c_char_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     "nb_process_bam_rows_any_order": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_uint64]),
+    "nb_process_bam_bulk": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int]),
+    "nb_bam_dump_pairs_bulk": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_char_p]),
     "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
     "nb_cells_reset": (C.c_int, [C.c_void_p]),
@@ -672,7 +674,7 @@ def fastq_dump(input_files, out_path, num_cores=1, chunk_bytes=0):
 
 
 def process_bam(input_file, reference_json_paths, output_paths, strand_filter="unstranded", trim=None, num_cores=1, force_bam_paired=False, device=0,
-                matrix_dirs=None, any_order=False, device_budget=None):
+                matrix_dirs=None, any_order=False, device_budget=None, bulk=False):
     """process::bam::process behind main.rs's library loop (src/process/bam.rs:45-243, src/bin/main.rs:95-156).
     matrix_dirs=[dir per library]: also a cell x feature matrix per library (nb_process_bam_cells); output_paths=None with
     matrix_dirs: no TSV rows at all.  any_order=True: from a BAM in any record order, scopes formed on the GPU, no
@@ -680,7 +682,17 @@ def process_bam(input_file, reference_json_paths, output_paths, strand_filter="u
     driver's rows on the (UMI, CB)-sorted file) or the matrices (output_paths=None, matrix_dirs: nb_process_bam_cells_any_order).
     device_budget=bytes (any_order only): the device memory that path may allocate; it takes passes over the file by UMI
     bucket when the records do not fit (nb_process_bam_cells_any_order_budget), and writes the same bytes (the rows: the
-    same lines, pass by pass)."""
+    same lines, pass by pass).  bulk=True: a BAM without cell barcodes in any record order, counted as FASTQ mode counts the
+    reads it stands for (nb_process_bam_bulk): output_paths get exactly what process_fastq writes; trim is ignored, as FASTQ
+    mode ignores it; no matrix_dirs, any_order, force_bam_paired or device_budget."""
+    if bulk:
+        if matrix_dirs is not None or any_order or force_bam_paired or device_budget is not None:
+            raise NbError(-1, "bulk counts a BAM as FASTQ mode counts reads: it takes no matrix_dirs, any_order, force_bam_paired or device_budget")
+        if output_paths is None or len(output_paths) != len(reference_json_paths):
+            raise NbError(-1, "bulk needs one output path per reference library")
+        _ck(lib().nb_process_bam_bulk(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths), len(reference_json_paths),
+                                      CHEM[strand_filter], num_cores, device))
+        return
     if device_budget is not None:
         _check_budget(device_budget, any_order)
     if any_order:
@@ -782,6 +794,12 @@ def bam_dump_scopes_any_order(input_file, out_path, num_cores=1, device=0, devic
         _ck(lib().nb_bam_dump_scopes_any_order_budget(str(input_file).encode(), num_cores, device, int(device_budget), str(out_path).encode()))
         return
     _ck(lib().nb_bam_dump_scopes_any_order(str(input_file).encode(), num_cores, device, str(out_path).encode()))
+
+
+def bam_dump_pairs_bulk(input_file, out_path, num_cores=1, device=0):
+    """The pairs of process_bam(bulk=True), one line per pair sorted by R1 ordinal (nb_bam_dump_pairs_bulk): R1 ordinal,
+    R2 ordinal, both lengths, both NB_FLAG_* bytes; '-' for every R2 field of a single-end file."""
+    _ck(lib().nb_bam_dump_pairs_bulk(str(input_file).encode(), num_cores, device, str(out_path).encode()))
 
 
 def any_order_umi_bucket(umi):

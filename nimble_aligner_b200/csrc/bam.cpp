@@ -490,7 +490,7 @@ int header_end(const u8* d, size_t len, bool eof, size_t& end) {
 
 // What SortedBamReader::fill_buffer (src/parse/sorted_bam_reader.rs:31-107) does with a record: keep it, skip it, or fail
 // on it.  The any-order producer adds failures of its own after these kinds.
-enum Keep { KEEP, SKIP, NO_UMI, EMPTY_UMI, UMI_NOT_PACKED, CB_UNKNOWN };
+enum Keep { KEEP, SKIP, NO_UMI, EMPTY_UMI, UMI_NOT_PACKED, CB_UNKNOWN, NO_SEQ };
 inline Keep keep_of(const Rec& r, bool force_paired) {
   if (!r.is_paired() && force_paired) return SKIP;
   if (!r.cb) return SKIP;
@@ -1218,6 +1218,19 @@ namespace {
 
 struct AnyOrderLoad {   // what the producer saw (NB_BAM_STATS)
   u64 n_records = 0, n_kept = 0, meta_text = 0; u32 max_len = 1; size_t peak_window = 0; double t_wait = 0, t_meta = 0;   // meta_text: M(r) bytes staged
+  u64 first_paired = ~0ull, first_single = ~0ull;   // bulk: ordinals of the first kept records with and without flag 0x1
+};
+
+// What the streaming loader keeps of a record and stages with it.  BAM mode in any record order: SortedBamReader::fill_buffer's
+// filters (CB, UMI), the CB looked up in the run's dictionary, the UMI key and the quals.  Bulk mode (nb_process_bam_bulk):
+// every record that is neither secondary nor supplementary, no tag read, no quals, no TSO clip, and SEQ "*" refused.
+struct LoadPolicy {
+  bool primary = false;   // keep rule: false = fill_buffer's, true = flag & 0x900 == 0
+  bool cells = true;      // CB dictionary lookup and UMI key
+  bool quals = true;      // stage the quals
+  bool rows = false;      // stage M(r) and the field-0 length (rows mode)
+  static LoadPolicy any_order(bool rows) { LoadPolicy p; p.rows = rows; return p; }
+  static LoadPolicy bulk() { LoadPolicy p; p.primary = true; p.cells = false; p.quals = false; return p; }
 };
 
 // Budget mode: a pass stages the records of UMI buckets [lo, hi) (nbg::umi_bucket); hi starts at N_BUCKETS and only falls.
@@ -1267,7 +1280,8 @@ int plan_window(nbg::Device* dev, Passes& P, u64 ncb, bool& lowered) {
 // cells: every kept record's full CB, ids in order of first appearance.  With P (budget mode) only the records of buckets
 // [P->lo, P->hi) are staged, and passes after the first only look the CBs up.  rows: every staged record also gets its
 // metadata text M(r) (append_data_values without SKIP_ALIGN) and the length of its field 0, formatted on the host threads.
-int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, bool rows, Passes* P = nullptr) {
+int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg::Device* dev, CellDict& cells, AnyOrderLoad& st, const LoadPolicy& pol, Passes* P = nullptr) {
+  const bool rows = pol.rows;
   Bgzf z; int rc = z.open(input_file); if (rc) return rc;
   RawBuf data; size_t len = 0; bool eof = false, header_done = false;
   std::vector<Rec> all;
@@ -1285,16 +1299,26 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
     if (all.empty()) { if (eof) break; continue; }   // one record larger than the window: read on
     const size_t n = all.size();
     const int T = n > 65536 ? threads : 1;
-    parallel_ranges(T, n, [&](size_t a, size_t b, int) { for (size_t i = a; i < b; i++) all[i].scan_keys(); });
+    if (pol.cells) parallel_ranges(T, n, [&](size_t a, size_t b, int) { for (size_t i = a; i < b; i++) all[i].scan_keys(); });
     // keep / skip / fail per record; the first failing record in file order decides the error
-    std::vector<u8> keep(n, 0); std::vector<u64> umi(n); std::vector<u32> cb(n, NONE32); std::vector<u64> cb_hash(n);
+    const size_t nc = pol.cells ? n : 0;
+    std::vector<u8> keep(n, 0); std::vector<u64> umi(nc); std::vector<u32> cb(nc, NONE32); std::vector<u64> cb_hash(nc);
     FirstBad bad(T); std::vector<u64> cnt(T + 1, 0), nib(T + 1, 0), nam(T + 1, 0); std::vector<u32> mx(T, 1);
+    std::vector<u64> fpair(T, ~0ull), fsingle(T, ~0ull);   // bulk: first kept record of the slice with / without flag 0x1
     std::vector<std::vector<u32>> miss(T);
     std::vector<u32> bucket(P ? n : 0);
     parallel_ranges(T, n, [&](size_t a, size_t b, int t) {
       u64 c = 0, nb_ = 0, nm = 0; u32 m = 1;
       for (size_t i = a; i < b; i++) {
         const Rec& r = all[i];
+        if (pol.primary) {
+          if (r.flag() & 0x900) continue;
+          if (r.l_seq() == 0) { bad.set(t, i, NO_SEQ); break; }
+          m = std::max<u32>(m, r.l_seq());
+          u64& first = r.is_paired() ? fpair[t] : fsingle[t]; first = std::min<u64>(first, i);
+          keep[i] = 1; c++; nb_ += (r.l_seq() + 1) / 2; nm += r.qname_len();
+          continue;
+        }
         Keep k = keep_of(r, false);
         if (k == SKIP) continue;
         if (k == KEEP && !nbg::pack_umi(r.umi, r.umi_len, umi[i])) k = UMI_NOT_PACKED;
@@ -1311,8 +1335,13 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
       if (kind == NO_UMI) return fail(NB_ERR_PARSE, "Error -- Could not read UMI.");
       if (kind == EMPTY_UMI) return fail(NB_ERR_UNSUPPORTED, "a kept record has an empty UMI string (where the reference groups it depends on the file order): record " + std::to_string(st.n_records + first) + " of " + input_file);
       if (kind == UMI_NOT_PACKED) return fail(NB_ERR_UNSUPPORTED, "UMI \"" + std::string(all[first].umi, all[first].umi_len) + "\" of record " + std::to_string(st.n_records + first) + " cannot be packed into the exact device key (at most " + std::to_string((int)nbg::MAX_UMI_CHARS) + " characters of ACGTN)");
-      if (kind == CB_UNKNOWN) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see"); }
-    for (int t = 0; t < T; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
+      if (kind == CB_UNKNOWN) return fail(NB_ERR_IO, std::string("the input changed between passes: record ") + std::to_string(st.n_records + first) + " of " + input_file + " has a cell barcode the first pass did not see");
+      if (kind == NO_SEQ) return fail(NB_ERR_UNSUPPORTED, "record " + std::to_string(st.n_records + first) + " of " + input_file + " has no SEQ (\"*\"): a kept record needs its bases"); }
+    for (int t = 0; t < T; t++) {
+      if (fpair[t] != ~0ull) st.first_paired = std::min(st.first_paired, st.n_records + fpair[t]);
+      if (fsingle[t] != ~0ull) st.first_single = std::min(st.first_single, st.n_records + fsingle[t]);
+    }
+    for (int t = 0; t < T && pol.cells; t++) for (u32 i : miss[t]) cb[i] = cells.intern(all[i].cb, all[i].cb_len, cb_hash[i]);   // file order: ids follow first appearance
     // rows: M(r) of the kept records, back to back per thread slice (the slices of every parallel_ranges(T, n) below)
     std::vector<std::string> mt(rows ? T : 0); std::vector<u32> mlen(rows ? n : 0), f0l(rows ? n : 0); std::vector<u64> met(T + 1, 0);
     if (rows) {
@@ -1353,9 +1382,10 @@ int any_order_load(const char* input_file, int threads, size_t window_bytes, nbg
         if (keep[i]) {
           const Rec& r = all[i]; const u32 l = r.l_seq(), nbytes = (l + 1) / 2, ql = r.qname_len();
           memcpy(sg->nib + bo, r.seq4(), nbytes);
-          memcpy(sg->qual + 2 * bo, r.qual(), l);   // one qual byte per base, at the base's offset
+          if (pol.quals) memcpy(sg->qual + 2 * bo, r.qual(), l);   // one qual byte per base, at the base's offset
           memcpy(sg->name + no, r.qname_ptr(), ql);
-          sg->umi[k] = umi[i]; sg->cb[k] = cb[i]; sg->nib_off[k] = sg->nib0 + bo; sg->lseq[k] = l; sg->flag[k] = (u16)r.flag();
+          if (pol.cells) { sg->umi[k] = umi[i]; sg->cb[k] = cb[i]; }
+          sg->nib_off[k] = sg->nib0 + bo; sg->lseq[k] = l; sg->flag[k] = (u16)r.flag();
           sg->name_off[k] = sg->name0 + no; sg->name_len[k] = (u8)ql; sg->ordinal[k] = ord0 + i;
           if (rows) { memcpy(sg->meta + mo, mt[t].data() + src, mlen[i]); sg->meta_off[k] = sg->meta0 + mo; sg->meta_len[k] = mlen[i]; sg->f0_len[k] = f0l[i]; mo += mlen[i]; }
           k++; bo += nbytes; no += ql;
@@ -1401,7 +1431,7 @@ int any_order_passes(const char* input_file, int threads, size_t window_bytes, n
     if (budget) { P.begin(lo); if (P.pass) rc = nbg::begin_pass(dev); }
     const double t0 = now();
     AnyOrderLoad ld;
-    if (rc == NB_OK) rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld, rows, budget ? &P : nullptr);
+    if (rc == NB_OK) rc = any_order_load(input_file, threads, window_bytes, dev, cells, ld, LoadPolicy::any_order(rows), budget ? &P : nullptr);
     if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); ld.t_wait += now() - tw; }
     const double t1 = now(); run.t_windows.push_back(t1 - t0);
     nbg::Grouped g;
@@ -1618,7 +1648,116 @@ int dump_scopes_any_order(const char* input_file, int num_cores, int device, u64
   return NB_OK;
 }
 
+// ------------------------------------------------------------------ bulk mode (nb_process_bam_bulk)
+struct BulkRun { AnyOrderLoad ld; nbg::BulkPairs bp; bool paired = true; double t_load = 0, t_pair = 0; };
+
+// The file into the store (LoadPolicy::bulk) and its pairs on the device.  A file with both paired and single-end kept
+// records is refused before anything is aligned.
+int bulk_load_pair(const char* input_file, int threads, nbg::Device* dev, BulkRun& run) {
+  nbg::set_bulk(dev, true);
+  CellDict none;
+  const double t0 = now();
+  int rc = any_order_load(input_file, threads, window_bytes(), dev, none, run.ld, LoadPolicy::bulk());
+  if (rc == NB_OK) { const double tw = now(); rc = nbg::sync(dev); run.ld.t_wait += now() - tw; }
+  if (rc) return rc;
+  const double t1 = now(); run.t_load = t1 - t0;
+  if (run.ld.first_paired != ~0ull && run.ld.first_single != ~0ull)
+    return fail(NB_ERR_UNSUPPORTED, std::string("--bulk needs a file whose kept records are either all paired (flag 0x1) or all single-end: record ") + std::to_string(run.ld.first_paired) +
+                                    " of " + input_file + " is paired and record " + std::to_string(run.ld.first_single) + " is not");
+  run.paired = run.ld.first_single == ~0ull;
+  u32 bits = 64;   // NB_BULK_NAME_HASH_BITS=b keeps b bits of the name key (tests force collisions with it)
+  if (const char* e = getenv("NB_BULK_NAME_HASH_BITS")) bits = (u32)std::max(1L, std::min(64L, strtol(e, nullptr, 10)));
+  rc = nbg::pair_bulk(dev, run.paired, bits, run.bp);
+  run.t_pair = now() - t1;
+  return rc;
+}
+
+// Batches of at most 2^20 pairs; NB_BULK_BATCH_PAIRS=N makes them smaller (tests use it to cut a file into many batches).
+u64 bulk_batch_pairs() {
+  u64 n = 1u << 20;
+  if (const char* e = getenv("NB_BULK_BATCH_PAIRS")) n = std::min<u64>(n, std::max<u64>(1, strtoull(e, nullptr, 10)));
+  return n;
+}
+
+// The library loop of nb_process_fastq with the BAM in place of the FASTQs: per library its index and one whole-run
+// context; the file is loaded and paired once, before the first library's batches; every pair is aligned, the counts
+// finalized once and written by the FASTQ-mode writer (append, header iff the file is empty).
+int process_bam_bulk(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs, int strand_filter, int num_cores, int device) {
+  if (!input_file || !reference_json || !output_paths || n_refs < 1) return fail(NB_ERR_INVALID, "need an input BAM and >=1 reference/output pair");
+  const double t_start = now();
+  const int threads = std::max(1, num_cores);
+  nbg::Device* dev = nullptr;
+  struct Store { nbg::Device*& d; ~Store() { nbg::destroy(d); } } store{dev};
+  int rc = nbg::create(device, &dev);
+  if (rc) return rc;
+  BulkRun run; double t_align = 0; u64 n_batches = 0;
+  const u64 BATCH = bulk_batch_pairs();
+  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+    nb_library* lib = nullptr; nb_index* ix = nullptr; nb_ctx* ctx = nullptr;
+    rc = nb_library_load_json(reference_json[li], strand_filter, &lib);
+    if (rc == NB_OK) rc = nb_index_build_cached(lib, nullptr, device, threads, &ix);
+    if (rc == NB_OK) rc = nb_ctx_create(ix, lib, device, nbg::stream_of(dev), &ctx);   // the batches point into the store: its stream
+    if (rc == NB_OK) rc = nb_ctx_set_option(ctx, "max_batch_pairs", BATCH);
+    if (rc == NB_OK && li == 0) rc = bulk_load_pair(input_file, threads, dev, run);
+    const double ta = now();
+    for (u64 p0 = 0; p0 < run.bp.n_pairs && rc == NB_OK; p0 += BATCH) {
+      nb_batch b; rc = nbg::batch(dev, p0, std::min(run.bp.n_pairs, p0 + BATCH), 0, run.bp.max_len, b);
+      if (rc == NB_OK) rc = nb_align_batch(ctx, &b, nullptr, nullptr);
+      n_batches++;
+    }
+    nb_counts cts;
+    if (rc == NB_OK) rc = nb_counts_finalize(ctx, &cts);
+    t_align += now() - ta;
+    if (rc == NB_OK) rc = nb_write_fastq_tsv(output_paths[li], lib, &cts);
+    nb_ctx_free(ctx); nb_index_free(ix); nb_library_free(lib);
+  }
+  if (getenv("NB_BAM_STATS")) {
+    const nbg::BulkPairs& bp = run.bp;
+    fprintf(stderr, "nb_process_bam_bulk: %llu records, %llu kept, %s, %llu pairs, dropped %llu singletons, %llu unsplit (not one READ1-only and one READ2-only), %llu in templates of 3+, %llu batches; windows (read+inflate+stage+upload) %.2fs, upload wait %.3fs, largest window %.0f MB, key+sort+pairing %.3fs, align+finalize %.3fs, total %.2fs, store %llu bytes, peak RSS %.0f MB\n",
+            (unsigned long long)run.ld.n_records, (unsigned long long)run.ld.n_kept, run.paired ? "paired" : "single-end", (unsigned long long)bp.n_pairs, (unsigned long long)bp.singletons,
+            (unsigned long long)bp.unsplit, (unsigned long long)bp.multi, (unsigned long long)n_batches, run.t_load, run.ld.t_wait, run.ld.peak_window / 1048576.0, run.t_pair, t_align,
+            now() - t_start, (unsigned long long)nbg::store_bytes(dev), peak_rss_mb());
+  }
+  return rc;
+}
+
+// One line per pair, sorted by R1 ordinal: R1 ordinal, R2 ordinal ('-' single-end), both lengths, both NB_FLAG_* bytes
+// ('-' for the missing mate).
+int dump_pairs_bulk(const char* input_file, int num_cores, int device, const char* out_path) {
+  if (!input_file || !out_path) return fail(NB_ERR_INVALID, "null argument");
+  nbg::Device* dev = nullptr;
+  struct Store { nbg::Device*& d; ~Store() { nbg::destroy(d); } } store{dev};
+  int rc = nbg::create(device, &dev);
+  BulkRun run;
+  if (rc == NB_OK) rc = bulk_load_pair(input_file, std::max(1, num_cores), dev, run);
+  std::vector<u64> o1, o2; std::vector<u8> f1, f2; std::vector<u32> l1, l2;
+  if (rc == NB_OK) rc = nbg::pairs_to_host(dev, o1, o2, f1, f2, l1, l2);
+  if (rc) return rc;
+  std::vector<u64> order(o1.size());
+  for (u64 p = 0; p < order.size(); p++) order[p] = p;
+  std::sort(order.begin(), order.end(), [&](u64 a, u64 b) { return o1[a] < o1[b]; });
+  std::string out; char line[160];
+  for (u64 p : order) {
+    if (run.paired) snprintf(line, sizeof line, "%llu\t%llu\t%u\t%u\t%u\t%u\n", (unsigned long long)o1[p], (unsigned long long)o2[p], l1[p], l2[p], f1[p], f2[p]);
+    else snprintf(line, sizeof line, "%llu\t-\t%u\t-\t%u\t-\n", (unsigned long long)o1[p], l1[p], f1[p]);
+    out += line;
+  }
+  FILE* f = fopen(out_path, "wb"); if (!f) return fail(NB_ERR_IO, std::string("could not open ") + out_path);
+  const bool ok = fwrite(out.data(), 1, out.size(), f) == out.size();
+  if (fclose(f) != 0 || !ok) return fail(NB_ERR_IO, std::string("short write on ") + out_path);
+  return NB_OK;
+}
+
 }  // namespace
+
+extern "C" int nb_process_bam_bulk(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
+                                   int strand_filter, int num_cores, int device) {
+  return process_bam_bulk(input_file, reference_json, output_paths, n_refs, strand_filter, num_cores, device);
+}
+
+extern "C" int nb_bam_dump_pairs_bulk(const char* input_file, int num_cores, int device, const char* out_path) {
+  return dump_pairs_bulk(input_file, num_cores, device, out_path);
+}
 
 extern "C" int nb_process_bam_cells_any_order(const char* input_file, const char* const* reference_json, const char* const* matrix_dirs, uint32_t n_refs,
                                               int strand_filter, const char* trim, int num_cores, int device) {

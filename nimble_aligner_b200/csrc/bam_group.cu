@@ -10,6 +10,8 @@
 // Rows mode (nb_process_bam_rows_any_order) keeps every record's metadata text in a fourth byte store, and the row kernels
 // below turn each aligned batch into the grouped driver's TSV rows next to it.  One driver, process_bam_any_order in bam.cpp,
 // runs both modes, with or without a budget: they differ only in what follows each batch's finalize.
+// Bulk mode (nb_process_bam_bulk) keeps a store without quals, UMI keys or CB ids and pairs the mates by name instead:
+// one radix sort of a 64-bit QNAME hash, then templates resolved by exact name compare within each run of equal key.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -184,6 +186,96 @@ __global__ void k_local_scope(const u32* __restrict__ scope, u32* __restrict__ l
 }
 
 inline u32 blocks(u64 n, u32 t = 256) { return (u32)((n + t - 1) / t); }
+
+// ------------------------------------------------------------------------------------------------ bulk mode (pair_bulk)
+// name key of every kept record: a 64-bit hash of its QNAME bytes, low `mask` bits kept; val = kept index
+__global__ void k_name_keys(const u64* __restrict__ name_off, const u8* __restrict__ name_len, const char* __restrict__ names, u64 mask, u64* __restrict__ key, u32* __restrict__ val, u32 n) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const u8* p = (const u8*)names + name_off[i]; const u32 l = name_len[i];
+  u64 h = 0xCBF29CE484222325ull ^ l;
+  for (u32 k = 0; k < l; k++) h = (h ^ p[k]) * 0x100000001B3ull;
+  h ^= h >> 30; h *= 0xBF58476D1CE4E5B9ull; h ^= h >> 27; h *= 0x94D049BB133111EBull; h ^= h >> 31;
+  key[i] = h & mask; val[i] = i;
+}
+__global__ void k_key_heads(const u64* __restrict__ key, u32* __restrict__ head, u32 n) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) head[i] = (i == 0 || key[i] != key[i - 1]) ? 1u : 0u;
+}
+
+const u32 NO_REC = 0xFFFFFFFFu;
+const u32 LONG_RUN = 32;   // longer runs of equal key are resolved by the whole warp
+// The template of the record at sorted position j of the run [a, b) when j is its first record there (false otherwise):
+// its size n and its READ1-only and READ2-only members.
+__device__ bool bulk_template(const Recs& d, u32 a, u32 b, u32 j, u32& n, u32& r1, u32& r2) {
+  const u32 r = d.perm[j];
+  for (u32 k = a; k < j; k++) if (same_name(d, d.perm[k], r)) return false;
+  n = 0; r1 = r2 = NO_REC;
+  for (u32 k = j; k < b; k++) {
+    const u32 x = d.perm[k];
+    if (k != j && !same_name(d, x, r)) continue;
+    n++;
+    const u32 f = d.flag[x] & 0xC0;
+    if (f == 0x40) r1 = x; else if (f == 0x80) r2 = x;
+  }
+  return true;
+}
+// a template's pair, or its records counted by why they are dropped (st: singletons, unsplit, multi, longest read)
+__device__ __forceinline__ bool bulk_pair(u32 n, u32 r1, u32 r2, unsigned long long* st) {
+  if (n == 2 && r1 != NO_REC && r2 != NO_REC) return true;
+  if (st) atomicAdd(st + (n == 1 ? 0 : n == 2 ? 1 : 2), (unsigned long long)n);
+  return false;
+}
+__device__ __forceinline__ void bulk_slot(const Recs& d, u32 r, u64& o, u32& l, u8& f) {
+  o = 2 * d.nib_off[r]; l = d.lseq[r]; f = (d.flag[r] & 16) ? (u8)NB_FLAG_REVCOMP_FASTQ : (u8)0;
+}
+__device__ __forceinline__ void bulk_write(const Recs& d, const PairsOut& out, u64 p, u32 r1, u32 r2, unsigned long long* st) {
+  bulk_slot(d, r1, out.o1[p], out.l1[p], out.f1[p]); bulk_slot(d, r2, out.o2[p], out.l2[p], out.f2[p]);
+  out.idx1[p] = r1; out.idx2[p] = r2;
+  atomicMax(st + 3, (unsigned long long)max(out.l1[p], out.l2[p]));
+}
+// Runs [start[s], start[s + 1]) of equal name key, s < n_runs: a thread per run, and every run longer than LONG_RUN taken by
+// its whole warp in turn.  WRITE = false: cnt[s] = the run's pairs (cnt[n_runs] = 0) and the drop counts; true: the pairs at
+// pair0[s] on, in the order of their first records in the run.  The grid covers n_runs + 1 threads in whole warps.
+template <bool WRITE>
+__global__ void k_bulk_pairs(Recs d, const u32* __restrict__ start, u32 n_runs, u64* __restrict__ cnt, const u64* __restrict__ pair0, PairsOut out, unsigned long long* st) {
+  const u32 s = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31;
+  const bool mine = s < n_runs;
+  const u32 a = mine ? start[s] : 0, b = mine ? start[s + 1] : 0;
+  const bool lng = mine && b - a > LONG_RUN;
+  if (!WRITE && s == n_runs) cnt[n_runs] = 0;
+  if (mine && !lng) {
+    u64 np = 0;
+    for (u32 j = a; j < b; j++) {
+      u32 n, r1, r2;
+      if (!bulk_template(d, a, b, j, n, r1, r2) || !bulk_pair(n, r1, r2, WRITE ? nullptr : st)) continue;
+      if (WRITE) bulk_write(d, out, pair0[s] + np, r1, r2, st);
+      np++;
+    }
+    if (!WRITE) cnt[s] = np;
+  }
+  for (unsigned L = __ballot_sync(0xFFFFFFFFu, lng); L; L &= L - 1) {
+    const int src = __ffs(L) - 1;
+    const u32 la = __shfl_sync(0xFFFFFFFFu, a, src), lb = __shfl_sync(0xFFFFFFFFu, b, src), ls = __shfl_sync(0xFFFFFFFFu, s, src);
+    u64 np = 0;
+    for (u32 j0 = la; j0 < lb; j0 += 32) {
+      const u32 j = j0 + lane; u32 n = 0, r1 = NO_REC, r2 = NO_REC;
+      const bool ok = j < lb && bulk_template(d, la, lb, j, n, r1, r2) && bulk_pair(n, r1, r2, WRITE ? nullptr : st);
+      const unsigned m = __ballot_sync(0xFFFFFFFFu, ok);
+      if (WRITE && ok) bulk_write(d, out, pair0[ls] + np + __popc(m & ((1u << lane) - 1)), r1, r2, st);
+      np += __popc(m);
+    }
+    if (!WRITE && lane == 0) cnt[ls] = np;
+  }
+}
+// single-end: one slot per kept record, in kept order
+__global__ void k_bulk_single(Recs d, PairsOut out, u32 n, unsigned long long* st) {
+  const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  bulk_slot(d, i, out.o1[i], out.l1[i], out.f1[i]);
+  out.o2[i] = out.o1[i]; out.l2[i] = 0; out.f2[i] = 0; out.idx1[i] = out.idx2[i] = i;
+  atomicMax(st + 3, (unsigned long long)out.l1[i]);
+}
 
 // ---------------------------------------------------------------------------------------- compaction (budget mode)
 // keep flag of every record (its UMI bucket is below hi) and its kept nibble / name bytes; entry n is 0, so exclusive
@@ -407,6 +499,7 @@ struct Device {
   Grow nib, qual, name, umi, cb, nib_off, lseq, flag, name_off, name_len, ordinal, meta, meta_off, meta_len, f0_len;
   u64 n_rec = 0, n_nib = 0, n_name = 0, n_meta = 0;
   bool rows = false;
+  bool bulk = false, paired = true;   // bulk mode: no quals, UMI keys or CB ids in the store; whole-run batches
   // staging: two slots, the producer fills one while the other's copies run
   struct Slot { Stage st; Pinned nib, qual, name, umi, cb, nib_off, lseq, flag, name_off, name_len, ordinal, meta, meta_off, meta_len, f0_len; cudaEvent_t done = nullptr; bool used = false; } slot[2];
   int cur = 0;
@@ -530,6 +623,7 @@ u64 store_bytes(Device* d) { return d->total(); }
 u64 group_bytes(Device* d) { return d->g_bytes + d->p_bytes; }
 void set_budget(Device* d, u64 budget_bytes) { d->mem.budget = budget_bytes; }
 void set_rows(Device* d, bool rows) { d->rows = rows; }
+void set_bulk(Device* d, bool bulk) { d->bulk = bulk; }
 u64 meta_bytes(Device* d) { return d->meta.cap + d->meta_off.cap + d->meta_len.cap + d->f0_len.cap; }
 u64 peak_bytes(Device* d) { return d->mem.peak; }
 
@@ -604,8 +698,9 @@ int stage(Device* d, u64 n_rec, u64 n_nib, u64 n_name, u64 n_meta, Stage*& st) {
   if (sl.used) GK(cudaEventSynchronize(sl.done));
   int e = NB_OK;
   const u64 r = std::max<u64>(n_rec, 1);
-  if (!e) e = sl.nib.ensure(n_nib + 1); if (!e) e = sl.qual.ensure(2 * n_nib + 1); if (!e) e = sl.name.ensure(n_name + 1);
-  if (!e) e = sl.umi.ensure(8 * r); if (!e) e = sl.cb.ensure(4 * r); if (!e) e = sl.nib_off.ensure(8 * r); if (!e) e = sl.lseq.ensure(4 * r);
+  const u64 rk = d->bulk ? 0 : r;   // bulk: no quals, UMI keys or CB ids
+  if (!e) e = sl.nib.ensure(n_nib + 1); if (!e) e = sl.qual.ensure(2 * (rk ? n_nib : 0) + 1); if (!e) e = sl.name.ensure(n_name + 1);
+  if (!e) e = sl.umi.ensure(8 * rk + 8); if (!e) e = sl.cb.ensure(4 * rk + 4); if (!e) e = sl.nib_off.ensure(8 * r); if (!e) e = sl.lseq.ensure(4 * r);
   if (!e) e = sl.flag.ensure(2 * r); if (!e) e = sl.name_off.ensure(8 * r); if (!e) e = sl.name_len.ensure(r); if (!e) e = sl.ordinal.ensure(8 * r);
   if (d->rows) { if (!e) e = sl.meta.ensure(n_meta + 1); if (!e) e = sl.meta_off.ensure(8 * r); if (!e) e = sl.meta_len.ensure(4 * r); if (!e) e = sl.f0_len.ensure(4 * r); }
   if (e) return e;
@@ -625,13 +720,15 @@ int upload(Device* d, u64 reserve) {
   if (R >= 0x7FFFFFFFull) return fail(NB_ERR_UNSUPPORTED, "more than 2^31 - 1 kept records");
   cudaStream_t s = d->s;
   u64 need[Device::N_ARR], keep[Device::N_ARR]; Device::needs(R, NB, NM, NT, need); Device::needs(d->n_rec, d->n_nib, d->n_name, d->n_meta, keep);
+  if (d->bulk) for (int k : {1, 3, 4}) need[k] = keep[k] = 0;   // quals, UMI keys, CB ids
   u64 tot = 0; for (int k = 0; k < d->n_arr(); k++) tot += need[k];
   const bool exact = d->mem.budget && !grows_within(d, R, NB, NM, NT, reserve, false);   // the slack would not fit: grow exactly
   for (int k = 0; k < d->n_arr(); k++) { const int e = d->arrays[k]->ensure(need[k], keep[k], s, WHAT[k], tot, d->mem, reserve, exact); if (e) return e; }
   auto cp = [&](Grow& g, u64 at, const void* src, u64 n) -> cudaError_t { return n ? cudaMemcpyAsync((char*)g.p + at, src, n, cudaMemcpyHostToDevice, s) : cudaSuccess; };
   const u64 r0 = d->n_rec, n = t.n_rec;
-  GK(cp(d->nib, d->n_nib, t.nib, t.n_nib)); GK(cp(d->qual, 2 * d->n_nib, t.qual, 2 * t.n_nib)); GK(cp(d->name, d->n_name, t.name, t.n_name));
-  GK(cp(d->umi, 8 * r0, t.umi, 8 * n)); GK(cp(d->cb, 4 * r0, t.cb, 4 * n)); GK(cp(d->nib_off, 8 * r0, t.nib_off, 8 * n)); GK(cp(d->lseq, 4 * r0, t.lseq, 4 * n));
+  GK(cp(d->nib, d->n_nib, t.nib, t.n_nib)); GK(cp(d->name, d->n_name, t.name, t.n_name));
+  if (!d->bulk) { GK(cp(d->qual, 2 * d->n_nib, t.qual, 2 * t.n_nib)); GK(cp(d->umi, 8 * r0, t.umi, 8 * n)); GK(cp(d->cb, 4 * r0, t.cb, 4 * n)); }
+  GK(cp(d->nib_off, 8 * r0, t.nib_off, 8 * n)); GK(cp(d->lseq, 4 * r0, t.lseq, 4 * n));
   GK(cp(d->flag, 2 * r0, t.flag, 2 * n)); GK(cp(d->name_off, 8 * r0, t.name_off, 8 * n)); GK(cp(d->name_len, r0, t.name_len, n)); GK(cp(d->ordinal, 8 * r0, t.ordinal, 8 * n));
   if (d->rows) { GK(cp(d->meta, d->n_meta, t.meta, t.n_meta)); GK(cp(d->meta_off, 8 * r0, t.meta_off, 8 * n)); GK(cp(d->meta_len, 4 * r0, t.meta_len, 4 * n)); GK(cp(d->f0_len, 4 * r0, t.f0_len, 4 * n)); }
   GK(cudaEventRecord(sl.done, s));
@@ -706,6 +803,22 @@ int compact(Device* d, u32 hi) {
   return rc;
 }
 
+namespace {
+// the pair arrays for np pairs (the previous ones released)
+int alloc_pairs(Device* d, u64 np, PairsOut& out) {
+  d->n_pairs = np;
+  d->mem.release(d->p_buf, d->p_bytes); d->p_bytes = 0;
+  const PairLayout P = pair_layout(np);
+  if (d->mem.alloc(&d->p_buf, P.bytes) != cudaSuccess) { cudaGetLastError(); d->p_buf = nullptr; return fail(NB_ERR_CUDA, "not enough device memory for the pairs: " + std::to_string(P.bytes) + " bytes needed"); }
+  d->p_bytes = P.bytes;
+  char* Q = (char*)d->p_buf;
+  d->o1 = (u64*)(Q + P.o[0]); d->o2 = (u64*)(Q + P.o[1]); d->l1 = (u32*)(Q + P.o[2]); d->l2 = (u32*)(Q + P.o[3]); d->f1 = (u8*)(Q + P.o[4]); d->f2 = (u8*)(Q + P.o[5]);
+  d->scope = (u32*)(Q + P.o[6]); d->idx1 = (u32*)(Q + P.o[7]); d->idx2 = (u32*)(Q + P.o[8]); d->local = (u32*)(Q + P.o[9]);
+  out = PairsOut{d->o1, d->o2, d->l1, d->l2, d->f1, d->f2, d->scope, d->idx1, d->idx2};
+  return NB_OK;
+}
+}  // namespace
+
 int group(Device* d, const std::vector<u32>& cb_rank, const std::vector<u32>& cb_prefix, Grouped& g) {
   GK(cudaSetDevice(d->device));
   cudaStream_t s = d->s;
@@ -751,15 +864,8 @@ int group(Device* d, const std::vector<u32>& cb_rank, const std::vector<u32>& cb
   GK(cudaMemcpyAsync(g.scope_cb.data(), scb, 4ull * n_scopes, cudaMemcpyDeviceToHost, s));
   GK(cudaStreamSynchronize(s));
   const u64 np = g.n_pairs = g.scope_pair0[n_scopes];
-  d->n_pairs = np;
-  d->mem.release(d->p_buf, d->p_bytes); d->p_bytes = 0;
-  const PairLayout P = pair_layout(np);
-  if (d->mem.alloc(&d->p_buf, P.bytes) != cudaSuccess) { cudaGetLastError(); d->p_buf = nullptr; return fail(NB_ERR_CUDA, "not enough device memory for the pairs: " + std::to_string(P.bytes) + " bytes needed"); }
-  d->p_bytes = P.bytes;
-  char* Q = (char*)d->p_buf;
-  d->o1 = (u64*)(Q + P.o[0]); d->o2 = (u64*)(Q + P.o[1]); d->l1 = (u32*)(Q + P.o[2]); d->l2 = (u32*)(Q + P.o[3]); d->f1 = (u8*)(Q + P.o[4]); d->f2 = (u8*)(Q + P.o[5]);
-  d->scope = (u32*)(Q + P.o[6]); d->idx1 = (u32*)(Q + P.o[7]); d->idx2 = (u32*)(Q + P.o[8]); d->local = (u32*)(Q + P.o[9]);
-  PairsOut out{d->o1, d->o2, d->l1, d->l2, d->f1, d->f2, d->scope, d->idx1, d->idx2};
+  PairsOut out;
+  if (int e = alloc_pairs(d, np, out)) return e;
   if (np) k_pair_write<<<blocks(n_scopes, 128), 128, 0, s>>>(R, start, pair0, out, n_scopes);
   GK(cudaGetLastError());
   GK(cudaStreamSynchronize(s));
@@ -768,12 +874,69 @@ int group(Device* d, const std::vector<u32>& cb_rank, const std::vector<u32>& cb
   return NB_OK;
 }
 
+int pair_bulk(Device* d, bool paired, u32 hash_bits, BulkPairs& bp) {
+  GK(cudaSetDevice(d->device));
+  cudaStream_t s = d->s;
+  const u32 n = (u32)d->n_rec;
+  bp = BulkPairs(); d->paired = paired;
+  if (n == 0) { d->n_pairs = 0; return NB_OK; }
+  // the sort and run arrays are group()'s layout with no CB ranks: name keys in u1 -> u2, kept indices in v0 -> v2
+  GroupLayout L;
+  if (int e = group_layout(n, 0, s, L)) return e;
+  d->mem.release(d->g_buf, d->g_bytes); d->g_bytes = 0;
+  const u64 st_bytes = 256;
+  if (d->mem.alloc(&d->g_buf, L.bytes + st_bytes) != cudaSuccess) { cudaGetLastError(); d->g_buf = nullptr; return fail(NB_ERR_CUDA, "not enough device memory to pair the records: " + std::to_string(L.bytes + st_bytes) + " bytes needed"); }
+  d->g_bytes = L.bytes + st_bytes;
+  char* B = (char*)d->g_buf;
+  u32* v0 = (u32*)(B + L.o_v0); u32* perm = (u32*)(B + L.o_v2); u64* u1 = (u64*)(B + L.o_u1); u64* u2 = (u64*)(B + L.o_u2);
+  u32* head = (u32*)(B + L.o_head); u32* sid = (u32*)(B + L.o_sid); u32* start = (u32*)(B + L.o_start); u64* cnt = (u64*)(B + L.o_cnt); u64* pair0 = (u64*)(B + L.o_p0);
+  void* tmp = B + L.o_tmp; unsigned long long* st = (unsigned long long*)(B + L.bytes);   // singletons, unsplit, multi, longest read
+  GK(cudaMemsetAsync(st, 0, 32, s));
+  Recs R{perm, (const u64*)d->nib_off.p, (const u32*)d->lseq.p, (const u16*)d->flag.p, (const u64*)d->name_off.p, (const u8*)d->name_len.p, (const char*)d->name.p, nullptr};
+  PairsOut out;
+  if (!paired) {
+    if (int e = alloc_pairs(d, n, out)) return e;
+    k_bulk_single<<<blocks(n), 256, 0, s>>>(R, out, n, st);
+  } else {
+    const u32 bits = std::max<u32>(1, std::min<u32>(hash_bits, 64));
+    k_name_keys<<<blocks(n), 256, 0, s>>>((const u64*)d->name_off.p, (const u8*)d->name_len.p, (const char*)d->name.p, bits == 64 ? ~0ull : (1ull << bits) - 1, u1, v0, n);
+    size_t tb = L.tmp_bytes;
+    GK(cub::DeviceRadixSort::SortPairs(tmp, tb, u1, u2, v0, perm, (int)n, 0, (int)bits, s));
+    k_key_heads<<<blocks(n), 256, 0, s>>>(u2, head, n);
+    tb = L.tmp_bytes; GK(cub::DeviceScan::InclusiveSum(tmp, tb, head, sid, (int)n, s));
+    k_starts<<<blocks(n), 256, 0, s>>>(head, sid, start, n);
+    u32 n_runs = 0;
+    GK(cudaMemcpyAsync(&n_runs, sid + n - 1, 4, cudaMemcpyDeviceToHost, s));
+    GK(cudaStreamSynchronize(s));
+    k_bulk_pairs<false><<<blocks((u64)n_runs + 1, 128), 128, 0, s>>>(R, start, n_runs, cnt, nullptr, PairsOut{}, st);
+    tb = L.tmp_bytes; GK(cub::DeviceScan::ExclusiveSum(tmp, tb, cnt, pair0, (int)n_runs + 1, s));
+    u64 np = 0;
+    GK(cudaMemcpyAsync(&np, pair0 + n_runs, 8, cudaMemcpyDeviceToHost, s));
+    GK(cudaStreamSynchronize(s));
+    if (int e = alloc_pairs(d, np, out)) return e;
+    if (np) k_bulk_pairs<true><<<blocks((u64)n_runs + 1, 128), 128, 0, s>>>(R, start, n_runs, cnt, pair0, out, st);
+  }
+  unsigned long long h[4];
+  GK(cudaMemcpyAsync(h, st, 32, cudaMemcpyDeviceToHost, s));
+  GK(cudaGetLastError());
+  GK(cudaStreamSynchronize(s));
+  bp.n_pairs = d->n_pairs; bp.singletons = h[0]; bp.unsplit = h[1]; bp.multi = h[2]; bp.max_len = (u32)h[3];
+  { const u64 gb = d->g_bytes; d->mem.release(d->g_buf, gb); d->g_bytes = 0; }
+  return NB_OK;
+}
+
 int batch(Device* d, u64 p0, u64 p1, u64 scope0, u32 max_read_len, nb_batch& b) {
   memset(&b, 0, sizeof b);
   const u64 np = p1 - p0;
+  b.n_pairs = np; b.location = NB_MEM_DEVICE; b.max_read_len = max_read_len; b.encoding = NB_SEQ_BAM4;
+  if (d->bulk) {   // one whole-run scope, no quals (FASTQ mode does not trim)
+    b.r1 = (const u8*)d->nib.p; b.r2 = d->paired ? (const u8*)d->nib.p : nullptr;
+    b.r1_off = d->o1 + p0; b.r1_len = d->l1 + p0; b.flags1 = d->f1 + p0;
+    if (d->paired) { b.r2_off = d->o2 + p0; b.r2_len = d->l2 + p0; b.flags2 = d->f2 + p0; }
+    return NB_OK;
+  }
   if (np) k_local_scope<<<(u32)((np + 255) / 256), 256, 0, d->s>>>(d->scope + p0, d->local + p0, np, (u32)scope0);
   GK(cudaGetLastError());
-  b.n_pairs = np; b.location = NB_MEM_DEVICE; b.max_read_len = max_read_len; b.encoding = NB_SEQ_BAM4;
   b.r1 = b.r2 = (const u8*)d->nib.p; b.q1 = b.q2 = (const u8*)d->qual.p;
   b.r1_off = d->o1 + p0; b.r2_off = d->o2 + p0; b.r1_len = d->l1 + p0; b.r2_len = d->l2 + p0;
   b.flags1 = d->f1 + p0; b.flags2 = d->f2 + p0; b.scope_id = d->local + p0;

@@ -1,7 +1,8 @@
 // bam_group.hpp — the device record store of BAM mode in any record order (bam.cpp's process_bam_any_order, the one driver
 // behind nb_process_bam_cells_any_order[_budget] and nb_process_bam_rows_any_order): the host producer stages every kept
 // record's nibbles, quals, name and keys window by window; the device sorts the records by (UMI, CB), cuts the
-// (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into the store.
+// (UMI, CB[..len-2]) scopes, pairs each scope's records and hands out scoped batches that point into the store.  Bulk mode
+// (bam.cpp's process_bam_bulk) stages no quals or cell keys and pairs the mates of the whole file by name (pair_bulk).
 // Host-only declarations (bam.cpp includes them; bam_group.cu implements them).
 #pragma once
 #include <functional>
@@ -95,12 +96,30 @@ struct Grouped {
 };
 // cb_rank[id] = rank of CB id in byte order, cb_prefix[id] = id of its CB[..len-2]
 int group(Device*, const std::vector<u32>& cb_rank, const std::vector<u32>& cb_prefix, Grouped& g);
-// Fills a device-resident NB_SEQ_BAM4 batch over pairs [p0, p1) whose scope ids are local to the batch (scope - scope0).
+// Fills a device-resident NB_SEQ_BAM4 batch over pairs [p0, p1) whose scope ids are local to the batch (scope - scope0);
+// bulk mode: a whole-run batch (scope0 unused).
 int batch(Device*, u64 p0, u64 p1, u64 scope0, u32 max_read_len, nb_batch& b);
 // Test hook: per pair the file ordinals of both slots, their flags and clipped lengths.
 int pairs_to_host(Device*, std::vector<u64>& ord1, std::vector<u64>& ord2, std::vector<u8>& f1, std::vector<u8>& f2, std::vector<u32>& l1, std::vector<u32>& l2);
 // Test hook: per pair the base offsets of both slots into the store, and the nibble and qual stores as they are now.
 int slots_to_host(Device*, std::vector<u64>& off1, std::vector<u64>& off2, std::vector<u8>& nib, std::vector<u8>& qual);
+// ---- bulk mode (nb_process_bam_bulk): FASTQ-mode counts of a BAM without cell barcodes, mates paired by name on the device
+// Before the first stage: the store keeps nibbles, names, offsets, lengths, flags and ordinals only (no quals, UMI keys or
+// CB ids are staged or uploaded), and batch() hands out whole-run batches (no scope ids, no quals; r2 = NULL single-end).
+void set_bulk(Device*, bool bulk);
+struct BulkPairs {
+  u64 n_pairs = 0;
+  u64 singletons = 0, unsplit = 0, multi = 0;   // dropped records: templates of one record, of two that are not READ1-only + READ2-only, of three or more
+  u32 max_len = 0;                              // longest read of a pair
+};
+// After the last upload.  paired: every kept record has flag 0x1 (else none has): a template is the kept records with
+// byte-equal QNAME, and one of exactly two records, one READ1-only (0x40 without 0x80) and one READ2-only, is a pair
+// (R1 in slot 1); every other record is dropped.  The name key is a 64-bit hash of the QNAME (hash_bits < 64 keeps its
+// low bits: tests force collisions); one radix sort of (key -> kept index), runs of equal key, and per run a count pass,
+// a scan and a write pass resolve the templates by exact name compare (a thread per run, a warp per run of more than 32
+// records).  Single-end: one slot per kept record.  A REVERSE record's slot carries NB_FLAG_REVCOMP_FASTQ.  No TSO clip.
+int pair_bulk(Device*, bool paired, u32 hash_bits, BulkPairs& bp);
+
 u64 store_records(Device*);     // records in the store
 u64 store_bytes(Device*);       // device bytes of the record store (nibbles, quals, names, per-record keys)
 u64 group_bytes(Device*);       // device bytes of the sort, scope and pair arrays

@@ -211,6 +211,16 @@ __device__ __forceinline__ u64 nib16_to_codes(u64 x) {
   c = (c | (c >> 8)) & 0x0000FFFF0000FFFFULL; c = (c | (c >> 16)) & 0xFFFFFFFFULL;
   return c;
 }
+// 16 nibbles -> 16 two-bit fields in the low 32 bits, 3 where the nibble is A, C, G or T and 0 elsewhere
+__device__ __forceinline__ u64 nib16_acgt(u64 x) {
+  const u64 M = 0x1111111111111111ULL;
+  u64 sum = (x & M) + ((x >> 1) & M) + ((x >> 2) & M) + ((x >> 3) & M);
+  u64 v = sum & ~(sum >> 1) & ~(sum >> 2) & M;
+  u64 c = v | (v << 1);
+  c = (c | (c >> 2)) & 0x0F0F0F0F0F0F0F0FULL; c = (c | (c >> 4)) & 0x00FF00FF00FF00FFULL;
+  c = (c | (c >> 8)) & 0x0000FFFF0000FFFFULL; c = (c | (c >> 16)) & 0xFFFFFFFFULL;
+  return c;
+}
 template <int ENC>
 __global__ void __launch_bounds__(256) k_pack_enc(BatchDev b) {
   u32 idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -220,9 +230,12 @@ __global__ void __launch_bounds__(256) k_pack_enc(BatchDev b) {
   if (w == Wd - 1) b.pk[(u64)ri * b.W + Wd] = 0;
   u32 side = b.sides == 2 ? (ri & 1) : 0; u64 p = b.sides == 2 ? (ri >> 1) : ri;
   u64 o0 = b.off[side][p]; u32 len = b.len[side] ? b.len[side][p] : (u32)(b.off[side][p + 1] - o0);
-  bool rc = b.flags[side] != nullptr && (b.flags[side][p] & 2);
+  // NB_FLAG_REVCOMP_FASTQ (BAM4 only): reverse-complemented like NB_FLAG_REVCOMP, but a non-ACGT code stays A, as in the
+  // FASTQ that samtools writes for the record (its IUPAC complement is again non-ACGT, which FASTQ mode reads as A)
+  const bool fq = ENC == 2 && b.flags[side] != nullptr && (b.flags[side][p] & 4);
+  bool rc = fq || (b.flags[side] != nullptr && (b.flags[side][p] & 2));
   if (w == 0) { b.len_full[ri] = len; b.len_trim[ri] = len; }
-  u64 word = 0; u32 s = w * 32;
+  u64 word = 0, acgt = 0; u32 s = w * 32;
   if (s < len) {
     u32 cnt = min(32u, len - s);
     u64 src = rc ? (o0 + len - s - cnt) : (o0 + s);        // first base of the 32-base source stretch
@@ -240,9 +253,11 @@ __global__ void __launch_bounds__(256) k_pack_enc(BatchDev b) {
       u64 w0 = swap_nibbles(ld_al64(al, 0)), w1 = need > 64 ? swap_nibbles(ld_al64(al, 1)) : 0ULL, w2 = need > 128 ? swap_nibbles(ld_al64(al, 2)) : 0ULL;
       u64 lo = sh ? (w0 >> sh) | (w1 << (64 - sh)) : w0, hi = sh ? (w1 >> sh) | (w2 << (64 - sh)) : w1;
       word = nib16_to_codes(lo) | (nib16_to_codes(hi) << 32);
+      if (fq) acgt = nib16_acgt(lo) | (nib16_acgt(hi) << 32);
     }
     if (cnt < 32) word &= (1ULL << (2 * cnt)) - 1;
     if (rc) { word = rev2(word) >> (64 - 2 * cnt); word ^= cnt < 32 ? ((1ULL << (2 * cnt)) - 1) : ~0ULL; }
+    if (fq) word &= rev2(acgt) >> (64 - 2 * cnt);   // the complemented non-ACGT codes (T) back to A
   }
   b.pk[(u64)ri * b.W + w] = word;
 }
@@ -268,8 +283,8 @@ __global__ void __launch_bounds__(256) k_trim(BatchDev b, Tables t) {
   if (b.q[side] == nullptr) return;
   if (b.flags[side] != nullptr && (b.flags[side][p] & 1)) return;       // SKIP_ALIGN: the reference never trims (nor aligns) these, src/align.rs:527-528
   const u64 o0 = b.off[side][p]; const u32 len = b.len_full[ri];        // written by k_pack (packed encodings may carry explicit lengths)
-  const bool rc = b.flags[side] != nullptr && (b.flags[side][p] & 2);
-  const uintptr_t a0 = (uintptr_t)(b.q[side] + o0), a1 = a0 + len;
+  const bool rc = b.flags[side] != nullptr && (b.flags[side][p] & (b.enc == 2 ? 6 : 2));   // (NB_SEQ_BAM4: REVCOMP_FASTQ reverses like REVCOMP)
+  const uintptr_t a0 =(uintptr_t)(b.q[side] + o0), a1 = a0 + len;
   i64 acc = 0, best = INT64_MIN; u32 pos = 0, i = 0;
   auto step = [&](u32 qq) {
     acc += s_qp[qq];

@@ -25,7 +25,7 @@ static uint64_t parse_size(const std::string& t) {
 }
 
 int main(int argc, char** argv) {
-  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false, any_order = false; uint64_t device_budget = 0; bool have_budget = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
+  std::vector<std::string> refs, outs, ins, mats; bool have_mats = false, no_rows = false, any_order = false, bulk = false; uint64_t device_budget = 0; bool have_budget = false; std::string cores = "1", strand = "unstranded", trim, devs = getenv("NB_DEVICES") ? getenv("NB_DEVICES") : "0"; bool have_trim = false, force_paired = false;
   std::vector<std::string>* cur = nullptr;
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
@@ -42,6 +42,7 @@ int main(int argc, char** argv) {
     if (a == "--cell-matrix") { cur = &mats; have_mats = true; continue; }   // not in cli.yml: BAM mode, one directory per -r for a cell x feature matrix (10x v3 layout)
     if (a == "--no-rows") { no_rows = true; cur = nullptr; continue; }          // not in cli.yml: BAM mode, no TSV.gz rows (with --cell-matrix, without -o)
     if (a == "--any-order") { any_order = true; cur = nullptr; continue; }      // not in cli.yml: BAM mode, scopes from the tags of a BAM in any record order (-o rows, or --cell-matrix --no-rows)
+    if (a == "--bulk") { bulk = true; cur = nullptr; continue; }               // not in cli.yml: BAM input without cell barcodes, counted as FASTQ mode counts its FASTQs
     if (a == "--device-budget") { const std::string v = val("--device-budget"); device_budget = parse_size(v); have_budget = true; if (!device_budget) die("error: --device-budget needs a positive number of bytes with an optional K, M or G suffix, not '" + v + "'"); cur = nullptr; continue; }   // not in cli.yml: with --any-order, the device memory it may allocate
     if (a == "-h" || a == "--help") {
       printf("nimble 0.8.0 (B200)\nUSAGE: nimble [FLAGS] [OPTIONS] --input <input>... --output <output>... --reference <reference>...\n"
@@ -54,13 +55,16 @@ int main(int argc, char** argv) {
              "                                with --output, the TSV.gz rows in any order (assembled on the GPU); with\n"
              "                                --cell-matrix --no-rows, the matrices; (UMI, CB) scopes are formed on the GPU\n"
              "      --device-budget <size>    with --any-order: device memory it may allocate, bytes or with a K/M/G suffix\n"
-             "                                (powers of 1024); records that do not fit take more passes over the file\n");
+             "                                (powers of 1024); records that do not fit take more passes over the file\n"
+             "      --bulk                    BAM input without cell barcodes (e.g. STAR, HISAT2), any record order: the TSV that\n"
+             "                                FASTQ mode writes for its reads (mates paired by name on the GPU; -t is ignored)\n");
       return 0;
     }
     if (a == "-V" || a == "--version") { printf("nimble 0.8.0\n"); return 0; }
     if (!cur) die("error: Found argument '" + a + "' which wasn't expected, or isn't valid in this context");
     cur->push_back(a);
   }
+  if (bulk && (have_mats || no_rows || any_order || force_paired || have_budget)) die("error: --bulk counts a BAM as FASTQ mode counts reads: it takes no --cell-matrix, --no-rows, --any-order, -p or --device-budget");
   if (have_budget && !any_order) die("error: --device-budget needs --any-order");
   if (any_order && have_mats && !no_rows) die("error: --any-order writes either the TSV rows (--output) or the cell matrices (--cell-matrix --no-rows), not both: run the two modes separately");
   if (any_order && force_paired) die("error: --any-order cannot pair mates (-p): the mates of a position-sorted file are not neighbours");
@@ -90,13 +94,15 @@ int main(int argc, char** argv) {
   printf("Loading read sequences and aligning\n");
   std::vector<const char*> m; for (auto& s : mats) m.push_back(s.c_str());
   if (ends(first, ".fastq.gz") || ends(lower, ".fastq")) {
+    if (bulk) die("error: --bulk needs a BAM input");
     if (have_mats || no_rows || any_order) die("error: --cell-matrix, --no-rows and --any-order need a BAM input (FASTQ reads have no cells)");
     printf("Processing as FASTQ file\n");
     int rc = nb_process_fastq_devices(in.data(), (uint32_t)std::min<size_t>(in.size(), 2), r.data(), o.data(), (uint32_t)r.size(), chem, (int)ncores, devices.data(), (uint32_t)devices.size());
     if (rc != NB_OK) die(nb_last_error());
   } else if (ends(lower, ".bam")) {
     printf("Processing as BAM file\n");
-    int rc = (any_order && !have_mats) ? nb_process_bam_rows_any_order(in[0], r.data(), o.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], have_budget ? device_budget : 0)
+    int rc = bulk ? nb_process_bam_bulk(in[0], r.data(), o.data(), (uint32_t)r.size(), chem, (int)ncores, devices[0])
+           : (any_order && !have_mats) ? nb_process_bam_rows_any_order(in[0], r.data(), o.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], have_budget ? device_budget : 0)
            : any_order ? (have_budget ? nb_process_bam_cells_any_order_budget(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0], device_budget)
                                       : nb_process_bam_cells_any_order(in[0], r.data(), m.data(), (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, devices[0]))
                        : nb_process_bam_cells(in[0], r.data(), no_rows ? nullptr : o.data(), have_mats ? m.data() : nullptr, (uint32_t)r.size(), chem, have_trim ? trim.c_str() : nullptr, (int)ncores, force_paired ? 1 : 0, devices[0]);   // (BAM mode is bound by BGZF inflate and row formatting on the host: one GPU)
