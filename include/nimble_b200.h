@@ -461,6 +461,24 @@ int nb_process_bam_rows_any_order(const char* input_file, const char* const* ref
  * and align + finalize times, store bytes, peak RSS).  NB_BULK_BATCH_PAIRS=N: batches of at most N pairs (default and cap 2^20). */
 int nb_process_bam_bulk(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
                         int strand_filter, int num_cores, int device);
+/* Many samples in one run on one GPU: FASTQ samples (bulk 0: one or two .fastq / .fastq.gz inputs each, dispatched on the
+ * extension as the CLI's -i is) or bulk BAM samples (bulk 1: exactly one .bam each).  Sample s is names[s] with inputs
+ * inputs[2 s] and inputs[2 s + 1] (NULL for one input); library i's TSV of it is <output_dirs[i]>/<names[s]>.tsv.  Every such
+ * file gets exactly the bytes that the single run of that sample writes to that path — nb_process_fastq on its inputs, or
+ * nb_process_bam_bulk on its BAM, with the same libraries, strand filter and num_cores — including the append / header-if-
+ * empty behaviour and what is written for empty inputs.  The libraries, their indexes and contexts are set up once; then
+ * the samples run in order, each one library by library (the order of its single run) on the context reset by
+ * nb_counts_reset.  All libraries' contexts are alive together (and in bulk mode the record store of one sample next to
+ * them), so the device peak with several libraries is above a single run's, which holds one library's context at a time.
+ * Checked before any device work, each failure naming the sample: names match [A-Za-z0-9._-]+, are not "." or ".." and are
+ * unique (NB_ERR_INVALID); every sample has inputs of its kind (NB_ERR_INVALID); every input opens (NB_ERR_IO); then every
+ * output directory exists or is created, its parent existing (NB_ERR_IO), as nb_write_cell_matrix does.  A failure while a
+ * sample runs stops the run with the single run's code and message behind "sample <name>: ": the samples before it are
+ * complete, it leaves what its single run leaves, and later samples are not touched.  NB_FASTQ_STATS=1 (FASTQ) or
+ * NB_BAM_STATS=1 (bulk): one setup line (library, index and context times, the CUDA start-up included) and one line per
+ * sample (pairs; parse+align, or windows and pairing; finalize and write). */
+int nb_process_samples(const char* const* names, const char* const* inputs, uint32_t n_samples, const char* const* reference_json,
+                       const char* const* output_dirs, uint32_t n_refs, int strand_filter, int num_cores, int device, int bulk);
 /* test hook: the pairs of nb_process_bam_bulk, one line per pair sorted by R1 ordinal: R1 ordinal TAB R2 ordinal TAB R1 length
  * TAB R2 length TAB R1 flags TAB R2 flags (NB_FLAG_*); a single-end file has '-' for every R2 field.  NB_BULK_NAME_HASH_BITS=b
  * (1..64) keeps b bits of the name key, so that names collide and the exact compare separates them. */

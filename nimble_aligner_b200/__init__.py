@@ -9,11 +9,13 @@ reference's library entry points (paths under /root/reference):
   build_index                  debruijn_mapping::build_index::build_index::<Kmer30>  (src/bin/main.rs:121-128)
   get_calls / call             src/align.rs:392 / src/score.rs:14
   process_fastq                src/process/fastq.rs:7
+  process_samples              many FASTQ or bulk BAM samples in one run (nb_process_samples)
 
 There is no CPU fallback: if the shared library is missing or no sm_100 device is present, calls raise NbError.
 """
 import ctypes as C
 import os
+import re
 
 import numpy as np
 
@@ -158,6 +160,7 @@ _SIGS = {
     "nb_process_bam_rows_any_order": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_char_p, C.c_int, C.c_int, C.c_uint64]),
     "nb_process_bam_bulk": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int]),
     "nb_bam_dump_pairs_bulk": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.c_char_p]),
+    "nb_process_samples": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_int]),
     "nb_cells_roll": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64]),
     "nb_cells_finalize": (C.c_int, [C.c_void_p, C.POINTER(CellCounts)]),
     "nb_cells_reset": (C.c_int, [C.c_void_p]),
@@ -723,6 +726,77 @@ def process_bam(input_file, reference_json_paths, output_paths, strand_filter="u
         return
     _ck(lib().nb_process_bam(str(input_file).encode(), _strs(reference_json_paths), _strs(output_paths), len(reference_json_paths),
                              CHEM[strand_filter], trim.encode() if trim else None, num_cores, int(force_bam_paired), device))
+
+
+_SAMPLE_NAME = re.compile(r"[A-Za-z0-9._-]+")
+
+
+def read_manifest(path):
+    """The samples of a manifest file as [(name, [inputs], line)]: one sample per line, name<TAB>input1[<TAB>input2]; blank
+    lines and lines starting with '#' are skipped.  NbError(-1) naming the line on a syntax error, an illegal or repeated
+    name, or a manifest without samples."""
+    try:
+        with open(path, "rb") as f:
+            text = f.read().decode("utf-8")
+    except (OSError, UnicodeDecodeError) as e:
+        raise NbError(-1, "could not read the sample manifest %s: %s" % (path, e))
+    out, seen = [], {}
+    for k, line in enumerate(text.split("\n"), 1):
+        if line.endswith("\r"):
+            line = line[:-1]
+        if not line.strip(" \t") or line.startswith("#"):
+            continue
+        at = "%s line %d: " % (path, k)
+        col = line.split("\t")
+        if not 2 <= len(col) <= 3:
+            raise NbError(-1, at + "expected name<TAB>input1[<TAB>input2], found %d column(s)" % len(col))
+        if not all(col):
+            raise NbError(-1, at + "empty column")
+        if not _SAMPLE_NAME.fullmatch(col[0]) or col[0] in (".", ".."):
+            raise NbError(-1, at + "sample name '%s' must match [A-Za-z0-9._-]+ and not be '.' or '..'" % col[0])
+        if col[0] in seen:
+            raise NbError(-1, at + "sample name '%s' is already used on line %d" % (col[0], seen[col[0]]))
+        seen[col[0]] = k
+        out.append((col[0], col[1:], k))
+    if not out:
+        raise NbError(-1, "the sample manifest %s has no samples" % path)
+    return out
+
+
+def process_samples(samples, reference_json_paths, output_dirs, strand_filter="unstranded", num_cores=1, device=0, bulk=False):
+    """Many samples in one run on one GPU, the libraries set up once (nb_process_samples).  samples: a manifest path (see
+    read_manifest) or a list of (name, [inputs]): one or two FASTQs each, or with bulk=True one BAM each.  output_dirs: one
+    directory per library; library i's TSV of sample s is <output_dirs[i]>/<s>.tsv, exactly what process_fastq (or
+    process_bam(..., bulk=True)) writes for that sample alone.  Bad arguments raise NbError(-1) before the call; a failing
+    sample raises the single run's code with the message behind "sample <name> (line N): " (a list: "sample <name>: ")."""
+    if isinstance(samples, (str, os.PathLike)):
+        entries = read_manifest(os.fspath(samples))
+    else:
+        if not isinstance(samples, (list, tuple)) or not samples:
+            raise NbError(-1, "samples must be a manifest path or a non-empty list of (name, [inputs])")
+        entries = []
+        for k, smp in enumerate(samples):   # (names, duplicates and input kinds: nb_process_samples, before any device work)
+            if not isinstance(smp, (list, tuple)) or len(smp) != 2 or not isinstance(smp[0], str) or not isinstance(smp[1], (list, tuple)) \
+                    or not 1 <= len(smp[1]) <= 2 or not all(isinstance(x, (str, os.PathLike)) for x in smp[1]):
+                raise NbError(-1, "samples[%d]: expected (name, [one or two input paths])" % k)
+            entries.append((smp[0], [os.fspath(x) for x in smp[1]], None))
+    if isinstance(reference_json_paths, (str, os.PathLike)) or not reference_json_paths:
+        raise NbError(-1, "reference_json_paths must be a non-empty list")
+    if isinstance(output_dirs, (str, os.PathLike)) or output_dirs is None or len(output_dirs) != len(reference_json_paths):
+        raise NbError(-1, "process_samples needs one output directory per reference library")
+    if strand_filter not in CHEM:
+        raise NbError(-1, "unknown strand_filter %r" % (strand_filter,))
+    names = (C.c_char_p * len(entries))(*[e[0].encode("utf-8") for e in entries])
+    inputs = (C.c_char_p * (2 * len(entries)))(*[x for e in entries for x in (e[1][0].encode("utf-8"), e[1][1].encode("utf-8") if len(e[1]) > 1 else None)])
+    rc = lib().nb_process_samples(names, inputs, len(entries), _strs(reference_json_paths), _strs(output_dirs), len(reference_json_paths),
+                                  CHEM[strand_filter], int(num_cores), int(device), 1 if bulk else 0)
+    if rc != 0:
+        msg = lib().nb_last_error().decode("utf-8", "replace")
+        m = re.match(r"sample ([A-Za-z0-9._-]+): ", msg)
+        line = {e[0]: e[2] for e in entries}.get(m.group(1)) if m else None
+        if line is not None:
+            msg = msg[:m.end(1)] + " (line %d)" % line + msg[m.end(1):]
+        raise NbError(rc, msg)
 
 
 def cell_counts_dict(c):

@@ -1679,6 +1679,23 @@ u64 bulk_batch_pairs() {
   return n;
 }
 
+// One library's half of a bulk run: the loaded file's pairs aligned in batches of BATCH through ctx (fresh or reset), the
+// counts finalized and appended to output_path by the FASTQ-mode writer.  t_align: batches and finalize.
+int bulk_align_write(nbg::Device* dev, const BulkRun& run, nb_ctx* ctx, const nb_library* lib, u64 BATCH, const char* output_path, u64& n_batches, double& t_align) {
+  int rc = NB_OK;
+  const double ta = now();
+  for (u64 p0 = 0; p0 < run.bp.n_pairs && rc == NB_OK; p0 += BATCH) {
+    nb_batch b; rc = nbg::batch(dev, p0, std::min(run.bp.n_pairs, p0 + BATCH), 0, run.bp.max_len, b);
+    if (rc == NB_OK) rc = nb_align_batch(ctx, &b, nullptr, nullptr);
+    n_batches++;
+  }
+  nb_counts cts;
+  if (rc == NB_OK) rc = nb_counts_finalize(ctx, &cts);
+  t_align += now() - ta;
+  if (rc == NB_OK) rc = nb_write_fastq_tsv(output_path, lib, &cts);
+  return rc;
+}
+
 // The library loop of nb_process_fastq with the BAM in place of the FASTQs: per library its index and one whole-run
 // context; the file is loaded and paired once, before the first library's batches; every pair is aligned, the counts
 // finalized once and written by the FASTQ-mode writer (append, header iff the file is empty).
@@ -1699,16 +1716,7 @@ int process_bam_bulk(const char* input_file, const char* const* reference_json, 
     if (rc == NB_OK) rc = nb_ctx_create(ix, lib, device, nbg::stream_of(dev), &ctx);   // the batches point into the store: its stream
     if (rc == NB_OK) rc = nb_ctx_set_option(ctx, "max_batch_pairs", BATCH);
     if (rc == NB_OK && li == 0) rc = bulk_load_pair(input_file, threads, dev, run);
-    const double ta = now();
-    for (u64 p0 = 0; p0 < run.bp.n_pairs && rc == NB_OK; p0 += BATCH) {
-      nb_batch b; rc = nbg::batch(dev, p0, std::min(run.bp.n_pairs, p0 + BATCH), 0, run.bp.max_len, b);
-      if (rc == NB_OK) rc = nb_align_batch(ctx, &b, nullptr, nullptr);
-      n_batches++;
-    }
-    nb_counts cts;
-    if (rc == NB_OK) rc = nb_counts_finalize(ctx, &cts);
-    t_align += now() - ta;
-    if (rc == NB_OK) rc = nb_write_fastq_tsv(output_paths[li], lib, &cts);
+    if (rc == NB_OK) rc = bulk_align_write(dev, run, ctx, lib, BATCH, output_paths[li], n_batches, t_align);
     nb_ctx_free(ctx); nb_index_free(ix); nb_library_free(lib);
   }
   if (getenv("NB_BAM_STATS")) {
@@ -1749,6 +1757,53 @@ int dump_pairs_bulk(const char* input_file, int num_cores, int device, const cha
 }
 
 }  // namespace
+
+// The bulk samples of nb_process_samples: one device and store for the run, every library's context created once on its
+// stream; per sample the BAM is loaded and paired, aligned, finalized and written library by library, and the store and
+// pair arrays are dropped (nbg::begin_pass) before the next one.
+int nb::bulk_samples(const char* const* names, const char* const* inputs, u32 n_samples, const char* const* reference_json, const std::vector<std::string>& outs,
+                     u32 n_refs, int strand_filter, int num_cores, int device) {
+  const bool stats = getenv("NB_BAM_STATS") != nullptr;
+  const int threads = std::max(1, num_cores);
+  const u64 BATCH = bulk_batch_pairs();
+  const double t0 = now();
+  nbg::Device* dev = nullptr;
+  struct Store { nbg::Device*& d; ~Store() { nbg::destroy(d); } } store{dev};   // declared before L: the contexts on its stream go first
+  int rc = nbg::create(device, &dev);
+  if (rc) return rc;
+  const double t1 = now();
+  Libraries L;   // (owns them; set up as process_bam_bulk sets up its libraries)
+  L.libs.assign(n_refs, nullptr); L.idx.assign(n_refs, nullptr); L.ctx.assign(n_refs, nullptr);
+  double t_lib = 0, t_index = 0, t_ctx = 0;
+  for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+    const double a = now();
+    rc = nb_library_load_json(reference_json[li], strand_filter, &L.libs[li]);
+    const double b = now(); t_lib += b - a;
+    if (rc == NB_OK) rc = nb_index_build_cached(L.libs[li], nullptr, device, threads, &L.idx[li]);
+    const double c = now(); t_index += c - b;
+    if (rc == NB_OK) rc = nb_ctx_create(L.idx[li], L.libs[li], device, nbg::stream_of(dev), &L.ctx[li]);   // the batches point into the store: its stream
+    if (rc == NB_OK) rc = nb_ctx_set_option(L.ctx[li], "max_batch_pairs", BATCH);
+    t_ctx += now() - c;
+  }
+  if (rc) return rc;
+  if (stats) fprintf(stderr, "nb_process_samples: setup %.3f s (CUDA start-up included): device %.3f s, %u libraries, library %.3f s, index (GPU) %.3f s, contexts %.3f s\n",
+                     now() - t0, t1 - t0, n_refs, t_lib, t_index, t_ctx);
+  for (u32 s = 0; s < n_samples; s++) {
+    BulkRun run; double t_align = 0; u64 n_batches = 0;   // (process_bam_bulk's stats; not printed here)
+    rc = bulk_load_pair(inputs[2 * s], threads, dev, run);
+    const double ta = now();
+    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+      rc = nb_counts_reset(L.ctx[li]);
+      if (rc == NB_OK) rc = bulk_align_write(dev, run, L.ctx[li], L.libs[li], BATCH, outs[(size_t)s * n_refs + li].c_str(), n_batches, t_align);
+    }
+    const double t_write = now() - ta;
+    if (rc == NB_OK) rc = nbg::begin_pass(dev);
+    if (stats) fprintf(stderr, "nb_process_samples: sample %s: %llu records, %llu pairs, windows %.3f s, pairing %.3f s, align+finalize+tsv %.3f s\n",
+                       names[s], (unsigned long long)run.ld.n_records, (unsigned long long)run.bp.n_pairs, run.t_load, run.t_pair, t_write);
+    if (rc) return sample_failed(names[s], rc);
+  }
+  return NB_OK;
+}
 
 extern "C" int nb_process_bam_bulk(const char* input_file, const char* const* reference_json, const char* const* output_paths, uint32_t n_refs,
                                    int strand_filter, int num_cores, int device) {

@@ -24,6 +24,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cerrno>
 #include <condition_variable>
 #include <cstdio>
 #include <cstring>
@@ -564,6 +565,89 @@ extern "C" int nb_fastq_dump(const char* const* input_files, uint32_t n_inputs, 
   return rc;
 }
 
+namespace {
+
+double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + ts.tv_nsec * 1e-9; }
+
+// One reference library of a FASTQ run: the library, its index (the CUDA builder, or $NB_INDEX_CACHE) and one context per
+// device.  nb_process_fastq_devices sets one up per library in turn; nb_process_samples sets up all of them once and runs
+// every sample through them.
+struct FastqLib {
+  nb_library* lib = nullptr; nb_index* ix = nullptr; std::vector<nb_ctx*> ctx;
+  double t_lib = 0, t_index = 0, t_ctx = 0;
+  ~FastqLib() { for (nb_ctx* c : ctx) nb_ctx_free(c); nb_index_free(ix); nb_library_free(lib); }
+  int open(const char* reference_json, int strand_filter, int num_cores, const int* devices, u32 W) {
+    const u64 BATCH = 1u << 20;
+    ctx.assign(W, nullptr);
+    const double t0 = now();
+    int rc = nb_library_load_json(reference_json, strand_filter, &lib);
+    const double t1 = now();
+    if (rc == NB_OK) rc = nb_index_build_cached(lib, nullptr, devices[0], std::max(1, num_cores), &ix);   // K5: the CUDA builder (same artefact as nb_index_build), or $NB_INDEX_CACHE
+    const double t2 = now();
+    for (u32 d = 0; d < W && rc == NB_OK; d++) { rc = nb_ctx_create(ix, lib, devices[d], nullptr, &ctx[d]); if (rc == NB_OK) rc = nb_ctx_set_option(ctx[d], "max_batch_pairs", BATCH); }
+    t_lib = t1 - t0; t_index = t2 - t1; t_ctx = now() - t2;
+    return rc;
+  }
+};
+
+struct FastqJob { u64 pairs = 0, calls = 0; double t_align = 0, t_final = 0; };
+
+// One job of a library: the FASTQs streamed into nb_align_batch (batches dealt to the contexts in turn), the counts
+// finalized (merged across the contexts when there are several) and appended to output_path by write_tsv.  The contexts
+// are fresh or reset (nb_counts_reset).
+int fastq_job(FastqLib& L, const char* const* input_files, u32 n_inputs, int num_cores, const char* output_path, FastqJob& st) {
+  const int T = std::max(1, num_cores / (int)n_inputs);
+  const u32 W = (u32)L.ctx.size();
+  std::vector<nb_ctx*>& ctx = L.ctx;
+  const double t3 = now(); u64 n_pairs_fed = 0, n_calls = 0;
+  int rc = NB_OK;
+  std::unique_ptr<SegStream> s1, s2;
+  s1 = open_stream(input_files[0], T, 1u << 19, chunk_bytes_default(file_bytes(input_files[0]), T), 2 * (int)W); if (!s1) rc = fail(NB_ERR_IO, std::string("could not open ") + input_files[0]);
+  if (rc == NB_OK && n_inputs > 1) { s2 = open_stream(input_files[1], T, 1u << 19, chunk_bytes_default(file_bytes(input_files[1]), T), 2 * (int)W); if (!s2) rc = fail(NB_ERR_IO, std::string("could not open ") + input_files[1]); }
+  if (rc == NB_OK) {
+    // A segment goes back to its stream once the copies out of it have run: nb_align_batch blocks on the copies of a staging
+    // set before refilling it, so everything a context was given before its last two calls is free again (nimble_b200.h);
+    // with W contexts fed in turn that is everything older than 2 W calls.
+    struct Held { SegStream* s; Segment* g; u64 call; };
+    std::deque<Held> held; u64 calls = 0;
+    std::vector<u64> fed(W, 0);
+    auto release = [&](bool all) { while (!held.empty() && (all || held.front().call + 2 * W <= calls)) { held.front().s->recycle(held.front().g); held.pop_front(); } };
+    rc = consume(s1.get(), s2.get(),
+      [&](Segment* a, u64 ka, Segment* b2, u64 kb, u64 m) {
+        const u32 d = (u32)(calls % W);
+        nb_batch b; memset(&b, 0, sizeof b);
+        b.n_pairs = m; b.location = NB_MEM_HOST; b.max_read_len = std::max<u32>(a->maxlen, b2 ? b2->maxlen : 0);
+        b.r1 = a->seq.p; b.r1_off = a->off() + ka;
+        if (b2) { b.r2 = b2->seq.p; b.r2_off = b2->off() + kb; }
+        int r = NB_OK;
+        if (W > 1) r = nb_route_set_pair_base(ctx[d], n_pairs_fed - fed[d]);   // this batch's pairs are numbered n_pairs_fed.. in the job; the context adds its own count
+        if (r == NB_OK) r = nb_align_batch(ctx[d], &b, nullptr, nullptr);
+        calls++; release(false); n_pairs_fed += m; fed[d] += m; n_calls++;
+        return r;
+      },
+      [&](SegStream* s, Segment* g) { held.push_back({s, g, calls}); release(false); });
+    for (u32 d = 0; d < W; d++) if (nb_ctx_sync(ctx[d]) != NB_OK && rc == NB_OK) rc = NB_ERR_CUDA;
+    release(true);
+  }
+  if (s1) s1->finish();
+  if (s2) s2->finish();
+  const double t4 = now();
+  std::vector<nb_counts> cts(W);
+  if (rc == NB_OK && W == 1) rc = nb_counts_finalize(ctx[0], &cts[0]);
+  if (rc == NB_OK && W > 1) {   // collective: every context's call must be in flight at the same time
+    std::vector<int> rcs(W, NB_OK); std::vector<std::string> msgs(W); std::vector<std::thread> th;
+    for (u32 d = 0; d < W; d++) th.emplace_back([&, d] { rcs[d] = nb_merge_whole_run(ctx[d], &cts[d]); if (rcs[d] != NB_OK) msgs[d] = nb_last_error(); });
+    for (auto& x : th) x.join();
+    for (u32 d = 0; d < W && rc == NB_OK; d++) if (rcs[d] != NB_OK) rc = fail(rcs[d], msgs[d]);
+  }
+  if (rc == NB_OK) rc = write_tsv(output_path, L.lib, cts[0]);
+  s1.reset(); s2.reset();
+  st.pairs = n_pairs_fed; st.calls = n_calls; st.t_align = t4 - t3; st.t_final = now() - t4;
+  return rc;
+}
+
+}  // namespace
+
 // process::fastq::process with the library loop of src/bin/main.rs:95-133 in front of it, on one or several GPUs.
 // Several devices: one context per GPU behind the one feeder (the reference's shape is N-1 consumers behind one producer,
 // src/process/bam.rs:183-226); batches go to the contexts in turn with their global pair numbers, k_pair routes every
@@ -573,75 +657,28 @@ extern "C" int nb_process_fastq_devices(const char* const* input_files, uint32_t
                                         uint32_t n_refs, int strand_filter, int num_cores, const int* devices, uint32_t n_devices) {
   if (!input_files || !reference_json || !output_paths || n_inputs < 1 || n_inputs > 2 || n_refs < 1) return fail(NB_ERR_INVALID, "need 1-2 inputs and >=1 reference/output pair");
   if (!devices || n_devices < 1 || n_devices > 16) return fail(NB_ERR_INVALID, "need 1-16 devices");
-  const u64 BATCH = 1u << 20;
-  const int T = std::max(1, num_cores / (int)n_inputs);
   const u32 W = n_devices;
   const bool stats = getenv("NB_FASTQ_STATS") != nullptr;   // phase times on stderr
-  auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + ts.tv_nsec * 1e-9; };
   for (u32 li = 0; li < n_refs; li++) {
-    nb_library* lib = nullptr; nb_index* ix = nullptr; std::vector<nb_ctx*> ctx(W, nullptr);
-    const double t0 = now();
-    int rc = nb_library_load_json(reference_json[li], strand_filter, &lib);
-    const double t1 = now();
-    if (rc == NB_OK) rc = nb_index_build_cached(lib, nullptr, devices[0], std::max(1, num_cores), &ix);   // K5: the CUDA builder (same artefact as nb_index_build), or $NB_INDEX_CACHE
-    const double t2 = now();
-    for (u32 d = 0; d < W && rc == NB_OK; d++) { rc = nb_ctx_create(ix, lib, devices[d], nullptr, &ctx[d]); if (rc == NB_OK) rc = nb_ctx_set_option(ctx[d], "max_batch_pairs", BATCH); }
+    FastqLib L; FastqJob st;
+    int rc = L.open(reference_json[li], strand_filter, num_cores, devices, W);
+    std::vector<nb_ctx*>& ctx = L.ctx;
     if (rc == NB_OK && W > 1) {
       // inbox regions hold every record a peer sends during the job: sized from the input (a record of a 100-base read is
       // about 230 bytes of text, gzip packs it about five-fold); NB_ROUTE_RECORDS overrides; a region that fills up fails loudly
+      const double t0 = now();
       const char* e = getenv("NB_ROUTE_RECORDS");
       u64 est = file_bytes(input_files[0]) / 100; if (is_gzip(input_files[0])) est *= 6;
       const u64 rpp = e ? strtoull(e, nullptr, 10) : est * 2 / ((u64)W * W) + 65536;
       rc = nb_comm_init_all(ctx.data(), W);
       for (u32 d = 0; d < W && rc == NB_OK; d++) rc = nb_route_create(ctx[d], W, rpp, nullptr);
       for (u32 d = 0; d < W && rc == NB_OK; d++) rc = nb_route_attach_ctx(ctx[d], W, d, ctx.data(), 0);
+      L.t_ctx += now() - t0;
     }
-    const double t3 = now(); u64 n_pairs_fed = 0, n_calls = 0;
-    std::unique_ptr<SegStream> s1, s2;
-    if (rc == NB_OK) { s1 = open_stream(input_files[0], T, 1u << 19, chunk_bytes_default(file_bytes(input_files[0]), T), 2 * (int)W); if (!s1) rc = fail(NB_ERR_IO, std::string("could not open ") + input_files[0]); }
-    if (rc == NB_OK && n_inputs > 1) { s2 = open_stream(input_files[1], T, 1u << 19, chunk_bytes_default(file_bytes(input_files[1]), T), 2 * (int)W); if (!s2) rc = fail(NB_ERR_IO, std::string("could not open ") + input_files[1]); }
-    if (rc == NB_OK) {
-      // A segment goes back to its stream once the copies out of it have run: nb_align_batch blocks on the copies of a staging
-      // set before refilling it, so everything a context was given before its last two calls is free again (nimble_b200.h);
-      // with W contexts fed in turn that is everything older than 2 W calls.
-      struct Held { SegStream* s; Segment* g; u64 call; };
-      std::deque<Held> held; u64 calls = 0;
-      std::vector<u64> fed(W, 0);
-      auto release = [&](bool all) { while (!held.empty() && (all || held.front().call + 2 * W <= calls)) { held.front().s->recycle(held.front().g); held.pop_front(); } };
-      rc = consume(s1.get(), s2.get(),
-        [&](Segment* a, u64 ka, Segment* b2, u64 kb, u64 m) {
-          const u32 d = (u32)(calls % W);
-          nb_batch b; memset(&b, 0, sizeof b);
-          b.n_pairs = m; b.location = NB_MEM_HOST; b.max_read_len = std::max<u32>(a->maxlen, b2 ? b2->maxlen : 0);
-          b.r1 = a->seq.p; b.r1_off = a->off() + ka;
-          if (b2) { b.r2 = b2->seq.p; b.r2_off = b2->off() + kb; }
-          int r = NB_OK;
-          if (W > 1) r = nb_route_set_pair_base(ctx[d], n_pairs_fed - fed[d]);   // this batch's pairs are numbered n_pairs_fed.. in the job; the context adds its own count
-          if (r == NB_OK) r = nb_align_batch(ctx[d], &b, nullptr, nullptr);
-          calls++; release(false); n_pairs_fed += m; fed[d] += m; n_calls++;
-          return r;
-        },
-        [&](SegStream* s, Segment* g) { held.push_back({s, g, calls}); release(false); });
-      for (u32 d = 0; d < W; d++) if (nb_ctx_sync(ctx[d]) != NB_OK && rc == NB_OK) rc = NB_ERR_CUDA;
-      release(true);
-    }
-    if (s1) s1->finish();
-    if (s2) s2->finish();
-    const double t4 = now();
-    std::vector<nb_counts> cts(W);
-    if (rc == NB_OK && W == 1) rc = nb_counts_finalize(ctx[0], &cts[0]);
-    if (rc == NB_OK && W > 1) {   // collective: every context's call must be in flight at the same time
-      std::vector<int> rcs(W, NB_OK); std::vector<std::string> msgs(W); std::vector<std::thread> th;
-      for (u32 d = 0; d < W; d++) th.emplace_back([&, d] { rcs[d] = nb_merge_whole_run(ctx[d], &cts[d]); if (rcs[d] != NB_OK) msgs[d] = nb_last_error(); });
-      for (auto& x : th) x.join();
-      for (u32 d = 0; d < W && rc == NB_OK; d++) if (rcs[d] != NB_OK) rc = fail(rcs[d], msgs[d]);
-    }
-    if (rc == NB_OK) rc = write_tsv(output_paths[li], lib, cts[0]);
-    s1.reset(); s2.reset();
+    if (rc == NB_OK) rc = fastq_job(L, input_files, n_inputs, num_cores, output_paths[li], st);
     if (stats) fprintf(stderr, "nb_process_fastq: library %.3f s, index (GPU) %.3f s, %u context(s) %.3f s, parse+align %.3f s (%llu pairs in %llu calls, %d parser threads per file: %.1f M reads/s), finalize+tsv %.3f s\n",
-                       t1 - t0, t2 - t1, W, t3 - t2, t4 - t3, (unsigned long long)n_pairs_fed, (unsigned long long)n_calls, T, (double)n_pairs_fed * n_inputs / std::max(t4 - t3, 1e-9) / 1e6, now() - t4);
-    for (u32 d = 0; d < W; d++) nb_ctx_free(ctx[d]);
-    nb_index_free(ix); nb_library_free(lib);
+                       L.t_lib, L.t_index, W, L.t_ctx, st.t_align, (unsigned long long)st.pairs, (unsigned long long)st.calls, std::max(1, num_cores / (int)n_inputs),
+                       (double)st.pairs * n_inputs / std::max(st.t_align, 1e-9) / 1e6, st.t_final);
     if (rc != NB_OK) return rc;
   }
   return NB_OK;
@@ -650,4 +687,91 @@ extern "C" int nb_process_fastq_devices(const char* const* input_files, uint32_t
 extern "C" int nb_process_fastq(const char* const* input_files, uint32_t n_inputs, const char* const* reference_json, const char* const* output_paths,
                                 uint32_t n_refs, int strand_filter, int num_cores, int device) {
   return nb_process_fastq_devices(input_files, n_inputs, reference_json, output_paths, n_refs, strand_filter, num_cores, &device, 1);
+}
+
+namespace {
+
+bool ends_with(const std::string& s, const char* suf) { const size_t n = strlen(suf); return s.size() >= n && s.compare(s.size() - n, n, suf) == 0; }
+
+// What nb_process_samples checks before any device work, in this order: names, every sample's inputs (count and kind, as
+// the CLI dispatches -i on the extension), that every input opens, and that every output directory exists or can be made.
+int check_samples(const char* const* names, const char* const* inputs, u32 n_samples, const char* const* output_dirs, u32 n_refs, bool bulk) {
+  std::vector<std::string> seen;
+  for (u32 s = 0; s < n_samples; s++) {
+    const std::string name = names[s] ? names[s] : "";
+    auto bad = [&](int code, const std::string& m) { return fail(code, "sample " + name + ": " + m); };
+    bool legal = !name.empty() && name != "." && name != "..";
+    for (char c : name) legal = legal && ((c >= 'A' && c <= 'Z') || (c >= 'a' && c <= 'z') || (c >= '0' && c <= '9') || c == '.' || c == '_' || c == '-');
+    if (!legal) return bad(NB_ERR_INVALID, "a sample name matches [A-Za-z0-9._-]+ and is not '.' or '..'");
+    if (std::find(seen.begin(), seen.end(), name) != seen.end()) return bad(NB_ERR_INVALID, "the name is used by an earlier sample");
+    seen.push_back(name);
+    const char* in[2] = {inputs[2 * s], inputs[2 * s + 1]};
+    if (!in[0]) return bad(NB_ERR_INVALID, "no input");
+    if (bulk && in[1]) return bad(NB_ERR_INVALID, "a bulk sample has exactly one .bam input");
+    for (int k = 0; k < 2 && in[k]; k++) {
+      std::string lower = in[k]; std::transform(lower.begin(), lower.end(), lower.begin(), ::tolower);
+      const bool fastq = ends_with(in[k], ".fastq.gz") || ends_with(lower, ".fastq"), bam = ends_with(lower, ".bam");
+      if (bulk && !bam) return bad(NB_ERR_INVALID, std::string("a bulk sample has exactly one .bam input, not ") + in[k]);
+      if (!bulk && bam) return bad(NB_ERR_INVALID, std::string(in[k]) + " is a BAM: BAM samples run in bulk mode (--bulk)");
+      if (!bulk && !fastq) return bad(NB_ERR_INVALID, std::string("unsupported file format of ") + in[k] + ": FASTQ samples have .fastq or .fastq.gz inputs");
+    }
+  }
+  for (u32 s = 0; s < n_samples; s++)
+    for (int k = 0; k < 2 && inputs[2 * s + k]; k++) {
+      const int fd = ::open(inputs[2 * s + k], O_RDONLY);
+      if (fd < 0) return fail(NB_ERR_IO, std::string("sample ") + names[s] + ": could not open " + inputs[2 * s + k] + ": " + strerror(errno));
+      ::close(fd);
+    }
+  for (u32 li = 0; li < n_refs; li++) {   // created when missing, its parent must exist (as nb_write_cell_matrix does)
+    const char* dir = output_dirs[li];
+    if (!dir || !*dir) return fail(NB_ERR_INVALID, "empty output directory");
+    if (mkdir(dir, 0777) != 0 && errno != EEXIST) return fail(NB_ERR_IO, std::string("could not create output directory ") + dir + ": " + strerror(errno));
+    struct stat st; if (stat(dir, &st) != 0 || !S_ISDIR(st.st_mode)) return fail(NB_ERR_IO, std::string("output directory ") + dir + " is not a directory");
+  }
+  return NB_OK;
+}
+
+// FASTQ samples on one device: every library set up once (FastqLib), then sample by sample, library by library, a job on
+// the reset context.
+int fastq_samples(const char* const* names, const char* const* inputs, u32 n_samples, const char* const* reference_json, const std::vector<std::string>& outs,
+                  u32 n_refs, int strand_filter, int num_cores, int device) {
+  const bool stats = getenv("NB_FASTQ_STATS") != nullptr;
+  const double t0 = now();
+  std::vector<std::unique_ptr<FastqLib>> L(n_refs);
+  double t_lib = 0, t_index = 0, t_ctx = 0;
+  for (u32 li = 0; li < n_refs; li++) {
+    L[li].reset(new FastqLib());
+    const int rc = L[li]->open(reference_json[li], strand_filter, num_cores, &device, 1);
+    t_lib += L[li]->t_lib; t_index += L[li]->t_index; t_ctx += L[li]->t_ctx;
+    if (rc != NB_OK) return rc;
+  }
+  if (stats) fprintf(stderr, "nb_process_samples: setup %.3f s (CUDA start-up included): %u libraries, library %.3f s, index (GPU) %.3f s, contexts %.3f s\n", now() - t0, n_refs, t_lib, t_index, t_ctx);
+  for (u32 s = 0; s < n_samples; s++) {
+    const u32 n_inputs = inputs[2 * s + 1] ? 2 : 1;
+    FastqJob sum;
+    int rc = NB_OK;
+    for (u32 li = 0; li < n_refs && rc == NB_OK; li++) {
+      FastqJob st;
+      rc = nb_counts_reset(L[li]->ctx[0]);
+      if (rc == NB_OK) rc = fastq_job(*L[li], inputs + 2 * s, n_inputs, num_cores, outs[(size_t)s * n_refs + li].c_str(), st);
+      sum.pairs = st.pairs; sum.t_align += st.t_align; sum.t_final += st.t_final;
+    }
+    if (stats) fprintf(stderr, "nb_process_samples: sample %s: %llu pairs, parse+align %.3f s, finalize+tsv %.3f s\n", names[s], (unsigned long long)sum.pairs, sum.t_align, sum.t_final);
+    if (rc != NB_OK) return sample_failed(names[s], rc);
+  }
+  return NB_OK;
+}
+
+}  // namespace
+
+extern "C" int nb_process_samples(const char* const* names, const char* const* inputs, uint32_t n_samples, const char* const* reference_json,
+                                  const char* const* output_dirs, uint32_t n_refs, int strand_filter, int num_cores, int device, int bulk) {
+  if (!names || !inputs || !reference_json || !output_dirs || n_samples < 1 || n_refs < 1) return fail(NB_ERR_INVALID, "need >=1 sample and >=1 reference library / output directory pair");
+  for (u32 li = 0; li < n_refs; li++) if (!reference_json[li]) return fail(NB_ERR_INVALID, "null reference library");
+  int rc = check_samples(names, inputs, n_samples, output_dirs, n_refs, bulk != 0);
+  if (rc != NB_OK) return rc;
+  std::vector<std::string> outs;   // library li's TSV of sample s: outs[s * n_refs + li] = <output_dirs[li]>/<name>.tsv
+  for (u32 s = 0; s < n_samples; s++) for (u32 li = 0; li < n_refs; li++) outs.push_back(std::string(output_dirs[li]) + "/" + names[s] + ".tsv");
+  if (bulk) return bulk_samples(names, inputs, n_samples, reference_json, outs, n_refs, strand_filter, num_cores, device);
+  return fastq_samples(names, inputs, n_samples, reference_json, outs, n_refs, strand_filter, num_cores, device);
 }

@@ -34,6 +34,12 @@ inline u8 base_code(u8 c) {
 
 int natural_lexical_cmp(const std::string& a, const std::string& b);
 
+// nb_process_samples (fastq.cpp): a failing sample keeps the code and message of its single run behind "sample <name>: "
+inline int sample_failed(const char* name, int rc) { return fail(rc, std::string("sample ") + name + ": " + nb_last_error()); }
+// its bulk samples (bam.cpp), after the checks: inputs[2 s] = sample s's BAM, outs[s * n_refs + li] = library li's TSV of it
+int bulk_samples(const char* const* names, const char* const* inputs, u32 n_samples, const char* const* reference_json, const std::vector<std::string>& outs,
+                 u32 n_refs, int strand_filter, int num_cores, int device);
+
 }  // namespace nb
 
 // Reference + AlignFilterConfig (src/reference_library.rs:11-17, src/align.rs:80-95) plus the integer tables the
